@@ -2,6 +2,7 @@
 """bench.py — ensemble chain-steps/sec of the step_all()/measure() hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c1|c3|c4]
+                    [--dump-outputs DIR]
 
 Headline workload (N=1 and per rank for N>1, weak scaling): BASELINE.json configs[1] — demo/toymodel_xypotentialwell:
 2 real params, E = x^2+y^2, T = 0.1, 65,536 chains x 10^5 steps, measure every 10 steps (DXY:39-44), FP64.
@@ -26,6 +27,8 @@ check.invariance: SHA-256 of the state block of global chains 0..255 after one p
 cpu_baseline / --impl reference: the UNMODIFIED reference (baseline/_ref, or /root/reference in the build container;
          kind "reference") driven by its own README loop on the host cores, one chain per process; if neither copy is on
          the box, the numpy port of the same loop (oracle/py_port.py, pinned bit-for-bit against the reference; kind "port").
+--dump-outputs DIR: after the timed steps, what the timed path handed its caller in its last step as float64 DIR/<name>.npy
+         (see dump_outputs), so that two builds can be compared output for output on identical seeded inputs.
 """
 import argparse
 import json
@@ -33,6 +36,8 @@ import os
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True        # the tree may be read-only: the bench writes nothing into it
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -512,10 +517,10 @@ def per_chain_large_pass(ctx, hbm_peak, steps=3, warmup=2, chains=32768, measure
     return rec
 
 
-def c4_pass(ctx, peaks, steps=3, warmup=3, measures=100):
+def c4_pass(ctx, peaks, steps=3, warmup=3, measures=100, dump=None):
     """BASELINE config 4: 1 real + 64 complex, shared proposal covariance, 32,768 chains per GPU; tcgen05 path.  One pass =
     `measures` x (10 x step_all() + measure()), the pooled-covariance update (and, for N > 1, its moment all-reduce)
-    at every measure."""
+    at every measure.  `dump`: directory for dump_outputs() after the timed passes."""
     import metropolisengine_b200 as me
     torch = ctx.torch
     chains, M, spm = 32768, measures, 10
@@ -533,6 +538,9 @@ def c4_pass(ctx, peaks, steps=3, warmup=3, measures=100):
     l0[0] = eng.launch_count
     ms = ctx.timed(one, steps, 0)
     launches = eng.launch_count - l0[0]
+    if dump:
+        dump_outputs(dump, eng, {"covariance_matrix_real": eng.covariance_matrix_real,
+                                 "covariance_matrix_complex": eng.covariance_matrix_complex})
     value = chains * ctx.world * M * spm * steps / (ms * 1e-3)
     a, b = ctx.event(), ctx.event()
     a.record(ctx.stream)
@@ -600,6 +608,47 @@ def c5_pass(ctx, steps=3, warmup=3, total_chains=1 << 20, launches=20):
     return rec
 
 
+# per-chain state and time-series samples; with the pooled statistics the dump stays well under 64 MB
+DUMP_STATE_BYTES, DUMP_TS_BYTES = 24 << 20, 32 << 20
+
+
+def _sorted_sample(rng, n, k):
+    import numpy as np
+    return np.arange(n) if k >= n else np.sort(rng.choice(n, k, replace=False))
+
+
+def dump_outputs(out_dir, eng, extra):
+    """Write what the timed path handed its caller after its last step as float64 ``out_dir/<name>.npy``: the per-chain
+    state block ``state`` [words, chains] (parameters, energy, widths, means, covariances, counters), the recorded rows
+    ``time_series`` [rows, columns, chains] and the arrays of ``extra`` (complex values get a trailing [re, im] axis,
+    scalars become shape (1,), empty arrays are not written).
+    Chains (and, for very long series, rows) are a fixed seeded sample sized to the byte budgets above; the sampled
+    indices are written beside the arrays (``state_chains``, ``time_series_chains``, ``time_series_rows``)."""
+    import numpy as np
+    import torch
+    rng = np.random.default_rng(0)
+    words, n = eng.state.shape
+    chains = _sorted_sample(rng, n, DUMP_STATE_BYTES // (8 * words))
+    out = {"state": eng.state[:, torch.as_tensor(chains, device=eng.state.device)], "state_chains": chains}
+    ts = eng.time_series()
+    if ts.shape[0]:
+        rows, row_bytes = ts.shape[0], 8 * ts.shape[1]
+        ts_chains = chains[_sorted_sample(rng, len(chains), max(1, DUMP_TS_BYTES // (row_bytes * rows)))]
+        ts_rows = _sorted_sample(rng, rows, DUMP_TS_BYTES // (row_bytes * len(ts_chains)))
+        sub = ts.index_select(2, torch.as_tensor(ts_chains, device=ts.device))
+        out.update(time_series=sub[torch.as_tensor(ts_rows, device=ts.device)], time_series_chains=ts_chains,
+                   time_series_rows=ts_rows)
+    out.update(extra)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        a = np.atleast_1d(np.asarray(a.cpu() if isinstance(a, torch.Tensor) else a))
+        if a.size == 0:                   # e.g. complex statistics of an all-real workload: nothing was computed
+            continue
+        if np.iscomplexobj(a):
+            a = np.stack([a.real, a.imag], axis=-1)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 def run_ours(args):
     import ctypes
     import hashlib
@@ -652,6 +701,10 @@ def run_ours(args):
         ev1.record(stream)
         ctx.barrier()
     launches = eng.launch_count - launches0
+    if args.dump_outputs:
+        ps = eng.pooled_statistics()          # collective when sharded: every rank must call it
+        if rank == 0:
+            dump_outputs(args.dump_outputs, eng, {"pooled_" + k: v for k, v in ps.items()})
     ms_total = ctx.max_over_ranks(ev0.elapsed_time(ev1))
     chain_steps_per_pass = chains * world * M * spm
     value = chain_steps_per_pass * args.steps / (ms_total * 1e-3)
@@ -805,7 +858,8 @@ def run_c4(args):
     ctx = Ctx()
     peaks = _peaks() or {}
     with ClockSampler(ctx.local_rank) as clocks:
-        rec = c4_pass(ctx, peaks, steps=args.steps, warmup=args.warmup, measures=(args.measures or 100))
+        rec = c4_pass(ctx, peaks, steps=args.steps, warmup=args.warmup, measures=(args.measures or 100),
+                      dump=args.dump_outputs if ctx.rank == 0 else None)
     if ctx.rank != 0:
         ctx.close()
         return 0
@@ -842,7 +896,13 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-workloads", action="store_true", help="skip the c1/c3/c4/c5 sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64, under 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3                                   # timing rule: W >= 3
     if args.impl == "reference":
