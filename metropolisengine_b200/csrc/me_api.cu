@@ -437,6 +437,21 @@ void base_params(me_engine *e, MeParams &p) {
     p.m = e->cfg.n_real + e->cfg.n_complex;
     p.temp = e->cfg.temp;
     p.inv_temp = e->cfg.temp != 0 ? 1.0 / e->cfg.temp : 0.0;
+    /* FP32 window of the throughput build's Metropolis test (me_device.cuh, Rng::accept_window).  Its error budget is
+       relative to T and holds while T ln2 and 4e-5 T are normal floats far from overflow, i.e. for 1e-30 <= T <= 1e30.
+       T = 0: the half-width is the smallest denormal, so that the window is [-2^-149, 2^-149] and a dE that rounds to
+       +-0 in FP32 takes the exact test.  Any other T: an infinite half-width sends every decision to the exact test. */
+    const double t = e->cfg.temp;
+    if (t == 0) {
+        p.t_ln2 = 0.0f;
+        p.t_band = 0x1p-149f;
+    } else if (t >= 1e-30 && t <= 1e30) {
+        p.t_ln2 = (float)(t * 0.69314718055994531);
+        p.t_band = (float)(t * 4e-5);
+    } else {
+        p.t_ln2 = 0.0f;
+        p.t_band = HUGE_VALF;
+    }
     p.target = e->cfg.target_acceptance;
     p.ratio = e->cfg.ratio;
     memcpy(p.consts, e->consts, sizeof(p.consts));

@@ -176,16 +176,23 @@ struct Rng {
      * threshold.  u 2^32 lies in [w0, w0 + 1); with w0 >= 2^18 the estimate ln u ~ ln((w0 + 1/2) 2^-32) is off by at most
      * 1.9e-6, MUFU.LG2 by 2^-22 relative of |log2 u| <= 14 (7.7e-6 ln2 in ln u at worst over the full range), the
      * conversion and the FP32 FMA / adds by < 4e-6 T: |estimate - (-T ln u)| < 1.1e-5 T; the window half-width is 4e-5 T.
-     * dE <= lo accepts, dE > hi rejects, in between (probability ~2e-5 per step) the caller computes the exact threshold.
-     * w0 < 2^18 (probability 2^-14): window [0, inf), i.e. always the exact path for uphill moves.  T == 0: lo = hi = 0. */
-    __device__ __forceinline__ static void accept_window(unsigned w0, float t_ln2, float t_band, double &lo, double &hi) {
+     * The caller decides: dE <= lo accepts, dE > hi rejects, anything else — in between (probability ~2e-5 per step) or
+     * NaN — takes the exact test dE <= -T ln u.
+     * Invariant: every decision equals the exact test, so the chains are those of an exact FP64 comparison, bit for bit.
+     *   1e-30 <= T <= 1e30 (t_ln2 = T ln2, t_band = 4e-5 T, both rounded once on the host): |thr| <= 9.8 T, so the
+     *   rounding of lo / hi (relative 2^-24, absolute 2^-150 below the normal range) adds < 6e-7 T + 2^-150 to the
+     *   1.1e-5 T of the estimate, well inside the half-width.  A NaN dE fails both comparisons.
+     *   w0 < 2^18 (probability 2^-14): [-2^-149, inf), i.e. only dE <= -2^-149 (< 0 <= -T ln u) is decided here.
+     *   T == 0 (t_ln2 = 0, t_band = 2^-149): [-2^-149, 2^-149], so a dE of magnitude below 2^-149 is exact.
+     *   Any other T (t_band = inf): (-inf, inf), every decision is exact. */
+    __device__ __forceinline__ static void accept_window(unsigned w0, float t_ln2, float t_band, float &lo, float &hi) {
         float lg;
         const float f = __uint2float_rn(w0) + 0.5f;
         asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg) : "f"(f));
         const float thr = (32.0f - lg) * t_ln2;                   /* T ln2 (32 - log2(w0 + 1/2)) */
         const bool wide = w0 < 0x40000u;
-        lo = (double)(wide ? 0.0f : thr - t_band);
-        hi = (double)(wide ? __int_as_float(0x7f800000) : thr + t_band);
+        lo = wide ? -0x1p-149f : thr - t_band;
+        hi = wide ? __int_as_float(0x7f800000) : thr + t_band;
     }
 };
 
@@ -356,9 +363,10 @@ __device__ __forceinline__ int refactor(const Stats<L> &s, Chain<L> &c) {
 template <class L>
 struct Draws {                 /* everything random one step consumes; independent of the chain's state */
     double z[(L::D + 1) / 2 * 2];
-    double u;                  /* parity build: the accept uniform; throughput build: lower edge of the threshold window */
-    double uhi;                /* throughput build: upper edge of the threshold window (Rng::accept_window) */
-    double u2, uhi2;           /* D = 1 (ShareCall): the same two for the odd step of the pair; z[1] is its normal */
+    double u;                  /* parity build: the accept uniform */
+    float lo, hi;              /* throughput build: the threshold window (Rng::accept_window) */
+    double u2;                 /* D = 1 (ShareCall): the same for the odd step of the pair; z[1] is its normal */
+    float lo2, hi2;
 };
 
 template <class L>
@@ -373,36 +381,36 @@ __device__ __forceinline__ void gen_bits(const Rng &rng, unsigned step, Raw<L> &
     for (int q = 0; q < (L::D + 1) / 2; q++) raw.r[q] = rng.bits(step, (unsigned)q);
 }
 
-/* D = 1: everything the two steps of a pair consume, from the pair's call: z[0] / (u, uhi) for the even step, z[1] /
-   (u2, uhi2) for the odd one */
+/* D = 1: everything the two steps of a pair consume, from the pair's call: z[0] / (u | lo, hi) for the even step, z[1] /
+   (u2 | lo2, hi2) for the odd one */
 template <class L, bool STRICT, class Tab>
 __device__ __forceinline__ void shape_pair(const Raw<L> &raw, const MathTables &T, Draws<L> &d, const Pins &pins,
-                                           double half_temp, const Tab &logtab) {
+                                           const MeParams &p, const Tab &logtab) {
     const U4 r = raw.r[0];
     Rng::box_muller<STRICT, Tab>(share_radius_bits(r), T, d.z[0], d.z[1], pins.unit, pins.angle, logtab);
     const Spare se = share_spare(r, 0u), so = share_spare(r, 1u);
     if (STRICT) {
-        d.u = Rng::accept_uniform(se); d.uhi = 0.0;
-        d.u2 = Rng::accept_uniform(so); d.uhi2 = 0.0;
+        d.u = Rng::accept_uniform(se);
+        d.u2 = Rng::accept_uniform(so);
     } else {
-        const float t2 = (float)(2.0 * half_temp);
-        Rng::accept_window(se.w0, t2 * 0.69314718f, t2 * 4e-5f, d.u, d.uhi);
-        Rng::accept_window(so.w0, t2 * 0.69314718f, t2 * 4e-5f, d.u2, d.uhi2);
+        Rng::accept_window(se.w0, p.t_ln2, p.t_band, d.lo, d.hi);
+        Rng::accept_window(so.w0, p.t_ln2, p.t_band, d.lo2, d.hi2);
     }
 }
 /* the odd step of a pair takes over what the even step carried */
 template <class L>
 __device__ __forceinline__ void take_second_half(const Draws<L> &even, Draws<L> &odd) {
     odd.z[0] = even.z[1]; odd.z[1] = even.z[1];
-    odd.u = even.u2; odd.uhi = even.uhi2; odd.u2 = even.u2; odd.uhi2 = even.uhi2;
+    odd.u = even.u2; odd.u2 = even.u2;
+    odd.lo = even.lo2; odd.hi = even.hi2; odd.lo2 = even.lo2; odd.hi2 = even.hi2;
 }
 
 template <class L, bool STRICT, class Tab>
 __device__ __forceinline__ void shape_draws(const Raw<L> &raw, const MathTables &T, Draws<L> &d, const Pins &pins,
-                                            double half_temp, const Tab &logtab, unsigned step = 0u) {
+                                            const MeParams &p, const Tab &logtab, unsigned step = 0u) {
     constexpr int NQ = (L::D + 1) / 2;
     if (ShareCall<L>::value) {            /* stateless form: the draws of `step` from its pair's call */
-        shape_pair<L, STRICT, Tab>(raw, T, d, pins, half_temp, logtab);
+        shape_pair<L, STRICT, Tab>(raw, T, d, pins, p, logtab);
         if (step & 1u) { const Draws<L> e = d; take_second_half<L>(e, d); }
         return;
     }
@@ -414,22 +422,18 @@ __device__ __forceinline__ void shape_draws(const Raw<L> &raw, const MathTables 
         Rng::box_muller<STRICT, Tab>(raw.r[q], T, d.z[2 * q], d.z[2 * q + 1], pins.unit, pins.angle, logtab);
     }
     /* strict build: the uniform itself; throughput build: a window around the energy threshold -T ln u */
-    if (STRICT) {
-        d.u = Rng::accept_uniform(sp);
-        d.uhi = 0.0;
-    } else {
-        const float t2 = (float)(2.0 * half_temp);
-        Rng::accept_window(sp.w0, t2 * 0.69314718f, t2 * 4e-5f, d.u, d.uhi);
-    }
-    d.u2 = d.uhi2 = 0.0;
+    if (STRICT) d.u = Rng::accept_uniform(sp);
+    else Rng::accept_window(sp.w0, p.t_ln2, p.t_band, d.lo, d.hi);
+    d.u2 = 0.0;
+    d.lo2 = d.hi2 = 0.0f;
 }
 
 template <class L, bool STRICT, class Tab>
 __device__ __forceinline__ void gen_draws(const Rng &rng, unsigned step, const MathTables &T, Draws<L> &d,
-                                          const Pins &pins, double half_temp, const Tab &logtab) {
+                                          const Pins &pins, const MeParams &p, const Tab &logtab) {
     Raw<L> raw;
     gen_bits<L>(rng, step, raw);
-    shape_draws<L, STRICT, Tab>(raw, T, d, pins, half_temp, logtab, step);
+    shape_draws<L, STRICT, Tab>(raw, T, d, pins, p, logtab, step);
 }
 
 template <class L>
@@ -587,23 +591,48 @@ struct MeasureClock {
     __device__ __forceinline__ void start(long long n) { dn = (double)n; inv_dn = __drcp_rn(dn); }
 };
 
+/* Everything of one measure period of the throughput build that depends on the measure counter alone, i.e. is the same
+ * for every chain of the launch: the Robbins-Monro gains of the period's steps and the coefficients of the measure that
+ * ends it.  run_body has the threads of a CTA compute a chunk of these rows into shared memory once, instead of every
+ * thread recomputing its row (two reciprocals with their slow-path tests, the gains) in every period. */
+struct MeasureRow {
+    double up, ndown;                          /* Gains::up / ndown of the period's steps */
+    double inv_n, inv_n1, shrink, decay, grow; /* the measure: counter n0 -> n0 + 1 */
+    double pad;
+};
+static_assert(sizeof(MeasureRow) == 64, "run_body's shared-memory budget counts 64 bytes per MeasureRow");
+
+/* the row of the period that starts at counter n0 (the same values as a MeasureClock started at n0 and advanced by
+   one measure) */
+__device__ __forceinline__ void fill_measure_row(long long n0, const MeParams &p, MeasureRow &r) {
+    MeasureClock clk;
+    clk.start(n0);
+    const Gains g = make_gains<true>(n0, p, clk.inv_dn);
+    const double dn1 = clk.dn, dn = dn1 + 1.0, dn2 = dn1 - 1.0;
+    const double inv_n = __drcp_rn(dn), inv_n1 = clk.inv_dn;
+    r.up = g.up; r.ndown = g.ndown;
+    r.inv_n = inv_n; r.inv_n1 = inv_n1;
+    r.shrink = dn1 * inv_n; r.decay = dn2 * inv_n1; r.grow = dn * inv_n1;
+    r.pad = 0.0;
+}
+
 template <class L, bool STRICT>
-__device__ __forceinline__ void measure_update(Chain<L> &c, Stats<L> &s, long long n, MeasureClock *clk = nullptr) {
+__device__ __forceinline__ void measure_update(Chain<L> &c, Stats<L> &s, long long n, const MeasureRow *row = nullptr) {
     constexpr int NR = L::NR, NC = L::NC;
-    double dn, dn1, dn2, inv_n, inv_n1;
-    if (!STRICT && clk != nullptr) {          /* clk holds the counter before this measure (n - 1) */
-        dn1 = clk->dn; inv_n1 = clk->inv_dn;
-        dn = dn1 + 1.0; dn2 = dn1 - 1.0;
-        inv_n = __drcp_rn(dn);
-        clk->dn = dn; clk->inv_dn = inv_n;
+    double dn = 0.0, dn1 = 0.0, inv_n, inv_n1, shrink, decay, grow;
+    if (!STRICT && row != nullptr) {          /* the row of the period this measure ends (counter n - 1 -> n) */
+        inv_n = row->inv_n; inv_n1 = row->inv_n1;
+        shrink = row->shrink; decay = row->decay; grow = row->grow;
     } else {
-        dn = (double)n; dn1 = (double)(n - 1); dn2 = (double)(n - 2);
+        dn = (double)n; dn1 = (double)(n - 1);
+        const double dn2 = (double)(n - 2);
         /* throughput build: two reciprocals per measure instead of a division per element */
         inv_n = STRICT ? 1.0 / dn : __drcp_rn(dn); inv_n1 = STRICT ? 1.0 / dn1 : __drcp_rn(dn1);
+        shrink = STRICT ? dn1 / dn : dn1 * inv_n;
+        decay = STRICT ? dn2 / dn1 : dn2 * inv_n1;
+        grow = STRICT ? dn / dn1 : dn * inv_n1;
     }
-    const double shrink = STRICT ? dn1 / dn : dn1 * inv_n;
     const bool adapt_cov = n > 50;
-    const double decay = STRICT ? dn2 / dn1 : dn2 * inv_n1, grow = STRICT ? dn / dn1 : dn * inv_n1;
     if (NR > 0) {
         double old[nz(NR)];
 #pragma unroll
@@ -810,9 +839,9 @@ __device__ __forceinline__ void pool_mma_update(const Chain<L> &c, const double 
  * (ME:253-257) -> width adaptation (ME:258 / group variants ME:440-456). */
 template <class Cfg, class Tab = LogTabGlobal>
 __device__ __forceinline__ bool finish_step(Chain<Lay<Cfg::NR, Cfg::NC>> &c, double (&prop)[Lay<Cfg::NR, Cfg::NC>::D],
-                                            double u, const Gains &g, const MeParams &p, const MathTables &tables,
-                                            int group, double uhi = 0.0, const Rng *rng = nullptr, unsigned step = 0u,
-                                            const Tab *logtab = nullptr, double half_temp = 0.0) {
+                                            const Draws<Lay<Cfg::NR, Cfg::NC>> &d, const Gains &g, const MeParams &p,
+                                            const MathTables &tables, int group, const Rng &rng, unsigned step,
+                                            const Tab &logtab) {
     using L = Lay<Cfg::NR, Cfg::NC>;
     using Energy = typename Cfg::Energy;
     constexpr bool STRICT = Cfg::STRICT;
@@ -826,39 +855,49 @@ __device__ __forceinline__ bool finish_step(Chain<Lay<Cfg::NR, Cfg::NC>> &c, dou
     }
     bool accept = false;
     const bool wall = p.use_reject && Energy::reject(prop, prop + L::NR, prop + L::NR + L::NC, p.consts);
-    if (!wall) {
-        const double e_new = Energy::eval(prop, prop + L::NR, prop + L::NR + L::NC, p.consts);
-        if (e_new != e_new) c.status |= ME_STATUS_ENERGY_NAN;
-        const double diff = e_new - c.e;
-        accept = decide<STRICT>(diff, u, p, tables, g.hot, g.k64);
-        if (!STRICT && rng != nullptr) {
-            /* inside the FP32 window (about 2 steps in 10^5): the exact threshold from the same random bits.  The branch
-               is taken by the whole (converged part of the) warp on a vote, so the common path stays straight-line code
-               that the compiler can interleave with the draw stages of the following steps */
-            const bool inside = !accept && diff <= uhi;
-            if (__any_sync(__activemask(), inside)) {
-                Spare sp;
-                if (ShareCall<L>::value) sp = share_spare(rng->bits(step >> 1, 0u), step);
-                else Rng::keep_spare(rng->bits(step, 0u), 0, sp);
-                const double thr = Rng::accept_threshold(sp, *logtab, half_temp);
-                accept = accept | (inside & (diff <= thr));
-            }
-        }
-        if (STRICT) {
+    if (STRICT) {
+        if (!wall) {
+            const double e_new = Energy::eval(prop, prop + L::NR, prop + L::NR + L::NC, p.consts);
+            if (e_new != e_new) c.status |= ME_STATUS_ENERGY_NAN;
+            accept = decide<STRICT>(e_new - c.e, d.u, p, tables, g.hot, g.k64);
             if (accept) {
                 c.e = e_new;
 #pragma unroll
                 for (int i = 0; i < D; i++) c.x[i] = prop[i];
                 c.nacc_new += 1u;
             }
-        } else {
-            /* throughput build: selects, not a divergent branch — a reconvergence region in the middle of the step would
-               stop the compiler from interleaving the state update with the draw stages of the following steps */
-            c.e = accept ? e_new : c.e;
-#pragma unroll
-            for (int i = 0; i < D; i++) c.x[i] = accept ? prop[i] : c.x[i];
-            c.nacc_new += accept ? 1u : 0u;
         }
+    } else {
+        /* throughput build: dE against the FP32 window (Rng::accept_window).  The comparison stays in FP64: deciding on
+           FP32(dE) instead was measured slower on the B200 (C2: 41.2 against 40.1 ms per pass), the conversion sits on
+           the step's dependent chain */
+        double e_new = 0.0, diff = 0.0;
+        bool inside = false;
+        if (!wall) {
+            e_new = Energy::eval(prop, prop + L::NR, prop + L::NR + L::NC, p.consts);
+            diff = e_new - c.e;
+            accept = diff <= (double)d.lo;
+            inside = !accept && !(diff > (double)d.hi);
+        }
+        /* inside the window (about 2 steps in 10^5) or NaN: the exact threshold from the same random bits.  The branch
+           is taken by the whole warp on a vote, so the common path stays straight-line code that the compiler can
+           interleave with the draw stages of the following steps.  The warp is converged here: the step loop has
+           uniform trip counts, lanes without a chain run it too, and the vote sits outside the wall's branch. */
+        if (__any_sync(ME_FULL, inside)) {
+            /* a NaN energy gives a NaN dE, which is always inside: the status bit needs no test on the common path */
+            if (inside && e_new != e_new) c.status |= ME_STATUS_ENERGY_NAN;
+            Spare sp;
+            if (ShareCall<L>::value) sp = share_spare(rng.bits(step >> 1, 0u), step);
+            else Rng::keep_spare(rng.bits(step, 0u), 0, sp);
+            const double thr = Rng::accept_threshold(sp, logtab, 0.5 * p.temp);
+            accept = accept | (inside & (diff <= thr));
+        }
+        /* selects, not a divergent branch — a reconvergence region in the middle of the step would stop the compiler from
+           interleaving the state update with the draw stages of the following steps */
+        c.e = accept ? e_new : c.e;
+#pragma unroll
+        for (int i = 0; i < D; i++) c.x[i] = accept ? prop[i] : c.x[i];
+        c.nacc_new += accept ? 1u : 0u;
     }
     if (L::NC > 0 && group == 4) {
         /* phase redraw: no width adapts, on the wall or otherwise (ME:194-207) */
@@ -1017,7 +1056,6 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     Draws<L> cur;
     Raw<L> raw_a, raw_b;
     const Pins pins = load_pins(tables);
-    const double half_temp = 0.5 * p.temp;
     /* log table: read-only global path for small shapes, per-CTA shared copy for larger ones (see me_math.cuh) */
     /* static shared-memory budget (48 KB): the pooled-moment staging of a large shape (9 x POOLW doubles, up to 43 KB at
        ME_MAX_POOLW) and the 16 KB table copy do not both fit; such shapes read the table through the read-only path */
@@ -1034,7 +1072,7 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     typedef typename TabSelect<TAB_SMEM>::type Tab;
     const Tab logtab{TAB_SMEM ? logtab_s : reinterpret_cast<const double2 *>(p.logtab)};
     if (!inject && p.spm > 0 && AHEAD) {
-        gen_draws<L, STRICT, Tab>(rng, step_first, tables, cur, pins, half_temp, logtab);
+        gen_draws<L, STRICT, Tab>(rng, step_first, tables, cur, pins, p, logtab);
         if (DEEP) gen_bits<L>(rng, step_first + 1u, raw_a);
     }
 
@@ -1058,15 +1096,15 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
                     take_second_half<L>(use, make);
                 } else {                             /* next step opens the pair whose bits are waiting; step + 2 shares it */
                     raw_out = raw_in;
-                    shape_pair<L, STRICT, Tab>(raw_in, tables, make, pins, half_temp, logtab);
+                    shape_pair<L, STRICT, Tab>(raw_in, tables, make, pins, p, logtab);
                 }
             } else if (DEEP) {
                 gen_bits<L>(rng, step32 + 2u, raw_out);
-                shape_draws<L, STRICT, Tab>(raw_in, tables, make, pins, half_temp, logtab);
+                shape_draws<L, STRICT, Tab>(raw_in, tables, make, pins, p, logtab);
             } else if (AHEAD) {
-                gen_draws<L, STRICT, Tab>(rng, step32 + 1u, tables, make, pins, half_temp, logtab);
+                gen_draws<L, STRICT, Tab>(rng, step32 + 1u, tables, make, pins, p, logtab);
             } else {
-                gen_draws<L, STRICT, Tab>(rng, step32, tables, use, pins, half_temp, logtab);
+                gen_draws<L, STRICT, Tab>(rng, step32, tables, use, pins, p, logtab);
             }
             apply_proposal<L>(c, use.z, prop);
             if (MP && L::NC > 0 && group >= 3) {
@@ -1074,82 +1112,99 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
                 else propose_phases<L>(c, rng, step32, prop);
             }
         }
-        accept = finish_step<Cfg, Tab>(c, prop, use.u, g, p, tables, group, use.uhi, inject ? nullptr : &rng, step32,
-                                       &logtab, half_temp);
+        accept = finish_step<Cfg, Tab>(c, prop, use, g, p, tables, group, rng, step32, logtab);
         step32++;
     };
     const unsigned spm = (unsigned)p.spm;
-    MeasureClock clk;
-    clk.start(n);
     /* running row pointer of the time series (one 64-bit add per measure instead of the full index arithmetic) */
     double *row = p.record ? p.ts + (p.ts_row0 + b_first) * (long long)L::TSCOLS * ld + ch : nullptr;
     const long long row_stride = (long long)L::TSCOLS * ld;
 
-    for (long long b = 0; b < n_blocks; b++) {
-        Gains g = make_gains<!STRICT>(n, p, clk.inv_dn);
-        g.k64 = pins.k64;
-        /* steps in pairs so that the two draw buffers swap roles by name instead of by register moves */
-        Draws<L> nxt;
-        unsigned k = 0;
-        if (ME_PAIR_BIG || DEEP) {
-            for (; k + 1 < spm; k += 2) {
-                one_step(g, cur, nxt, raw_a, raw_b);
-                one_step(g, nxt, cur, raw_b, raw_a);
-            }
-            if (k < spm) {
-                one_step(g, cur, nxt, raw_a, raw_b);
-                if (!inject) { cur = nxt; if (DEEP) raw_a = raw_b; }
-            }
-        } else {
-            /* larger shapes: one step per iteration (the pair-unrolled loop of a 3r+4c shape is 27 KB of code) */
-#pragma unroll 1
-            for (; k < spm; k++) {
-                one_step(g, cur, nxt, raw_a, raw_b);
-                if (!inject && AHEAD) cur = nxt;
-            }
+    /* per-measure values (MeasureRow) from a per-CTA table, a chunk of periods at a time; larger shapes (254 registers)
+       keep computing them per thread, the loop nest would cost them spills */
+    constexpr bool MTAB = !STRICT && SEGMENTED;
+    constexpr int MCHUNK = 32;
+    __shared__ MeasureRow mrow[MTAB ? MCHUNK : 1];
+    for (long long b0 = 0; b0 < n_blocks; b0 += MCHUNK) {
+        const int nb = n_blocks - b0 < MCHUNK ? (int)(n_blocks - b0) : MCHUNK;
+        if (MTAB) {
+            __syncthreads();                   /* every thread is done with the previous chunk */
+            for (int j = threadIdx.x; j < nb; j += blockDim.x) fill_measure_row(n + (p.do_measure ? j : 0), p, mrow[j]);
+            __syncthreads();
         }
-        if (p.do_measure) {
-            n += 1;
-            if (STATS_REG) {
-                measure_update<L, STRICT>(c, sreg, n, &clk);
+        for (int j = 0; j < nb; j++) {
+            Gains g;
+            if (!MTAB) {
+                g = make_gains<!STRICT>(n, p, STRICT ? 0.0 : __drcp_rn((double)n));
             } else {
-                Stats<L> s;
-                load_stats<L>(s, st, ld, ch);
-                measure_update<L, STRICT>(c, s, n, &clk);
-                if (active) store_stats<L>(s, st, ld, ch);
+                g = Gains{};
+                g.up = mrow[j].up;
+                g.ndown = mrow[j].ndown;
             }
-            if (p.record && active) {
-#pragma unroll
-                for (int i = 0; i < D; i++) __stcs(row + (long long)i * ld, c.x[i]);
-                __stcs(row + (long long)D * ld, c.e);
-                if (L::KIND == 0) {
-                    __stcs(row + (long long)(D + 1) * ld, c.sig[0]);
-                    __stcs(row + (long long)(D + 2) * ld, c.sig[1]);
-                } else {
-                    __stcs(row + (long long)(D + 1) * ld, c.sig[L::SIGIDX]);
+            g.k64 = pins.k64;
+            /* steps in pairs so that the two draw buffers swap roles by name instead of by register moves */
+            Draws<L> nxt;
+            unsigned k = 0;
+            if (ME_PAIR_BIG || DEEP) {
+                for (; k + 1 < spm; k += 2) {
+                    one_step(g, cur, nxt, raw_a, raw_b);
+                    one_step(g, nxt, cur, raw_b, raw_a);
+                }
+                if (k < spm) {
+                    one_step(g, cur, nxt, raw_a, raw_b);
+                    if (!inject) { cur = nxt; if (DEEP) raw_a = raw_b; }
+                }
+            } else {
+                /* larger shapes: one step per iteration (the pair-unrolled loop of a 3r+4c shape is 27 KB of code) */
+#pragma unroll 1
+                for (; k < spm; k++) {
+                    one_step(g, cur, nxt, raw_a, raw_b);
+                    if (!inject && AHEAD) cur = nxt;
                 }
             }
-            if (p.record) row += row_stride;
-            if (pooling) {
-                if (POOL_REG) {
-for_each_pool_word<L>(c, shift, [&](int w, double v) { pacc[w] += v; });
-                } else if (POOL_MMA) {
-                    const int warp = threadIdx.x >> 5;
-                    pool_mma_update<L, !STRICT>(c, shift, active, ybuf[warp], pool_warp[warp]);
+            if (p.do_measure) {
+                n += 1;
+                if (STATS_REG) {
+                    measure_update<L, STRICT>(c, sreg, n, MTAB ? &mrow[j] : nullptr);
                 } else {
-                    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-                    for_each_pool_word<L>(c, shift, [&](int w, double v) {
-                        v = warp_sum(active ? v : 0.0);
-                        if (lane == 0) pool_warp[warp][w] = v;
-                    });
-                    __syncthreads();
-                    const int nw = (blockDim.x + 31) >> 5;
-                    for (int w = threadIdx.x; w < L::POOLW; w += blockDim.x) {
-                        double t = 0.0;
-                        for (int q = 0; q < nw; q++) t += pool_warp[q][w];
-                        pool_cta[w] += t;
+                    Stats<L> s;
+                    load_stats<L>(s, st, ld, ch);
+                    measure_update<L, STRICT>(c, s, n, MTAB ? &mrow[j] : nullptr);
+                    if (active) store_stats<L>(s, st, ld, ch);
+                }
+                if (p.record && active) {
+#pragma unroll
+                    for (int i = 0; i < D; i++) __stcs(row + (long long)i * ld, c.x[i]);
+                    __stcs(row + (long long)D * ld, c.e);
+                    if (L::KIND == 0) {
+                        __stcs(row + (long long)(D + 1) * ld, c.sig[0]);
+                        __stcs(row + (long long)(D + 2) * ld, c.sig[1]);
+                    } else {
+                        __stcs(row + (long long)(D + 1) * ld, c.sig[L::SIGIDX]);
                     }
-                    __syncthreads();
+                }
+                if (p.record) row += row_stride;
+                if (pooling) {
+                    if (POOL_REG) {
+                        for_each_pool_word<L>(c, shift, [&](int w, double v) { pacc[w] += v; });
+                    } else if (POOL_MMA) {
+                        const int warp = threadIdx.x >> 5;
+                        pool_mma_update<L, !STRICT>(c, shift, active, ybuf[warp], pool_warp[warp]);
+                    } else {
+                        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+                        for_each_pool_word<L>(c, shift, [&](int w, double v) {
+                            v = warp_sum(active ? v : 0.0);
+                            if (lane == 0) pool_warp[warp][w] = v;
+                        });
+                        __syncthreads();
+                        const int nw = (blockDim.x + 31) >> 5;
+                        for (int w = threadIdx.x; w < L::POOLW; w += blockDim.x) {
+                            double t = 0.0;
+                            for (int q = 0; q < nw; q++) t += pool_warp[q][w];
+                            pool_cta[w] += t;
+                        }
+                        __syncthreads();
+                    }
                 }
             }
         }
@@ -1266,7 +1321,7 @@ __device__ __forceinline__ void propose_body(const MeParams &p) {
         const Rng rng(p, p.chain_offset + (unsigned long long)ch);
         Draws<L> d;
         const unsigned step = p.ctr_dev ? (unsigned)p.ctr_dev[0] : (unsigned)p.step0;
-        gen_draws<L, Cfg::STRICT, LogTabGlobal>(rng, step, tables, d, load_pins(tables), 0.5 * p.temp,
+        gen_draws<L, Cfg::STRICT, LogTabGlobal>(rng, step, tables, d, load_pins(tables), p,
                                                 LogTabGlobal{reinterpret_cast<const double2 *>(p.logtab)});
         apply_proposal<L>(c, d.z, prop);
         if (L::NC > 0 && p.group >= 3) {

@@ -5,7 +5,7 @@
 #ifndef ME_PARAMS_H
 #define ME_PARAMS_H
 
-#define ME_PARAMS_VERSION 9
+#define ME_PARAMS_VERSION 10
 #define ME_MAX_CONSTS 16
 
 /* status bits written to the per-chain STATUS word (SURVEY §5 "failure detection") */
@@ -29,6 +29,8 @@ struct MeParams {
     int m;                         /* n_real + n_complex (ME:103) */
     int record;                    /* 1: store a time-series row at every measure */
     double temp, inv_temp;
+    float t_ln2, t_band;           /* throughput build's FP32 threshold window (me_device.cuh, Rng::accept_window): T ln2 and
+                                      the half-width 4e-5 T, see me_api.cu base_params */
     double target;                 /* target acceptance p* (ME:101) */
     double ratio;                  /* ME:105-107 */
     double consts[ME_MAX_CONSTS];  /* energy-functor constants */
