@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define ME_ABI_VERSION 5
+#define ME_ABI_VERSION 6
 
 enum me_status_code {
     ME_OK = 0,
@@ -138,7 +138,20 @@ int me_device_counters(me_engine *eng, int32_t enable, void *stream);
  * block of the records of groups 3 / 4 holds the ABSOLUTE proposed values, not increments. */
 int me_set_group(me_engine *eng, int32_t group);
 
-/* Launch geometry the handle uses; the pool buffer has grid * POOL_WORDS doubles. */
+/* Temperature ladder (parallel tempering).  Global chain g runs at temps[g % n_rungs]; the handle's chains must be whole
+ * ladders (chain_offset and n_chains multiples of n_rungs).  swap_every > 0: replica exchange — at every measure whose
+ * counter is a multiple of swap_every, neighbour rungs (deterministic even/odd pairing) swap configurations, energies and
+ * walker labels with probability min(1, exp((1/T_lo - 1/T_hi)(E_lo - E_hi))); then n_rungs is 2, 4, 8, 16 or 32 and the
+ * temperatures are finite, > 0 and strictly increasing.  swap_every = 0: a temperature sweep, any n_rungs >= 2, temps >= 0.
+ * walker[n_chains] (device, int32) holds each chain's walker label, swap_acc[n_chains] (device, uint32) the accepted swaps
+ * between the chain's rung and the next one up; both are read and written by me_run.  Fused shapes (D <= 32) with a device
+ * functor, group 0, Philox draws only.  Call before me_bind: it may change the launch geometry, and the pool buffer of a
+ * ladder with a power-of-two n_rungs <= 32 holds n_rungs rows of POOL_WORDS per CTA (rung-major), other ladders pool
+ * nothing.  The temperatures are copied. */
+int me_set_ladder(me_engine *eng, const double *temps, int32_t n_rungs, int64_t swap_every, int32_t *walker,
+                  uint32_t *swap_acc);
+
+/* Launch geometry the handle uses; the pool buffer has grid * POOL_WORDS doubles (see me_set_ladder for ladders). */
 int me_launch_dims(me_engine *eng, int32_t *grid, int32_t *block);
 
 typedef struct me_buffers {

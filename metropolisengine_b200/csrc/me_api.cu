@@ -42,7 +42,7 @@ struct KernelRef {
     bool valid() const { return rt != nullptr || drv != nullptr; }
 };
 struct KernelSet {
-    KernelRef run, init, propose, accept, energy, run_mp;
+    KernelRef run, init, propose, accept, energy, run_mp, run_pt;
     bool valid() const { return run.valid(); }
 };
 
@@ -179,6 +179,11 @@ int nvrtc_compile(int n_real, int n_complex, int energy_id, const std::string &u
            "extern \"C\" __global__ void __maxnreg__(160) me_k_run(const __grid_constant__ MeParams p) { me::run_body<UserCfg>(p); }\n"
            "#else\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run(const __grid_constant__ MeParams p) { me::run_body<UserCfg>(p); }\n"
+           "#endif\n"
+           "#if ME_NR + 2 * ME_NC <= 4\n"
+           "extern \"C\" __global__ void __maxnreg__(160) me_k_run_pt(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, true>(p); }\n"
+           "#else\n"
+           "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run_pt(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, true>(p); }\n"
            "#endif\n"
            "#if ME_NC > 0\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run_mp(const __grid_constant__ MeParams p) { me::run_body<UserCfg, true>(p); }\n"
@@ -345,6 +350,13 @@ struct me_engine {
     double *pool_partial = nullptr;            /* first-stage rows of the pooled-moment reduction (large ensembles) */
     unsigned long long *ctr_dev = nullptr;     /* device copy of (step, n_measure) for CUDA-graph replay of the unfused step */
     bool use_ctr = false;
+    /* temperature ladder (me_set_ladder): n_rungs > 1 runs the PT instantiation of the fused kernel */
+    int n_rungs = 1;
+    long long swap_every = 0;
+    void *ladder_dev = nullptr;                /* rung temperatures [R] (double), then the FP32 windows [R][2] */
+    int *walker = nullptr;
+    unsigned *swap_acc = nullptr;
+    int pool_rungs = 1;                        /* rows of POOL_WORDS per CTA in the pool buffer: R for a ladder that pools */
     std::string err;
 };
 
@@ -418,6 +430,25 @@ const double *log_table(int device) {
     return dev;
 }
 
+/* FP32 window of the throughput build's Metropolis test (me_device.cuh, Rng::accept_window).  Its error budget is
+   relative to T and holds while T ln2 and 4e-5 T are normal floats far from overflow, i.e. for 1e-30 <= T <= 1e30.
+   T = 0: the half-width is the smallest denormal, so that the window is [-2^-149, 2^-149] and a dE that rounds to
+   +-0 in FP32 takes the exact test.  Any other T: an infinite half-width sends every decision to the exact test. */
+void accept_window_consts(double t, float &t_ln2, float &t_band) {
+    if (t == 0) {
+        t_ln2 = 0.0f;
+        t_band = 0x1p-149f;
+    } else if (t >= 1e-30 && t <= 1e30) {
+        t_ln2 = (float)(t * 0.69314718055994531);
+        t_band = (float)(t * 4e-5);
+    } else {
+        t_ln2 = 0.0f;
+        t_band = HUGE_VALF;
+    }
+}
+
+int pool_words(const me_engine *e) { return e->lay.POOL_WORDS * e->pool_rungs; }
+
 void base_params(me_engine *e, MeParams &p) {
     memset(&p, 0, sizeof(p));
     p.logtab = e->logtab;
@@ -437,21 +468,7 @@ void base_params(me_engine *e, MeParams &p) {
     p.m = e->cfg.n_real + e->cfg.n_complex;
     p.temp = e->cfg.temp;
     p.inv_temp = e->cfg.temp != 0 ? 1.0 / e->cfg.temp : 0.0;
-    /* FP32 window of the throughput build's Metropolis test (me_device.cuh, Rng::accept_window).  Its error budget is
-       relative to T and holds while T ln2 and 4e-5 T are normal floats far from overflow, i.e. for 1e-30 <= T <= 1e30.
-       T = 0: the half-width is the smallest denormal, so that the window is [-2^-149, 2^-149] and a dE that rounds to
-       +-0 in FP32 takes the exact test.  Any other T: an infinite half-width sends every decision to the exact test. */
-    const double t = e->cfg.temp;
-    if (t == 0) {
-        p.t_ln2 = 0.0f;
-        p.t_band = 0x1p-149f;
-    } else if (t >= 1e-30 && t <= 1e30) {
-        p.t_ln2 = (float)(t * 0.69314718055994531);
-        p.t_band = (float)(t * 4e-5);
-    } else {
-        p.t_ln2 = 0.0f;
-        p.t_band = HUGE_VALF;
-    }
+    accept_window_consts(e->cfg.temp, p.t_ln2, p.t_band);
     p.target = e->cfg.target_acceptance;
     p.ratio = e->cfg.ratio;
     memcpy(p.consts, e->consts, sizeof(p.consts));
@@ -464,6 +481,15 @@ void base_params(me_engine *e, MeParams &p) {
     p.scratch = e->buf.scratch;
     p.prop = e->buf.prop;
     p.group = e->group;
+    if (e->n_rungs > 1) {
+        p.n_rungs = e->n_rungs;
+        p.swap_every = e->swap_every;
+        p.rung_temp = static_cast<const double *>(e->ladder_dev);
+        p.rung_window = reinterpret_cast<const float *>(p.rung_temp + e->n_rungs);
+        p.walker = e->walker;
+        p.swap_acc = e->swap_acc;
+        if (e->pool_rungs != e->n_rungs) p.pool = nullptr;      /* a ladder that does not fit a warp pools nothing */
+    }
 }
 
 /* Time segmentation of a fused launch (me_device.cuh, run_body): when the whole grid is resident in one wave the
@@ -610,6 +636,7 @@ int resolve_kernels(me_engine *e, int energy_id, const std::string &user_src) {
             if (t[i].n_real == nr && t[i].n_complex == nc && t[i].energy_id == energy_id) {
                 e->ks.run.rt = t[i].run; e->ks.init.rt = t[i].init; e->ks.run_mp.rt = t[i].run_mp;
                 e->ks.propose.rt = t[i].propose; e->ks.accept.rt = t[i].accept; e->ks.energy.rt = t[i].energy;
+                e->ks.run_pt.rt = t[i].run_pt;
                 return ME_OK;
             }
     }
@@ -641,6 +668,7 @@ int resolve_kernels(me_engine *e, int energy_id, const std::string &user_src) {
         d.moduleGetFunction(&ks.propose.drv, mod, "me_k_propose") != CUDA_SUCCESS ||
         d.moduleGetFunction(&ks.accept.drv, mod, "me_k_accept") != CUDA_SUCCESS ||
         d.moduleGetFunction(&ks.energy.drv, mod, "me_k_energy") != CUDA_SUCCESS ||
+        d.moduleGetFunction(&ks.run_pt.drv, mod, "me_k_run_pt") != CUDA_SUCCESS ||
         (e->cfg.n_complex > 0 && d.moduleGetFunction(&ks.run_mp.drv, mod, "me_k_run_mp") != CUDA_SUCCESS))
         return fail(e, ME_ERR_CUDA, "cuModuleGetFunction failed on the runtime-compiled module");
     g_cache[key] = ks;
@@ -870,8 +898,9 @@ int me_create(const me_config *cfg, me_engine **out) {
 }
 
 int me_destroy(me_engine *e) {
-    if (e && (e->seg_flags || e->ctr_dev || e->pool_partial)) {
+    if (e && (e->seg_flags || e->ctr_dev || e->pool_partial || e->ladder_dev)) {
         DeviceGuard g(e->cfg.device);
+        if (e->ladder_dev) cudaFree(e->ladder_dev);
         if (e->seg_flags) cudaFree(e->seg_flags);
         if (e->ctr_dev) cudaFree(e->ctr_dev);
         if (e->pool_partial) cudaFree(e->pool_partial);
@@ -929,6 +958,59 @@ int me_set_group(me_engine *e, int32_t group) {
     if (group == 1 && e->cfg.n_real == 0) return fail(e, ME_ERR_INVALID, "engine has no real parameters");
     if (group >= 2 && e->cfg.n_complex == 0) return fail(e, ME_ERR_INVALID, "engine has no complex parameters");
     e->group = group;
+    return ME_OK;
+}
+
+int me_set_ladder(me_engine *e, const double *temps, int32_t n_rungs, int64_t swap_every, int32_t *walker,
+                  uint32_t *swap_acc) {
+    if (!e) return ME_ERR_INVALID;
+    if (e->bound) return fail(e, ME_ERR_STATE, "me_set_ladder comes before me_bind (it sets the launch geometry)");
+    if (e->generic) return fail(e, ME_ERR_UNSUPPORTED, "temperature ladders need a fused shape (n_real + 2 n_complex <= 32)");
+    if (!temps || !walker || !swap_acc) return fail(e, ME_ERR_INVALID, "temps, walker and swap_acc are required");
+    if (n_rungs < 2) return fail(e, ME_ERR_INVALID, "a ladder has at least 2 rungs");
+    if (swap_every < 0) return fail(e, ME_ERR_INVALID, "swap_every must be >= 0");
+    const long long R = n_rungs;
+    if (e->cfg.chain_offset % R != 0 || e->cfg.n_chains % R != 0)
+        return fail(e, ME_ERR_INVALID, "the chains of a handle must be whole ladders: chain_offset and n_chains multiples of " +
+                                           std::to_string(R));
+    const bool pow2 = n_rungs <= 32 && (n_rungs & (n_rungs - 1)) == 0;
+    if (swap_every > 0 && !pow2) return fail(e, ME_ERR_INVALID, "replica exchange needs 2, 4, 8, 16 or 32 rungs");
+    for (int r = 0; r < n_rungs; r++) {
+        if (!std::isfinite(temps[r]) || temps[r] < 0)
+            return fail(e, ME_ERR_INVALID, "ladder temperatures must be finite and >= 0");
+        if (swap_every > 0 && !(temps[r] > 0))
+            return fail(e, ME_ERR_INVALID, "replica exchange needs temperatures > 0");
+        if (swap_every > 0 && r > 0 && !(temps[r] > temps[r - 1]))
+            return fail(e, ME_ERR_INVALID, "replica exchange needs strictly increasing temperatures");
+    }
+    std::vector<char> host(sizeof(double) * R + sizeof(float) * 2 * R);
+    double *t = reinterpret_cast<double *>(host.data());
+    float *win = reinterpret_cast<float *>(t + R);
+    for (int r = 0; r < n_rungs; r++) {
+        t[r] = temps[r];
+        accept_window_consts(temps[r], win[2 * r], win[2 * r + 1]);
+    }
+    DeviceGuard g(e->cfg.device);
+    if (e->ladder_dev) { cudaFree(e->ladder_dev); e->ladder_dev = nullptr; }
+    if (cudaMalloc(&e->ladder_dev, host.size()) != cudaSuccess ||
+        cudaMemcpy(e->ladder_dev, host.data(), host.size(), cudaMemcpyHostToDevice) != cudaSuccess) {
+        cudaGetLastError();
+        if (e->ladder_dev) cudaFree(e->ladder_dev);
+        e->ladder_dev = nullptr;
+        return fail(e, ME_ERR_CUDA, "allocating the ladder failed");
+    }
+    e->n_rungs = n_rungs;
+    e->swap_every = swap_every;
+    e->walker = walker;
+    e->swap_acc = reinterpret_cast<unsigned *>(swap_acc);
+    /* pooled moments per rung need the ladder inside a warp (me_device.cuh, run_body PT); shapes that do not pool in
+       registers add the rung sums of every measure straight into their CTA's rows, so their CTAs are one warp */
+    e->pool_rungs = pow2 ? n_rungs : 0;
+    if (pow2 && e->lay.POOL_WORDS > ME_POOL_REG_MAX) {
+        e->block = 32;
+        e->grid = (int)((e->cfg.n_chains + 31) / 32);
+    }
+    e->run_slots = -1;
     return ME_OK;
 }
 
@@ -991,7 +1073,11 @@ static int run_common(me_engine *e, int64_t n_blocks, int64_t spm, int do_measur
     p.inj_delta = delta; p.inj_u = u;
     if (e->group >= 3 && !e->ks.run_mp.valid())
         return fail(e, ME_ERR_STATE, "no magnitude-phase kernel for this engine");
-    const KernelRef &kr = e->group >= 3 ? e->ks.run_mp : e->ks.run;
+    if (e->n_rungs > 1 && (e->group != 0 || delta != nullptr))
+        return fail(e, ME_ERR_UNSUPPORTED, "temperature ladders step all parameters with Philox draws only");
+    if (e->n_rungs > 1 && !e->ks.run_pt.valid())
+        return fail(e, ME_ERR_STATE, "no ladder kernel for this engine (device functors only)");
+    const KernelRef &kr = e->n_rungs > 1 ? e->ks.run_pt : (e->group >= 3 ? e->ks.run_mp : e->ks.run);
     const int segs = plan_segments(e, kr, n_blocks, spm, delta != nullptr, stream);
     if (segs < 0) return ME_ERR_CUDA;
     if (segs > 1) {
@@ -1027,6 +1113,7 @@ int me_propose(me_engine *e, double *prop, const double *inj_delta, void *stream
     if (!e->bound) return fail(e, ME_ERR_STATE, "me_bind first");
     if (!prop) return fail(e, ME_ERR_INVALID, "prop is required");
     if (inj_delta && !e->cfg.strict) return fail(e, ME_ERR_STATE, "draw injection needs a strict handle");
+    if (e->n_rungs > 1) return fail(e, ME_ERR_UNSUPPORTED, "temperature ladders step fused only (me_run)");
     MeParams p;
     base_params(e, p);
     p.prop = prop; p.inj_delta = inj_delta;
@@ -1039,6 +1126,7 @@ int me_accept(me_engine *e, const double *prop, const double *e_new, const unsig
     if (!e->bound) return fail(e, ME_ERR_STATE, "me_bind first");
     if (!prop || !e_new) return fail(e, ME_ERR_INVALID, "prop and e_new are required");
     if (inj_u && !e->cfg.strict) return fail(e, ME_ERR_STATE, "draw injection needs a strict handle");
+    if (e->n_rungs > 1) return fail(e, ME_ERR_UNSUPPORTED, "temperature ladders step fused only (me_run)");
     if (e->step + 1ull >= 0xffffffffull) return fail(e, ME_ERR_INVALID, "step index exceeds the 32-bit Philox counter word");
     MeParams p;
     base_params(e, p);
@@ -1083,9 +1171,9 @@ int me_energy_builtin(me_engine *e, const double *prop, double *e_out, unsigned 
 
 int me_pool_reduce(me_engine *e, double *out, int32_t reset, void *stream) {
     if (!e || !out) return ME_ERR_INVALID;
-    if (!e->bound || !e->buf.pool || e->lay.POOL_WORDS == 0) return fail(e, ME_ERR_STATE, "no pool buffer bound");
+    if (!e->bound || !e->buf.pool || pool_words(e) == 0) return fail(e, ME_ERR_STATE, "no pool buffer bound");
     DeviceGuard g(e->cfg.device);
-    const int words = e->lay.POOL_WORDS;
+    const int words = pool_words(e);
     if (e->grid > 4096 && words <= 256) {
         /* millions of rows: coalesced first stage into ME_POOL_STAGE_CTAS partial rows, then the fixed-order tree */
         if (!e->pool_partial &&
@@ -1427,9 +1515,9 @@ const char *me_comm_last_error(void) { return g_comm_error.c_str(); }
 /* first half of me_allreduce_stats: inc = fixed-order sum of the per-CTA accumulators (which are reset) | n_samples */
 int me_reduce_stats(me_engine *e, double *inc, int64_t n_samples, void *stream) {
     if (!e || !inc || n_samples < 0) return ME_ERR_INVALID;
-    if (!e->bound || !e->buf.pool || e->lay.POOL_WORDS == 0) return fail(e, ME_ERR_STATE, "no pool buffer bound");
+    if (!e->bound || !e->buf.pool || pool_words(e) == 0) return fail(e, ME_ERR_STATE, "no pool buffer bound");
     DeviceGuard g(e->cfg.device);
-    const int words = e->lay.POOL_WORDS;
+    const int words = pool_words(e);
     cudaStream_t st = (cudaStream_t)stream;
     if (e->grid > 4096 && words <= 256) {
         if (!e->pool_partial &&
@@ -1451,9 +1539,9 @@ int me_reduce_stats(me_engine *e, double *inc, int64_t n_samples, void *stream) 
    launches (ordered after me_reduce_stats by an event), so that the collective overlaps the next launch. */
 int me_accumulate_stats(me_engine *e, me_comm *comm, double *inc, double *totals, void *stream) {
     if (!e || !inc || !totals) return ME_ERR_INVALID;
-    if (e->lay.POOL_WORDS == 0) return fail(e, ME_ERR_STATE, "no pooled moments for this shape");
+    if (pool_words(e) == 0) return fail(e, ME_ERR_STATE, "no pooled moments for this shape");
     DeviceGuard g(e->cfg.device);
-    const int words = e->lay.POOL_WORDS;
+    const int words = pool_words(e);
     cudaStream_t st = (cudaStream_t)stream;
     if (comm && comm->world > 1) {
         std::string err;

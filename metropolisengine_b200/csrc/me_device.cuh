@@ -196,6 +196,14 @@ struct Rng {
     }
 };
 
+/* The temperature of a chain on a ladder (run_body's PT instantiation): its rung's T and FP32 window constants, loaded once
+ * per launch.  Functions that take `const LaneTemp *lt` use the launch's scalar temperature (MeParams::temp, t_ln2, t_band)
+ * when it is null, which is what every other instantiation passes. */
+struct LaneTemp {
+    double temp;
+    float t_ln2, t_band;
+};
+
 /* ------------------------------------------------------------------------------------------ per-chain registers */
 template <class L>
 struct Chain {
@@ -385,7 +393,8 @@ __device__ __forceinline__ void gen_bits(const Rng &rng, unsigned step, Raw<L> &
    (u2 | lo2, hi2) for the odd one */
 template <class L, bool STRICT, class Tab>
 __device__ __forceinline__ void shape_pair(const Raw<L> &raw, const MathTables &T, Draws<L> &d, const Pins &pins,
-                                           const MeParams &p, const Tab &logtab) {
+                                           const MeParams &p, const Tab &logtab, const LaneTemp *lt = nullptr) {
+    const float t_ln2 = lt ? lt->t_ln2 : p.t_ln2, t_band = lt ? lt->t_band : p.t_band;
     const U4 r = raw.r[0];
     Rng::box_muller<STRICT, Tab>(share_radius_bits(r), T, d.z[0], d.z[1], pins.unit, pins.angle, logtab);
     const Spare se = share_spare(r, 0u), so = share_spare(r, 1u);
@@ -393,8 +402,8 @@ __device__ __forceinline__ void shape_pair(const Raw<L> &raw, const MathTables &
         d.u = Rng::accept_uniform(se);
         d.u2 = Rng::accept_uniform(so);
     } else {
-        Rng::accept_window(se.w0, p.t_ln2, p.t_band, d.lo, d.hi);
-        Rng::accept_window(so.w0, p.t_ln2, p.t_band, d.lo2, d.hi2);
+        Rng::accept_window(se.w0, t_ln2, t_band, d.lo, d.hi);
+        Rng::accept_window(so.w0, t_ln2, t_band, d.lo2, d.hi2);
     }
 }
 /* the odd step of a pair takes over what the even step carried */
@@ -407,10 +416,11 @@ __device__ __forceinline__ void take_second_half(const Draws<L> &even, Draws<L> 
 
 template <class L, bool STRICT, class Tab>
 __device__ __forceinline__ void shape_draws(const Raw<L> &raw, const MathTables &T, Draws<L> &d, const Pins &pins,
-                                            const MeParams &p, const Tab &logtab, unsigned step = 0u) {
+                                            const MeParams &p, const Tab &logtab, unsigned step = 0u,
+                                            const LaneTemp *lt = nullptr) {
     constexpr int NQ = (L::D + 1) / 2;
     if (ShareCall<L>::value) {            /* stateless form: the draws of `step` from its pair's call */
-        shape_pair<L, STRICT, Tab>(raw, T, d, pins, p, logtab);
+        shape_pair<L, STRICT, Tab>(raw, T, d, pins, p, logtab, lt);
         if (step & 1u) { const Draws<L> e = d; take_second_half<L>(e, d); }
         return;
     }
@@ -423,17 +433,18 @@ __device__ __forceinline__ void shape_draws(const Raw<L> &raw, const MathTables 
     }
     /* strict build: the uniform itself; throughput build: a window around the energy threshold -T ln u */
     if (STRICT) d.u = Rng::accept_uniform(sp);
-    else Rng::accept_window(sp.w0, p.t_ln2, p.t_band, d.lo, d.hi);
+    else Rng::accept_window(sp.w0, lt ? lt->t_ln2 : p.t_ln2, lt ? lt->t_band : p.t_band, d.lo, d.hi);
     d.u2 = 0.0;
     d.lo2 = d.hi2 = 0.0f;
 }
 
 template <class L, bool STRICT, class Tab>
 __device__ __forceinline__ void gen_draws(const Rng &rng, unsigned step, const MathTables &T, Draws<L> &d,
-                                          const Pins &pins, const MeParams &p, const Tab &logtab) {
+                                          const Pins &pins, const MeParams &p, const Tab &logtab,
+                                          const LaneTemp *lt = nullptr) {
     Raw<L> raw;
     gen_bits<L>(rng, step, raw);
-    shape_draws<L, STRICT, Tab>(raw, T, d, pins, p, logtab, step);
+    shape_draws<L, STRICT, Tab>(raw, T, d, pins, p, logtab, step, lt);
 }
 
 template <class L>
@@ -548,11 +559,12 @@ __device__ __forceinline__ Gains make_gains(long long n_meas, const MeParams &p,
 /* Metropolis test (ME:319-338): ties accept; T == 0 rejects every uphill move; otherwise u <= exp(-1*diff/T). */
 template <bool STRICT>
 __device__ __forceinline__ bool decide(double diff, double u, const MeParams &p, const MathTables &T, bool hot,
-                                       const double k64 = ME_C_64_LN2) {
+                                       const double k64 = ME_C_64_LN2, const LaneTemp *lt = nullptr) {
     if (STRICT) {
+        const double temp = lt ? lt->temp : p.temp;
         if (diff <= 0) return true;
-        if (p.temp == 0) return false;
-        return u <= exp(-1 * diff / p.temp);
+        if (temp == 0) return false;
+        return u <= exp(-1 * diff / temp);
     }
     /* throughput build: `u` is the precomputed threshold -T ln u >= 0 (see the stream definition): one comparison;
        ties accept, NaN rejects, T == 0 accepts only dE <= 0 */
@@ -841,7 +853,7 @@ template <class Cfg, class Tab = LogTabGlobal>
 __device__ __forceinline__ bool finish_step(Chain<Lay<Cfg::NR, Cfg::NC>> &c, double (&prop)[Lay<Cfg::NR, Cfg::NC>::D],
                                             const Draws<Lay<Cfg::NR, Cfg::NC>> &d, const Gains &g, const MeParams &p,
                                             const MathTables &tables, int group, const Rng &rng, unsigned step,
-                                            const Tab &logtab) {
+                                            const Tab &logtab, const LaneTemp *lt = nullptr) {
     using L = Lay<Cfg::NR, Cfg::NC>;
     using Energy = typename Cfg::Energy;
     constexpr bool STRICT = Cfg::STRICT;
@@ -859,7 +871,7 @@ __device__ __forceinline__ bool finish_step(Chain<Lay<Cfg::NR, Cfg::NC>> &c, dou
         if (!wall) {
             const double e_new = Energy::eval(prop, prop + L::NR, prop + L::NR + L::NC, p.consts);
             if (e_new != e_new) c.status |= ME_STATUS_ENERGY_NAN;
-            accept = decide<STRICT>(e_new - c.e, d.u, p, tables, g.hot, g.k64);
+            accept = decide<STRICT>(e_new - c.e, d.u, p, tables, g.hot, g.k64, lt);
             if (accept) {
                 c.e = e_new;
 #pragma unroll
@@ -889,7 +901,7 @@ __device__ __forceinline__ bool finish_step(Chain<Lay<Cfg::NR, Cfg::NC>> &c, dou
             Spare sp;
             if (ShareCall<L>::value) sp = share_spare(rng.bits(step >> 1, 0u), step);
             else Rng::keep_spare(rng.bits(step, 0u), 0, sp);
-            const double thr = Rng::accept_threshold(sp, logtab, 0.5 * p.temp);
+            const double thr = Rng::accept_threshold(sp, logtab, 0.5 * (lt ? lt->temp : p.temp));
             accept = accept | (inside & (diff <= thr));
         }
         /* selects, not a divergent branch — a reconvergence region in the middle of the step would stop the compiler from
@@ -913,11 +925,77 @@ __device__ __forceinline__ bool finish_step(Chain<Lay<Cfg::NR, Cfg::NC>> &c, dou
     return accept;
 }
 
+/* ------------------------------------------------------------------------------------------ replica exchange
+ * Stream definition (identical in oracle/me_oracle_ladder.c, meo_run_ladder).  A ladder of R rungs (a power of two <= 32) lives in
+ * R consecutive lanes of a warp: global chain g is rung g % R.  Round k = n / swap_every, at a measure whose counter n (after
+ * its increment) is a multiple of swap_every, pairs rungs (r, r + 1) with r = k (mod 2) (deterministic even/odd).  With
+ * lo / hi the colder / hotter rung of a pair, the pair swaps iff  u <= exp((1/T_lo - 1/T_hi) (E_lo - E_hi)),  where u is
+ * built like the radius uniform, (K + 1/2) 2^-52 with K = y : x[31:12], from the Philox call with counter
+ * (lo(g_lo), hi(g_lo), lo32(n), 0xFFFFFFFF) and key = seed, g_lo the global id of the lower rung's chain (step draws use
+ * slots < 16).  Both lanes of a pair compute the test from the same operands, so they agree.  A swap exchanges the
+ * configuration, the energy and the walker label; everything adapted to a temperature (widths, means, covariances and
+ * factors, observable means, counters) stays with the rung. */
+__device__ __forceinline__ double swap_uniform(const U4 &r) {
+    const double d = __hiloint2double((int)(0x3ff00000u | (r.y >> 12)), (int)((r.y << 20) | (r.x >> 12)));
+    return d - (1.0 - 0x1p-53);                                               /* exact */
+}
+
+/* the rung a lane of rung r pairs with in an even / odd round; r itself when it sits out (odd rounds: the end rungs) */
+__device__ __forceinline__ int swap_partner(int r, int R, bool odd) {
+    const int pr = odd ? ((r + 1) ^ 1) - 1 : r ^ 1;
+    return pr >= 0 && pr < R ? pr : r;
+}
+
+/* 1/T_lo - 1/T_hi of the pair a lane of rung r belongs to in an even / odd round (0 when it sits out); computed once per
+   launch, so that the global loads and divisions stay off the swap's dependent chain */
+__device__ __forceinline__ double swap_dbeta(const MeParams &p, int r, bool odd) {
+    const int q = swap_partner(r, p.n_rungs, odd);
+    const int rlo = q > r ? r : q, rhi = q > r ? q : r;
+    return 1.0 / p.rung_temp[rlo] - 1.0 / p.rung_temp[rhi];
+}
+
+template <class L>
+__device__ __forceinline__ void swap_round(Chain<L> &c, int &walker, unsigned &swap_acc, bool odd, double dbeta,
+                                           long long n, unsigned long long gid, const MeParams &p) {
+    const int R = p.n_rungs;
+    const int lane = threadIdx.x & 31, r = lane & (R - 1);
+    const int q = swap_partner(r, R, odd);
+    const bool pairs = q != r;
+    const int partner = lane - r + q;
+    double xo[L::D];
+#pragma unroll
+    for (int i = 0; i < L::D; i++) xo[i] = __shfl_sync(ME_FULL, c.x[i], partner);
+    const double eo = __shfl_sync(ME_FULL, c.e, partner);
+    const int wo = __shfl_sync(ME_FULL, walker, partner);
+    const bool lower = q > r;
+    const int rlo = lower ? r : q;
+    const double e_lo = lower ? c.e : eo, e_hi = lower ? eo : c.e;
+    const double delta = dbeta * (e_lo - e_hi);
+    const unsigned long long glo = gid - (unsigned long long)r + (unsigned long long)rlo;
+    const U4 b = philox4x32((unsigned)glo, (unsigned)(glo >> 32), (unsigned)n, 0xFFFFFFFFu, p.rk);
+    const bool acc = pairs && swap_uniform(b) <= exp(delta);
+#pragma unroll
+    for (int i = 0; i < L::D; i++) c.x[i] = acc ? xo[i] : c.x[i];
+    c.e = acc ? eo : c.e;
+    walker = acc ? wo : walker;
+    swap_acc += (acc && lower) ? 1u : 0u;
+}
+
+/* sum of v over the lanes of the same rung of a warp (xor offsets >= R): lane r < R then holds its rung's sum */
+__device__ __forceinline__ double rung_sum(double v, int R) {
+    for (int o = 16; o >= R; o >>= 1) v += __shfl_xor_sync(ME_FULL, v, o);
+    return v;
+}
+
 /* ------------------------------------------------------------------------------------------ the fused kernel body
  * Cfg:  NR, NC, Energy (functor with eval / reject), STRICT (reference operation order + draw injection).   */
 /* MP: instantiation that also serves the magnitude / phase moves (groups 3, 4).  They are kept out of the default
- * instantiation so that their code (a second set of generator calls, hypot) does not sit in the hot step loop. */
-template <class Cfg, bool MP = false>
+ * instantiation so that their code (a second set of generator calls, hypot) does not sit in the hot step loop.
+ * PT: instantiation for temperature ladders (MeParams::n_rungs ...): every chain runs at its rung's temperature, swaps
+ * configurations with its neighbour rungs at the measures (swap_round) and pools its moments into its rung's row.  A ladder
+ * with swaps is R <= 32 consecutive lanes of one warp, so a launch needs chain_offset and the chain count to be multiples
+ * of R (me_set_ladder); the lanes without a chain then form whole ladders of their own. */
+template <class Cfg, bool MP = false, bool PT = false>
 __device__ __forceinline__ void run_body(const MeParams &p) {
     using L = Lay<Cfg::NR, Cfg::NC>;
     using Energy = typename Cfg::Energy;
@@ -940,12 +1018,14 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
 #endif
     /* mid-sized shapes: pooled moments on the FP64 tensor cores (pool_mma_update); their CTAs are at most
        me_pool_mma_max_block(D) threads (choose_dims in me_api.cu follows the same rule) */
-    constexpr bool POOL_MMA = ME_POOL_MMA && !POOL_REG && POOL_OK && me_pool_mma_shape(L::D, L::POOLW);
+    constexpr bool POOL_MMA = !PT && ME_POOL_MMA && !POOL_REG && POOL_OK && me_pool_mma_shape(L::D, L::POOLW);
     constexpr int POOL_MMA_BLOCK = me_pool_mma_max_block(L::D), YB_ROWS = POOL_MMA ? me_pool_mma_rows(L::D) : 1;
     constexpr int POOL_WARPS = (POOL_MMA ? POOL_MMA_BLOCK : ME_MAX_BLOCK) / 32;
-
-    __shared__ double pool_warp[POOL_WARPS][PW];
-    __shared__ double pool_cta[POOL_MMA ? 1 : PW];
+    /* ladders stage nothing in shared memory (it would cost one-warp CTAs occupancy): register-pooled shapes add their rung
+       rows to the CTA's rows in global memory warp by warp at the end of the launch; the others add every measure's rung
+       sums straight into the CTA's rows, which the host allows with one-warp CTAs only (me_set_ladder) */
+    __shared__ double pool_warp[PT ? 1 : POOL_WARPS][PT ? 1 : PW];
+    __shared__ double pool_cta[POOL_MMA || PT ? 1 : PW];
     __shared__ double ybuf[POOL_MMA ? POOL_WARPS : 1][YB_ROWS][ME_YB_LD];
     __shared__ MathTables tables;
     init_math_tables(tables);
@@ -1022,7 +1102,7 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     if (pooling && POOL_MMA) {
         for (int w = threadIdx.x; w < POOL_WARPS * PW; w += blockDim.x) (&pool_warp[0][0])[w] = 0.0;
         __syncthreads();
-    } else if (pooling && !POOL_REG) {
+    } else if (pooling && !POOL_REG && !PT) {
         for (int w = threadIdx.x; w < L::POOLW; w += blockDim.x) pool_cta[w] = 0.0;
         __syncthreads();
     }
@@ -1031,6 +1111,18 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     for (int i = 0; i < D; i++) shift[i] = pooling ? p.shift[i] : 0.0;
 
     const Rng rng(p, p.chain_offset + (unsigned long long)ch);
+    LaneTemp lane_temp;
+    int walker = 0;
+    unsigned swap_acc = 0u;
+    if (PT) {
+        const long long rung = (long long)((p.chain_offset + (unsigned long long)ch) % (unsigned long long)p.n_rungs);
+        lane_temp.temp = p.rung_temp[rung];
+        lane_temp.t_ln2 = p.rung_window[2 * rung];
+        lane_temp.t_band = p.rung_window[2 * rung + 1];
+        walker = __ldcg(p.walker + ch);
+        swap_acc = __ldcg(p.swap_acc + ch);
+    }
+    const LaneTemp *lt = PT ? &lane_temp : nullptr;
     const bool inject = STRICT && p.inj_delta != nullptr;
     const int group = p.group;
     /* under CUDA-graph replay the kernel parameters are frozen: the step index and the measure counter then come from
@@ -1039,6 +1131,17 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     long long n_meas0 = p.n_meas0;
     if (p.ctr_dev != nullptr) { step0 = __ldcg(p.ctr_dev); n_meas0 = (long long)__ldcg(p.ctr_dev + 1); }
     long long n = n_meas0 + (p.do_measure ? b_first : 0);
+    /* ladders: measures left until the next swap round, and that round's parity */
+    long long swap_in = 0;
+    bool swap_odd = false;
+    double dbeta_even = 0.0, dbeta_odd = 0.0;
+    if (PT && p.swap_every > 0) {
+        swap_in = p.swap_every - n % p.swap_every;
+        swap_odd = ((n / p.swap_every + 1) & 1) != 0;
+        const int r = (int)(threadIdx.x & 31) & (p.n_rungs - 1);
+        dbeta_even = swap_dbeta(p, r, false);
+        dbeta_odd = swap_dbeta(p, r, true);
+    }
     const unsigned step_first = (unsigned)(step0 + (unsigned long long)(b_first * p.spm));
     long long s_local = 0;
     bool accept = false;
@@ -1062,7 +1165,8 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     constexpr int TAB_ENTRIES = ME_LOGTAB_ENTRIES + ME_SINTAB_ENTRIES;       /* log table, then the sin/cos table */
     constexpr int POOL_SMEM = POOL_MMA ? POOL_WARPS * (PW + YB_ROWS * ME_YB_LD) * 8 : (ME_MAX_BLOCK / 32 + 1) * PW * 8;
     constexpr bool TAB_FITS = POOL_SMEM + TAB_ENTRIES * 16 + 1024 <= 48 * 1024;
-    constexpr bool TAB_SMEM = !STRICT && L::D > ME_SEG_MAX_D && TAB_FITS;
+    constexpr bool TAB_SMEM = !PT && !STRICT && L::D > ME_SEG_MAX_D && TAB_FITS;   /* ladders of larger shapes run one-warp
+                                                                                      CTAs: a per-CTA copy would cost occupancy */
     __shared__ double2 logtab_s[TAB_SMEM ? TAB_ENTRIES : 1];
     if (TAB_SMEM) {
         for (int i = threadIdx.x; i < TAB_ENTRIES; i += blockDim.x)
@@ -1072,7 +1176,7 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     typedef typename TabSelect<TAB_SMEM>::type Tab;
     const Tab logtab{TAB_SMEM ? logtab_s : reinterpret_cast<const double2 *>(p.logtab)};
     if (!inject && p.spm > 0 && AHEAD) {
-        gen_draws<L, STRICT, Tab>(rng, step_first, tables, cur, pins, p, logtab);
+        gen_draws<L, STRICT, Tab>(rng, step_first, tables, cur, pins, p, logtab, lt);
         if (DEEP) gen_bits<L>(rng, step_first + 1u, raw_a);
     }
 
@@ -1096,15 +1200,15 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
                     take_second_half<L>(use, make);
                 } else {                             /* next step opens the pair whose bits are waiting; step + 2 shares it */
                     raw_out = raw_in;
-                    shape_pair<L, STRICT, Tab>(raw_in, tables, make, pins, p, logtab);
+                    shape_pair<L, STRICT, Tab>(raw_in, tables, make, pins, p, logtab, lt);
                 }
             } else if (DEEP) {
                 gen_bits<L>(rng, step32 + 2u, raw_out);
-                shape_draws<L, STRICT, Tab>(raw_in, tables, make, pins, p, logtab);
+                shape_draws<L, STRICT, Tab>(raw_in, tables, make, pins, p, logtab, 0u, lt);
             } else if (AHEAD) {
-                gen_draws<L, STRICT, Tab>(rng, step32 + 1u, tables, make, pins, p, logtab);
+                gen_draws<L, STRICT, Tab>(rng, step32 + 1u, tables, make, pins, p, logtab, lt);
             } else {
-                gen_draws<L, STRICT, Tab>(rng, step32, tables, use, pins, p, logtab);
+                gen_draws<L, STRICT, Tab>(rng, step32, tables, use, pins, p, logtab, lt);
             }
             apply_proposal<L>(c, use.z, prop);
             if (MP && L::NC > 0 && group >= 3) {
@@ -1112,7 +1216,7 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
                 else propose_phases<L>(c, rng, step32, prop);
             }
         }
-        accept = finish_step<Cfg, Tab>(c, prop, use, g, p, tables, group, rng, step32, logtab);
+        accept = finish_step<Cfg, Tab>(c, prop, use, g, p, tables, group, rng, step32, logtab, lt);
         step32++;
     };
     const unsigned spm = (unsigned)p.spm;
@@ -1187,6 +1291,13 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
                 if (pooling) {
                     if (POOL_REG) {
                         for_each_pool_word<L>(c, shift, [&](int w, double v) { pacc[w] += v; });
+                    } else if (PT) {
+                        const int lane = threadIdx.x & 31, R = p.n_rungs;
+                        double *row_pool = p.pool + cgroup * (long long)(R * L::POOLW) + lane * L::POOLW;
+                        for_each_pool_word<L>(c, shift, [&](int w, double v) {
+                            v = rung_sum(active ? v : 0.0, R);
+                            if (lane < R) row_pool[w] = __ldcg(row_pool + w) + v;
+                        });
                     } else if (POOL_MMA) {
                         const int warp = threadIdx.x >> 5;
                         pool_mma_update<L, !STRICT>(c, shift, active, ybuf[warp], pool_warp[warp]);
@@ -1206,6 +1317,12 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
                         __syncthreads();
                     }
                 }
+                if (PT && p.swap_every > 0 && --swap_in == 0) {
+                    swap_round<L>(c, walker, swap_acc, swap_odd, swap_odd ? dbeta_odd : dbeta_even, n,
+                                  p.chain_offset + (unsigned long long)ch, p);
+                    swap_in = p.swap_every;
+                    swap_odd = !swap_odd;
+                }
             }
         }
     }
@@ -1214,8 +1331,25 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
         store_chain<L>(c, st, ld, ch);
         if (STATS_REG && p.do_measure) store_stats<L>(sreg, st, ld, ch);
         if (p.last_accept && p.spm > 0 && n_blocks > 0) p.last_accept[ch] = (unsigned char)accept;
+        if (PT) { p.walker[ch] = walker; p.swap_acc[ch] = swap_acc; }
     }
-    if (pooling) {
+    if (PT && pooling && POOL_REG) {       /* lanes 0..R-1 of every warp hold their rung's sums; rows rung-major */
+        const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, R = p.n_rungs;
+        double v[L::POOLW];
+#pragma unroll
+        for (int w = 0; w < L::POOLW; w++) v[w] = rung_sum(active ? pacc[w] : 0.0, R);
+        double *rows = p.pool + cgroup * (long long)(R * L::POOLW) + lane * L::POOLW;
+        const int nw = (blockDim.x + 31) >> 5;
+        for (int q = 0; q < nw; q++) {            /* warps in order: the sums do not depend on the schedule */
+            if (warp == q && lane < R) {
+#pragma unroll
+                for (int w = 0; w < L::POOLW; w++) rows[w] = __ldcg(rows + w) + v[w];
+            }
+            __syncthreads();
+        }
+    } else if (PT) {
+        /* other shapes added every measure's sums to the CTA's rows already */
+    } else if (pooling) {
         if (POOL_REG || POOL_MMA) {
             if (POOL_REG) {
                 const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;

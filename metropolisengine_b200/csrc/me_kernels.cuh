@@ -46,6 +46,33 @@ struct RunKernel<C, true> { static const void *get() { return (const void *)&k_r
 template <class C>
 struct RunKernel<C, false> { static const void *get() { return (const void *)&k_run<C>; } };
 #endif
+/* temperature ladders (me_set_ladder): the same register policy as k_run_small / k_run */
+template <class C>
+__global__ void __maxnreg__(ME_SMALL_MAXNREG) k_run_pt_small(const __grid_constant__ MeParams p) {
+    run_body<C, false, true>(p);
+}
+#ifdef ME_BIG_MAXNREG
+template <class C>
+__global__ void __maxnreg__(ME_BIG_MAXNREG) k_run_pt(const __grid_constant__ MeParams p) {
+    run_body<C, false, true>(p);
+}
+#else
+template <class C>
+__global__ void __launch_bounds__(ME_MAX_BLOCK, 1) k_run_pt(const __grid_constant__ MeParams p) {
+    run_body<C, false, true>(p);
+}
+#endif
+#ifndef ME_NVRTC
+/* caller-evaluated energies never run fused, so they get no ladder kernel */
+template <class C> struct IsExternal { static constexpr bool value = false; };
+template <int NR, int NC, bool S> struct IsExternal<Cfg<NR, NC, EnergyNone, S>> { static constexpr bool value = true; };
+template <class C, bool SMALL = (C::NR + 2 * C::NC <= 4), bool EXT = IsExternal<C>::value>
+struct RunPtKernel { static const void *get() { return (const void *)&k_run_pt_small<C>; } };
+template <class C>
+struct RunPtKernel<C, false, false> { static const void *get() { return (const void *)&k_run_pt<C>; } };
+template <class C, bool SMALL>
+struct RunPtKernel<C, SMALL, true> { static const void *get() { return nullptr; } };
+#endif
 /* the instantiation that also performs the magnitude / phase complex moves (me_set_group 3, 4; SURVEY §8 row f4) */
 template <class C>
 __global__ void __launch_bounds__(ME_MAX_BLOCK, 1) k_run_mp(const __grid_constant__ MeParams p) {
@@ -71,7 +98,7 @@ __global__ void __launch_bounds__(ME_MAX_BLOCK) k_energy(const __grid_constant__
 /* one ahead-of-time instantiation */
 struct MeAotEntry {
     int n_real, n_complex, energy_id, strict;
-    const void *run, *init, *propose, *accept, *run_mp, *energy;
+    const void *run, *init, *propose, *accept, *run_mp, *energy, *run_pt;
 };
 
 #define ME_AOT_ENTRY(NR, NC, ETMPL, EID, STRICT)                                                        \
@@ -80,7 +107,8 @@ struct MeAotEntry {
       (const void *)&me::k_propose<me::Cfg<NR, NC, ETMPL, STRICT>>,                                       \
       (const void *)&me::k_accept<me::Cfg<NR, NC, ETMPL, STRICT>>,                                        \
       me::RunMpKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                             \
-      (const void *)&me::k_energy<me::Cfg<NR, NC, ETMPL, STRICT>> }
+      (const void *)&me::k_energy<me::Cfg<NR, NC, ETMPL, STRICT>>,                                        \
+      me::RunPtKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get() }
 
 /* the shapes of BASELINE.json's configs plus the shapes of the golden fixtures */
 #define ME_AOT_TABLE(STRICT)                                                      \

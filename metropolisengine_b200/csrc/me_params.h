@@ -5,7 +5,7 @@
 #ifndef ME_PARAMS_H
 #define ME_PARAMS_H
 
-#define ME_PARAMS_VERSION 10
+#define ME_PARAMS_VERSION 11
 #define ME_MAX_CONSTS 16
 
 /* status bits written to the per-chain STATUS word (SURVEY §5 "failure detection") */
@@ -71,6 +71,14 @@ struct MeParams {
     unsigned long long seg_base;   /* ring capacity (a power of two >= seg_groups x seg_count) */
     unsigned long long *seg_flags; /* queue: [0] tickets, [1] pushes, [2 .. 2 + capacity) ring; the host writes the initial
                                       image (segment 0 of every group ready) before the launch */
+    /* temperature ladder (me_set_ladder; read by the PT instantiation of run_body only): global chain g is rung g % n_rungs */
+    int n_rungs;
+    long long swap_every;          /* replica-exchange round at every measure whose counter is a multiple; 0 = no swaps */
+    const double *rung_temp;       /* [n_rungs] temperatures */
+    const float *rung_window;      /* [n_rungs][2] t_ln2, t_band of each rung (the same expressions as the scalar ones) */
+    int *walker;                   /* [ld] walker label of the configuration a chain holds */
+    unsigned *swap_acc;            /* [ld] accepted swaps between this chain's rung and the next one up
+                                      (pooled moments of a ladder: n_rungs rows of POOLW words per CTA, rung-major) */
 };
 
 #endif

@@ -84,12 +84,18 @@ class MetropolisEngine:
     graph_callable    python energy callables only: capture the ``steps_per_measure`` steps between two measures
                       (propose -> callable -> accept, each) in a CUDA graph on first use and replay it in ``run()``;
                       the callable must then be capture-safe (static shapes, no host synchronisation)
+    replica_exchange  with ``temp`` a sequence of R temperatures (a ladder: global chain g runs at ``temp[g % R]``):
+                      0 = a temperature sweep without swaps; k > 0 = parallel tempering, a replica-exchange round of
+                      neighbour rungs (deterministic even/odd pairing) at every k-th measure.  Pooled attributes and
+                      ``pooled_statistics()`` of a ladder engine gain a leading rung axis of length R.
     """
 
     def __new__(cls, *args, adapt="per_chain", **kw):
         """One front door (SURVEY §5 config row): ``adapt="pooled"`` builds the shared-covariance engine (the proposal
         covariance of the complex block pooled over the ensemble, L.Z on the tensor cores) from the same arguments."""
         if adapt == "pooled" and cls is MetropolisEngine:
+            if np.ndim(kw.get("temp", args[9] if len(args) > 9 else 0)) > 0:
+                raise NotImplementedError("temperature ladders run with adapt='per_chain' only")
             from .engine_shared import SharedCovarianceEngine
             return SharedCovarianceEngine.from_reference_arguments(*args, **kw)
         if adapt not in ("per_chain", "pooled"):
@@ -101,7 +107,7 @@ class MetropolisEngine:
                  covariance_matrix_complex=None, params_names=None, target_acceptance=.3, temp=0,
                  complex_sample_method="multivariate-gaussian", *, n_chains=1, seed=0, device=None, strict=False,
                  record=True, callable_layout="chains_first", distributed=False, ts_chunk_bytes=1 << 30,
-                 graph_callable=False, adapt="per_chain", _shard=None):
+                 graph_callable=False, adapt="per_chain", replica_exchange=0, _shard=None):
         if initial_real_params is None and initial_complex_params is None:
             raise ValueError("must give a list containing at least one value for initial real or complex "
                              "parameters")                                                   # ME:37-39
@@ -109,6 +115,21 @@ class MetropolisEngine:
             # the reference prints a notice and falls back (ME:131-133); nothing is printed here (SURVEY App. B-12)
             complex_sample_method = "multivariate-gaussian"
         self.complex_sample_method = complex_sample_method
+        self._ladder = None             # temperatures [R] of a ladder engine
+        self._swap_every = int(replica_exchange)
+        if self._swap_every < 0:
+            raise ValueError("replica_exchange must be >= 0")
+        if np.ndim(temp) == 1:
+            temps = np.asarray(temp, dtype=np.float64)
+            if temps.size == 0:
+                raise ValueError("temp as a sequence needs at least one temperature")
+            if temps.size > 1:
+                self._ladder = temps
+            temp = float(temps[0])
+        elif np.ndim(temp) > 1:
+            raise ValueError("temp is a number or a 1-D sequence of temperatures")
+        if self._swap_every and self._ladder is None:
+            raise ValueError("replica_exchange needs temp as a sequence of at least 2 temperatures")
         if temp is None or not temp >= 0:
             raise AssertionError("temp must be >= 0")                                        # ME:92
         self._width_pair = None
@@ -146,9 +167,14 @@ class MetropolisEngine:
         self.n_chains_total = int(n_chains)
         self._group = None
         self._rank, self._world = (parallel.world() if distributed else (0, 1))
-        lo, hi = parallel.shard_range(self.n_chains_total, self._rank, self._world)
+        R = 1 if self._ladder is None else self._ladder.size
+        if self.n_chains_total % R:
+            raise ValueError("n_chains (%d) must be a multiple of the ladder's %d rungs" % (self.n_chains_total, R))
+        lo, hi = parallel.shard_range(self.n_chains_total, self._rank, self._world, granule=R)
         if _shard is not None:          # explicit global chain range [lo, hi) (tests, custom launchers)
             lo, hi = int(_shard[0]), int(_shard[1])
+            if lo % R or hi % R:
+                raise ValueError("a ladder engine's shard must hold whole ladders of %d chains" % R)
         self.chain_offset, self.n_chains = lo, hi - lo
         self._distributed = bool(distributed) and self._world > 1
 
@@ -169,7 +195,7 @@ class MetropolisEngine:
         self.observables_names.extend(["param_" + str(i) + "_squared" for i in range(nr)])
 
         # ---- adaptation constants (ME:91-107)
-        self.temp = temp
+        self.temp = temp if self._ladder is None else self._ladder.copy()
         self.target_acceptance = target_acceptance
         self.alpha, self.m, self.ratio = adaptation_constants(nr, nc, target_acceptance)
         self._sampling_width0 = float(sampling_width)
@@ -184,13 +210,22 @@ class MetropolisEngine:
         _lib.check(None, self._lib.me_create(ctypes.byref(cfg), ctypes.byref(h)))
         self._h = h
         grid, block = ctypes.c_int32(), ctypes.c_int32()
+        dev, f64 = self.device, torch.float64
+        self._walker = self._swap_acc = None
+        pw = self._lay.POOL_WORDS
+        if self._ladder is not None:
+            self._check_ladder_supported(energy_functions, reject_condition, complex_sample_method)
+            self._walker = torch.arange(lo, hi, dtype=torch.int32, device=dev)
+            self._swap_acc = torch.zeros(self.n_chains, dtype=torch.int32, device=dev)     # read as uint32 by the library
+            temps = (ctypes.c_double * R)(*self._ladder.tolist())
+            self._check(self._lib.me_set_ladder(self._h, temps, R, self._swap_every, _ptr(self._walker),
+                                                _ptr(self._swap_acc)))
+            pw = pw * R if R <= 32 and R & (R - 1) == 0 else 0      # per-rung rows; see me_set_ladder
         self._lib.me_launch_dims(self._h, ctypes.byref(grid), ctypes.byref(block))
         self._grid, self._block = grid.value, block.value
 
         # ---- device buffers (owned here, borrowed by the library)
-        dev, f64 = self.device, torch.float64
         self.state = torch.zeros((self._lay.WORDS, self.n_chains), dtype=f64, device=dev)
-        pw = self._lay.POOL_WORDS
         self._pool = torch.zeros((self._grid, pw), dtype=f64, device=dev) if pw > 0 else None
         self._shift = torch.tensor(self._shift_host, dtype=f64, device=dev)
         self._last_accept = torch.zeros(self.n_chains, dtype=torch.uint8, device=dev)
@@ -316,12 +351,30 @@ class MetropolisEngine:
         self._energy_spec = energy
 
     def set_energy_function(self, energy_function):                                        # ME:136-140
+        if self._ladder is not None:
+            self._check_ladder_supported(energy_function, self.reject_condition, self.complex_sample_method)
         self._callable = self._terms = None
         self._install_energy(energy_function)
 
     def set_reject_condition(self, reject_fct):                                            # ME:142-146
+        if self._ladder is not None and reject_fct is not None:
+            raise NotImplementedError("temperature ladders take the hard wall inside the device functor, not a python "
+                                      "reject_condition")
         self._check_reject_supported(reject_fct)
         self.reject_condition = reject_fct
+
+    def _check_ladder_supported(self, energy, reject_condition, complex_sample_method):
+        """Temperature ladders run in the fused step kernel only (its PT instantiation)."""
+        if self._d > 32:
+            raise NotImplementedError("temperature ladders need n_real + 2 n_complex <= 32 (fused shapes)")
+        if not isinstance(energy, (BuiltinEnergy, CudaEnergy, str)) and not (
+                isinstance(energy, tuple) and energy and isinstance(energy[0], str)):
+            raise NotImplementedError("temperature ladders need a device energy functor (BuiltinEnergy / CudaEnergy)")
+        if reject_condition is not None:
+            raise NotImplementedError("temperature ladders take the hard wall inside the device functor, not a python "
+                                      "reject_condition")
+        if complex_sample_method == "magnitude-phase":
+            raise NotImplementedError("temperature ladders do not run magnitude-phase complex moves")
 
     def _check_reject_supported(self, reject_fct):
         """A python predicate (ME:142-146) is evaluated on the proposal block between the proposal and the decision,
@@ -427,6 +480,9 @@ class MetropolisEngine:
         self._launch(self._lib.me_init(self._h, _ptr(x0), 0, sw, None, None, None, _ptr(e0), self._stream()))
         self._apply_width_pair()
         self._energy0 = self.state[self._lay.E].clone()
+        if self._ladder is not None:
+            self._walker.copy_(torch.arange(self.chain_offset, self.chain_offset + self.n_chains, dtype=torch.int32))
+            self._swap_acc.zero_()
         self.reset_pooled_statistics()
         self.clear_time_series()
         self.step_counter = 1
@@ -551,6 +607,8 @@ class MetropolisEngine:
 
     # ---- group-wise stepping (SURVEY §8 row f1; ME:209-239, 440-456)
     def _set_group(self, group):
+        if group and self._ladder is not None:
+            raise NotImplementedError("temperature ladders step all parameters at once (step_all / step / run)")
         if group != self._group_mode:
             self._check(self._lib.me_set_group(self._h, group))
             self._group_mode = group
@@ -683,6 +741,8 @@ class MetropolisEngine:
         """Parity mode (strict engines): drive the schedule with recorded draws (SURVEY §8c level L-A).
         ``delta``: [steps, D] or [steps, D, n_chains] increments in the order [real, Re c, Im c];
         ``u``: [steps] or [steps, n_chains] accept uniforms, NaN where none was drawn."""
+        if self._ladder is not None:
+            raise NotImplementedError("temperature ladders run on Philox draws only (no draw injection)")
         S = int(n_measures) * int(steps_per_measure)
         delta = torch.as_tensor(np.asarray(delta, dtype=np.float64), device=self.device)
         u = torch.as_tensor(np.asarray(u, dtype=np.float64), device=self.device)
@@ -822,11 +882,22 @@ class MetropolisEngine:
 
     # ------------------------------------------------------------------ pooled reads (reference attribute names)
     def _pooled(self, t):
-        """Mean over all chains of the job of a per-chain tensor [n_chains, ...] -> numpy."""
-        s = t.sum(dim=0)
+        """Mean over all chains of the job of a per-chain tensor [n_chains, ...] -> numpy.  Ladder engines: mean over
+        the ladders, per rung -> [R, ...] (a shard holds whole ladders, so local chain i is rung i % R)."""
+        if self._ladder is not None:
+            R = self._ladder.size
+            s = t.reshape((self.n_chains // R, R) + tuple(t.shape[1:])).sum(dim=0)
+            count = self.n_chains_total // R
+        else:
+            s, count = t.sum(dim=0), self.n_chains_total
         if self._distributed:
             parallel.allreduce_sum_(s, self._group)
-        return (s / self.n_chains_total).cpu().numpy()
+        return (s / count).cpu().numpy()
+
+    def _pooled_scalar(self, t):
+        """``_pooled`` of a per-chain scalar [n_chains]: a float, or numpy [R] for a ladder engine."""
+        v = self._pooled(t[:, None])[..., 0]
+        return float(v) if self._ladder is None else v
 
     def _single(self):
         return self.n_chains_total == 1
@@ -872,12 +943,11 @@ class MetropolisEngine:
 
     @property
     def real_group_sampling_width(self):                                                   # ME:98
-        v = self._pooled(self.real_group_sampling_width_per_chain[:, None])[0]
-        return float(v)
+        return self._pooled_scalar(self.real_group_sampling_width_per_chain)
 
     @property
     def complex_group_sampling_width(self):                                                # ME:99
-        return float(self._pooled(self.complex_group_sampling_width_per_chain[:, None])[0])
+        return self._pooled_scalar(self.complex_group_sampling_width_per_chain)
 
     @property
     def sampling_width(self):
@@ -895,23 +965,68 @@ class MetropolisEngine:
         """ME:125.  Live for mixed engines (ME:255); all-real / all-complex engines leave it at its initial value
         and keep the live energy in ``energy`` (SURVEY App. B-1)."""
         src = self.state[self._lay.E] if self._kind == "mixed" else self._energy0
-        return float(self._pooled(src[:, None])[0])
+        return self._pooled_scalar(src)
 
     @property
     def energy(self):
         """ME:152-156: dict of energy terms.  Single-callable engines have the one key ``"total"`` holding the live
         energy; for dict-of-terms engines each term is re-evaluated on the current state."""
         if self._terms is None:
-            return {"total": float(self._pooled(self.state[self._lay.E][:, None])[0])}
+            return {"total": self._pooled_scalar(self.state[self._lay.E])}
         full = self.state[:self._d]
-        return {t: float(self._pooled(self._eval_term(fn, full)[:, None])[0]) for t, fn in self._terms["all"].items()}
+        return {t: self._pooled_scalar(self._eval_term(fn, full)) for t, fn in self._terms["all"].items()}
 
     @property
     def acceptance_rate(self):
         steps = self.steps_done
         if steps == 0:
             return float("nan")
-        return float(self._pooled(self.accept_count_per_chain[:, None])[0]) / steps
+        return self._pooled_scalar(self.accept_count_per_chain) / steps
+
+    # ------------------------------------------------------------------ temperature ladders
+    @property
+    def temperatures(self):
+        """The temperatures, numpy [R] (R = 1 for a scalar ``temp``)."""
+        return self._ladder.copy() if self._ladder is not None else np.array([float(self.temp)])
+
+    @property
+    def rung_per_chain(self):
+        """Rung of every local chain, int64 [n_chains]: global chain g is rung g % R."""
+        R = 1 if self._ladder is None else self._ladder.size
+        return torch.arange(self.chain_offset, self.chain_offset + self.n_chains, device=self.device) % R
+
+    @property
+    def walker_per_chain(self):
+        """Label of the walker (the global id of the chain it started in) whose configuration each chain holds."""
+        if self._ladder is None:
+            return torch.arange(self.chain_offset, self.chain_offset + self.n_chains, dtype=torch.int32,
+                                device=self.device)
+        return self._walker
+
+    def _swap_attempts(self):
+        """Replica-exchange rounds each neighbour pair (r, r + 1) took part in, per ladder, numpy [R - 1]: rounds
+        k = n / swap_every over the measure counters n = 2 .. measure_step_counter, pair r in rounds k = r (mod 2)."""
+        R, e = self._ladder.size, self._swap_every
+        first, last = -(-2 // e), self.measure_step_counter // e
+        out = np.zeros(R - 1, dtype=np.int64)
+        for r in range(R - 1):
+            k0 = first + ((r - first) % 2)                  # first round >= first with k = r (mod 2)
+            out[r] = max(0, (last - k0) // 2 + 1) if last >= k0 else 0
+        return out
+
+    @property
+    def swap_acceptance_rate(self):
+        """Accepted over attempted swaps of every neighbour pair (r, r + 1), numpy [R - 1], pooled over ladders and
+        ranks (NaN before the first round of a pair)."""
+        if self._ladder is None or not self._swap_every:
+            raise AttributeError("swap_acceptance_rate needs a ladder engine with replica_exchange > 0")
+        R = self._ladder.size
+        acc = self._swap_acc.to(torch.int64).reshape(self.n_chains // R, R).sum(dim=0).to(torch.float64)
+        if self._distributed:
+            parallel.allreduce_sum_(acc, self._group)
+        att = self._swap_attempts() * (self.n_chains_total // R)
+        with np.errstate(invalid="ignore", divide="ignore"):
+            return acc.cpu().numpy()[:R - 1] / att
 
     # ------------------------------------------------------------------ clean pooled ensemble statistics
     def _library_comm(self):
@@ -933,6 +1048,8 @@ class MetropolisEngine:
         pw = self._lay.POOL_WORDS
         if pw == 0:
             raise NotImplementedError("parameter space too large for in-kernel pooled moments")
+        if self._pool is None:
+            raise NotImplementedError("pooled moments per rung need a ladder of 2, 4, 8, 16 or 32 rungs")
         if self._distributed and self._library_comm() is None:
             # no NCCL group (e.g. gloo on a CPU-only rendezvous): reduce locally, sum across ranks through torch
             self._launch(self._lib.me_allreduce_stats(self._h, None, _ptr(self._pool_inc), _ptr(self._pool_tot),
@@ -942,6 +1059,13 @@ class MetropolisEngine:
         else:
             self._flush_pool()
             tot = self._pool_tot.cpu().numpy()
+        if self._ladder is not None:          # rung-major rows of pw words; every rung has the same sample count
+            R = self._ladder.size
+            if tot[-1] / R < 2:
+                raise RuntimeError("pooled statistics need at least two measured samples")
+            per = [parallel.finalize_pooled(tot[r * pw:(r + 1) * pw], tot[-1] / R, self._shift_host,
+                                            self.num_real_params, self.num_complex_params) for r in range(R)]
+            return {k: np.stack([np.asarray(p[k]) for p in per]) for k in per[0]}
         if tot[-1] < 2:
             raise RuntimeError("pooled statistics need at least two measured samples")
         return parallel.finalize_pooled(tot[:pw], tot[-1], self._shift_host, self.num_real_params,
@@ -949,7 +1073,7 @@ class MetropolisEngine:
 
     def reset_pooled_statistics(self):
         """Forget the pooled moments accumulated so far (e.g. after burn-in)."""
-        if self._lay.POOL_WORDS:
+        if self._pool is not None:
             self._launch(self._lib.me_pool_reduce(self._h, _ptr(self._pool_out), 1, self._stream()))
         self._pool_tot.zero_()
         self._pool_pending = 0
@@ -1117,7 +1241,9 @@ class MetropolisEngine:
         self._lib.me_get_counters(self._h, ctypes.byref(n), ctypes.byref(s))
         return dict(state=self.state.clone(), n_measure=n.value, step=s.value, seed=self.seed,
                     chain_offset=self.chain_offset, pool=None if self._pool is None else self._pool.clone(),
-                    pool_tot=self._pool_tot.clone(), pool_pending=self._pool_pending)
+                    pool_tot=self._pool_tot.clone(), pool_pending=self._pool_pending,
+                    walker=None if self._walker is None else self._walker.clone(),
+                    swap_acc=None if self._swap_acc is None else self._swap_acc.clone())
 
     def load_state_dict(self, sd):
         if sd["state"].shape != self.state.shape:
@@ -1128,6 +1254,9 @@ class MetropolisEngine:
             self._pool.copy_(sd["pool"])
         self._pool_tot.copy_(sd["pool_tot"])
         self._pool_pending = int(sd["pool_pending"])
+        if self._walker is not None:
+            self._walker.copy_(sd["walker"])
+            self._swap_acc.copy_(sd["swap_acc"])
         self._check(self._lib.me_set_counters(self._h, int(sd["n_measure"]), int(sd["step"])))
         if self._ctr_on:
             self._check(self._lib.me_device_counters(self._h, 1, self._stream()))

@@ -9,15 +9,20 @@ import numpy as np
 import torch
 
 
-def shard_range(n_total, rank, world_size):
+def shard_range(n_total, rank, world_size, granule=1):
     """Contiguous global chain-id range [lo, hi) owned by ``rank``.  The Philox counter of a chain carries its
-    GLOBAL id, so results do not depend on ``world_size``."""
-    if n_total < world_size:
-        raise ValueError("fewer chains (%d) than ranks (%d)" % (n_total, world_size))
-    base, rem = divmod(n_total, world_size)
+    GLOBAL id, so results do not depend on ``world_size``.  ``granule``: the range is made of whole groups of that
+    many chains (the ladders of a tempering engine); ``n_total`` must be a multiple of it."""
+    if n_total % granule:
+        raise ValueError("n_total (%d) is not a multiple of the granule (%d)" % (n_total, granule))
+    units = n_total // granule
+    if units < world_size:
+        raise ValueError("fewer chains (%d) than ranks (%d)" % (n_total, world_size) if granule == 1 else
+                         "fewer ladders (%d) than ranks (%d)" % (units, world_size))
+    base, rem = divmod(units, world_size)
     lo = rank * base + min(rank, rem)
     hi = lo + base + (1 if rank < rem else 0)
-    return lo, hi
+    return lo * granule, hi * granule
 
 
 def world(group=None):
