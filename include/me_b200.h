@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define ME_ABI_VERSION 6
+#define ME_ABI_VERSION 7
 
 enum me_status_code {
     ME_OK = 0,
@@ -150,6 +150,20 @@ int me_set_group(me_engine *eng, int32_t group);
  * nothing.  The temperatures are copied. */
 int me_set_ladder(me_engine *eng, const double *temps, int32_t n_rungs, int64_t swap_every, int32_t *walker,
                   uint32_t *swap_acc);
+
+/* Hamiltonian ladder: me_set_ladder where every rung also has its own functor constants.  Rung r runs the handle's functor
+ * (eval and reject) with consts[r * n_consts .. (r + 1) * n_consts), 1 <= n_consts <= 16, at temps[r]; me_set_energy_builtin /
+ * me_set_energy_source must then be given n_consts constants (their values are not used by the ladder kernels).  With
+ * swap_every > 0 a pair of neighbour rungs a < b swaps configurations and walker labels with probability min(1, exp(-D)),
+ * D = (1/T_a)(E_a(x_b) - E_a(x_a)) + (1/T_b)(E_b(x_a) - E_b(x_b)), never when either cross-configuration is walled; a chain
+ * that takes a new configuration takes its own rung's energy of it.  Temperatures: finite and > 0 in any order with swaps
+ * (equal ones are the usual case), >= 0 without.  Chains, walkers, swap counts, pool rows and launch geometry as for
+ * me_set_ladder, before me_bind; consts = NULL is me_set_ladder.  ME_ERR_INVALID (with a message) for non-finite constants,
+ * n_consts outside [1, 16] or different from the registered functor's, and the temperature rules.  A handle with a rung
+ * table refuses me_energy_builtin (ME_ERR_UNSUPPORTED): there is no single constant vector to evaluate with.  The
+ * temperatures and constants are copied. */
+int me_set_hamiltonian_ladder(me_engine *eng, const double *temps, const double *consts /* [n_rungs][n_consts] */,
+                              int32_t n_consts, int32_t n_rungs, int64_t swap_every, int32_t *walker, uint32_t *swap_acc);
 
 /* Launch geometry the handle uses; the pool buffer has grid * POOL_WORDS doubles (see me_set_ladder for ladders). */
 int me_launch_dims(me_engine *eng, int32_t *grid, int32_t *block);

@@ -9,7 +9,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("ME_B200_LIB") or os.path.join(HERE, "lib", "libme_b200.so")   # override: kernel experiments
 
-ME_ABI_VERSION = 6
+ME_ABI_VERSION = 7
 
 ME_OK, ME_ERR_INVALID, ME_ERR_CUDA, ME_ERR_COMPILE, ME_ERR_UNSUPPORTED, ME_ERR_STATE = range(6)
 
@@ -61,6 +61,8 @@ SIGNATURES = {
     "me_check_energy_source": (ctypes.c_int, [_cp, _i32, _i32, _i32, _i32, _cp, _i64]),
     "me_set_group": (ctypes.c_int, [_vp, _i32]),
     "me_set_ladder": (ctypes.c_int, [_vp, ctypes.POINTER(_f64), _i32, _i64, _vp, _vp]),
+    "me_set_hamiltonian_ladder": (ctypes.c_int, [_vp, ctypes.POINTER(_f64), ctypes.POINTER(_f64), _i32, _i32, _i64, _vp,
+                                                 _vp]),
     "me_launch_dims": (ctypes.c_int, [_vp, ctypes.POINTER(_i32), ctypes.POINTER(_i32)]),
     "me_bind": (ctypes.c_int, [_vp, ctypes.POINTER(MeBuffers)]),
     "me_init": (ctypes.c_int, [_vp, _vp, _i32, _f64, _vp, _vp, _vp, _vp, _vp]),

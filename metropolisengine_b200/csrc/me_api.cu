@@ -42,7 +42,7 @@ struct KernelRef {
     bool valid() const { return rt != nullptr || drv != nullptr; }
 };
 struct KernelSet {
-    KernelRef run, init, propose, accept, energy, run_mp, run_pt;
+    KernelRef run, init, propose, accept, energy, run_mp, run_pt, run_hx;
     bool valid() const { return run.valid(); }
 };
 
@@ -181,9 +181,14 @@ int nvrtc_compile(int n_real, int n_complex, int energy_id, const std::string &u
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run(const __grid_constant__ MeParams p) { me::run_body<UserCfg>(p); }\n"
            "#endif\n"
            "#if ME_NR + 2 * ME_NC <= 4\n"
-           "extern \"C\" __global__ void __maxnreg__(160) me_k_run_pt(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, true>(p); }\n"
+           "extern \"C\" __global__ void __maxnreg__(160) me_k_run_pt(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, me::LADDER_TEMP>(p); }\n"
            "#else\n"
-           "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run_pt(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, true>(p); }\n"
+           "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run_pt(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, me::LADDER_TEMP>(p); }\n"
+           "#endif\n"
+           "#if ME_NR + 2 * ME_NC <= 4\n"
+           "extern \"C\" __global__ void __maxnreg__(160) me_k_run_hx(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, me::LADDER_HAM>(p); }\n"
+           "#else\n"
+           "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run_hx(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, me::LADDER_HAM>(p); }\n"
            "#endif\n"
            "#if ME_NC > 0\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run_mp(const __grid_constant__ MeParams p) { me::run_body<UserCfg, true>(p); }\n"
@@ -332,6 +337,7 @@ struct me_engine {
     int energy_id = -1;
     int use_reject = 0;
     double consts[ME_MAX_CONSTS];
+    int n_consts = 0;
     me_buffers buf;
     bool bound = false;
     long long n_measure = 1;           /* ME:73 */
@@ -357,6 +363,9 @@ struct me_engine {
     int *walker = nullptr;
     unsigned *swap_acc = nullptr;
     int pool_rungs = 1;                        /* rows of POOL_WORDS per CTA in the pool buffer: R for a ladder that pools */
+    /* Hamiltonian ladder (me_set_hamiltonian_ladder): rung_k > 0 runs the HX instantiation */
+    double *rung_consts = nullptr;             /* [R][rung_k] functor constants of each rung, device memory */
+    int rung_k = 0;
     std::string err;
 };
 
@@ -488,6 +497,8 @@ void base_params(me_engine *e, MeParams &p) {
         p.rung_window = reinterpret_cast<const float *>(p.rung_temp + e->n_rungs);
         p.walker = e->walker;
         p.swap_acc = e->swap_acc;
+        p.rung_consts = e->rung_consts;
+        p.n_consts = e->rung_k;
         if (e->pool_rungs != e->n_rungs) p.pool = nullptr;      /* a ladder that does not fit a warp pools nothing */
     }
 }
@@ -636,7 +647,7 @@ int resolve_kernels(me_engine *e, int energy_id, const std::string &user_src) {
             if (t[i].n_real == nr && t[i].n_complex == nc && t[i].energy_id == energy_id) {
                 e->ks.run.rt = t[i].run; e->ks.init.rt = t[i].init; e->ks.run_mp.rt = t[i].run_mp;
                 e->ks.propose.rt = t[i].propose; e->ks.accept.rt = t[i].accept; e->ks.energy.rt = t[i].energy;
-                e->ks.run_pt.rt = t[i].run_pt;
+                e->ks.run_pt.rt = t[i].run_pt; e->ks.run_hx.rt = t[i].run_hx;
                 return ME_OK;
             }
     }
@@ -669,6 +680,7 @@ int resolve_kernels(me_engine *e, int energy_id, const std::string &user_src) {
         d.moduleGetFunction(&ks.accept.drv, mod, "me_k_accept") != CUDA_SUCCESS ||
         d.moduleGetFunction(&ks.energy.drv, mod, "me_k_energy") != CUDA_SUCCESS ||
         d.moduleGetFunction(&ks.run_pt.drv, mod, "me_k_run_pt") != CUDA_SUCCESS ||
+        d.moduleGetFunction(&ks.run_hx.drv, mod, "me_k_run_hx") != CUDA_SUCCESS ||
         (e->cfg.n_complex > 0 && d.moduleGetFunction(&ks.run_mp.drv, mod, "me_k_run_mp") != CUDA_SUCCESS))
         return fail(e, ME_ERR_CUDA, "cuModuleGetFunction failed on the runtime-compiled module");
     g_cache[key] = ks;
@@ -898,9 +910,10 @@ int me_create(const me_config *cfg, me_engine **out) {
 }
 
 int me_destroy(me_engine *e) {
-    if (e && (e->seg_flags || e->ctr_dev || e->pool_partial || e->ladder_dev)) {
+    if (e && (e->seg_flags || e->ctr_dev || e->pool_partial || e->ladder_dev || e->rung_consts)) {
         DeviceGuard g(e->cfg.device);
         if (e->ladder_dev) cudaFree(e->ladder_dev);
+        if (e->rung_consts) cudaFree(e->rung_consts);
         if (e->seg_flags) cudaFree(e->seg_flags);
         if (e->ctr_dev) cudaFree(e->ctr_dev);
         if (e->pool_partial) cudaFree(e->pool_partial);
@@ -913,8 +926,12 @@ static int set_energy(me_engine *e, int id, const char *src, const double *const
     if (!e) return ME_ERR_INVALID;
     if (n_consts < 0 || n_consts > ME_MAX_CONSTS) return fail(e, ME_ERR_INVALID, "at most 16 functor constants");
     if (!builtin_template(id)) return fail(e, ME_ERR_INVALID, "unknown energy id");
+    if (e->rung_k > 0 && n_consts != e->rung_k)
+        return fail(e, ME_ERR_INVALID, "the handle's Hamiltonian ladder has " + std::to_string(e->rung_k) +
+                                           " constants per rung; the functor must take as many");
     memset(e->consts, 0, sizeof(e->consts));
     for (int i = 0; i < n_consts; i++) e->consts[i] = consts[i];
+    e->n_consts = n_consts;
     e->use_reject = use_reject ? 1 : 0;
     e->ks = KernelSet();
     e->run_slots = -1;
@@ -961,11 +978,18 @@ int me_set_group(me_engine *e, int32_t group) {
     return ME_OK;
 }
 
+/* me_set_ladder is the Hamiltonian ladder without a rung table (consts = NULL): the same checks, upload and geometry */
 int me_set_ladder(me_engine *e, const double *temps, int32_t n_rungs, int64_t swap_every, int32_t *walker,
                   uint32_t *swap_acc) {
+    return me_set_hamiltonian_ladder(e, temps, nullptr, 0, n_rungs, swap_every, walker, swap_acc);
+}
+
+int me_set_hamiltonian_ladder(me_engine *e, const double *temps, const double *consts, int32_t n_consts, int32_t n_rungs,
+                              int64_t swap_every, int32_t *walker, uint32_t *swap_acc) {
     if (!e) return ME_ERR_INVALID;
-    if (e->bound) return fail(e, ME_ERR_STATE, "me_set_ladder comes before me_bind (it sets the launch geometry)");
-    if (e->generic) return fail(e, ME_ERR_UNSUPPORTED, "temperature ladders need a fused shape (n_real + 2 n_complex <= 32)");
+    const bool ham = consts != nullptr;
+    if (e->bound) return fail(e, ME_ERR_STATE, "a ladder is set before me_bind (it sets the launch geometry)");
+    if (e->generic) return fail(e, ME_ERR_UNSUPPORTED, "ladders need a fused shape (n_real + 2 n_complex <= 32)");
     if (!temps || !walker || !swap_acc) return fail(e, ME_ERR_INVALID, "temps, walker and swap_acc are required");
     if (n_rungs < 2) return fail(e, ME_ERR_INVALID, "a ladder has at least 2 rungs");
     if (swap_every < 0) return fail(e, ME_ERR_INVALID, "swap_every must be >= 0");
@@ -980,8 +1004,17 @@ int me_set_ladder(me_engine *e, const double *temps, int32_t n_rungs, int64_t sw
             return fail(e, ME_ERR_INVALID, "ladder temperatures must be finite and >= 0");
         if (swap_every > 0 && !(temps[r] > 0))
             return fail(e, ME_ERR_INVALID, "replica exchange needs temperatures > 0");
-        if (swap_every > 0 && r > 0 && !(temps[r] > temps[r - 1]))
+        if (!ham && swap_every > 0 && r > 0 && !(temps[r] > temps[r - 1]))
             return fail(e, ME_ERR_INVALID, "replica exchange needs strictly increasing temperatures");
+    }
+    if (ham) {
+        if (n_consts < 1 || n_consts > ME_MAX_CONSTS)
+            return fail(e, ME_ERR_INVALID, "a Hamiltonian ladder has 1 to 16 constants per rung");
+        for (long long i = 0; i < R * n_consts; i++)
+            if (!std::isfinite(consts[i])) return fail(e, ME_ERR_INVALID, "rung constants must be finite");
+        if (e->energy_id >= 0 && e->n_consts != n_consts)
+            return fail(e, ME_ERR_INVALID, "the handle's functor takes " + std::to_string(e->n_consts) +
+                                               " constants; the rung table must have as many per rung");
     }
     std::vector<char> host(sizeof(double) * R + sizeof(float) * 2 * R);
     double *t = reinterpret_cast<double *>(host.data());
@@ -992,13 +1025,21 @@ int me_set_ladder(me_engine *e, const double *temps, int32_t n_rungs, int64_t sw
     }
     DeviceGuard g(e->cfg.device);
     if (e->ladder_dev) { cudaFree(e->ladder_dev); e->ladder_dev = nullptr; }
+    if (e->rung_consts) { cudaFree(e->rung_consts); e->rung_consts = nullptr; }
+    e->rung_k = 0;
+    const size_t kbytes = ham ? sizeof(double) * (size_t)(R * n_consts) : 0;
     if (cudaMalloc(&e->ladder_dev, host.size()) != cudaSuccess ||
-        cudaMemcpy(e->ladder_dev, host.data(), host.size(), cudaMemcpyHostToDevice) != cudaSuccess) {
+        cudaMemcpy(e->ladder_dev, host.data(), host.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
+        (ham && (cudaMalloc((void **)&e->rung_consts, kbytes) != cudaSuccess ||
+                 cudaMemcpy(e->rung_consts, consts, kbytes, cudaMemcpyHostToDevice) != cudaSuccess))) {
         cudaGetLastError();
         if (e->ladder_dev) cudaFree(e->ladder_dev);
+        if (e->rung_consts) cudaFree(e->rung_consts);
         e->ladder_dev = nullptr;
+        e->rung_consts = nullptr;
         return fail(e, ME_ERR_CUDA, "allocating the ladder failed");
     }
+    e->rung_k = ham ? n_consts : 0;
     e->n_rungs = n_rungs;
     e->swap_every = swap_every;
     e->walker = walker;
@@ -1075,9 +1116,10 @@ static int run_common(me_engine *e, int64_t n_blocks, int64_t spm, int do_measur
         return fail(e, ME_ERR_STATE, "no magnitude-phase kernel for this engine");
     if (e->n_rungs > 1 && (e->group != 0 || delta != nullptr))
         return fail(e, ME_ERR_UNSUPPORTED, "temperature ladders step all parameters with Philox draws only");
-    if (e->n_rungs > 1 && !e->ks.run_pt.valid())
+    const KernelRef &ladder = e->rung_k > 0 ? e->ks.run_hx : e->ks.run_pt;
+    if (e->n_rungs > 1 && !ladder.valid())
         return fail(e, ME_ERR_STATE, "no ladder kernel for this engine (device functors only)");
-    const KernelRef &kr = e->n_rungs > 1 ? e->ks.run_pt : (e->group >= 3 ? e->ks.run_mp : e->ks.run);
+    const KernelRef &kr = e->n_rungs > 1 ? ladder : (e->group >= 3 ? e->ks.run_mp : e->ks.run);
     const int segs = plan_segments(e, kr, n_blocks, spm, delta != nullptr, stream);
     if (segs < 0) return ME_ERR_CUDA;
     if (segs > 1) {
@@ -1163,6 +1205,8 @@ int me_energy_builtin(me_engine *e, const double *prop, double *e_out, unsigned 
     if (!e->bound) return fail(e, ME_ERR_STATE, "me_bind first");
     if (!prop || !e_out) return fail(e, ME_ERR_INVALID, "prop and e_out are required");
     if (e->energy_id < 0 || e->energy_id == ME_ENERGY_EXTERNAL) return fail(e, ME_ERR_STATE, "no device functor registered");
+    if (e->rung_k > 0)
+        return fail(e, ME_ERR_UNSUPPORTED, "a Hamiltonian ladder has no single constant vector to evaluate proposals with");
     MeParams p;
     base_params(e, p);
     p.prop = const_cast<double *>(prop); p.e_out = e_out; p.rej_out = rej_out;

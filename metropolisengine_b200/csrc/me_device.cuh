@@ -204,6 +204,11 @@ struct LaneTemp {
     float t_ln2, t_band;
 };
 
+/* Ladder mode of run_body: none (one temperature and one constant vector for every chain), a temperature ladder (PT), or
+ * a Hamiltonian ladder (HX: every rung also has its own functor constants, and a swap evaluates each rung's energy at its
+ * partner's configuration). */
+enum LadderMode { LADDER_NONE = 0, LADDER_TEMP = 1, LADDER_HAM = 2 };
+
 /* ------------------------------------------------------------------------------------------ per-chain registers */
 template <class L>
 struct Chain {
@@ -853,11 +858,13 @@ template <class Cfg, class Tab = LogTabGlobal>
 __device__ __forceinline__ bool finish_step(Chain<Lay<Cfg::NR, Cfg::NC>> &c, double (&prop)[Lay<Cfg::NR, Cfg::NC>::D],
                                             const Draws<Lay<Cfg::NR, Cfg::NC>> &d, const Gains &g, const MeParams &p,
                                             const MathTables &tables, int group, const Rng &rng, unsigned step,
-                                            const Tab &logtab, const LaneTemp *lt = nullptr) {
+                                            const Tab &logtab, const LaneTemp *lt = nullptr,
+                                            const double *krung = nullptr) {
     using L = Lay<Cfg::NR, Cfg::NC>;
     using Energy = typename Cfg::Energy;
     constexpr bool STRICT = Cfg::STRICT;
     constexpr int D = L::D;
+    const double *k = krung ? krung : p.consts;      /* the chain's rung constants on a Hamiltonian ladder */
     if (L::KIND == 0 && group != 0) {       /* group-wise step: the other block keeps its value */
 #pragma unroll
         for (int i = 0; i < D; i++) {
@@ -866,10 +873,10 @@ __device__ __forceinline__ bool finish_step(Chain<Lay<Cfg::NR, Cfg::NC>> &c, dou
         }
     }
     bool accept = false;
-    const bool wall = p.use_reject && Energy::reject(prop, prop + L::NR, prop + L::NR + L::NC, p.consts);
+    const bool wall = p.use_reject && Energy::reject(prop, prop + L::NR, prop + L::NR + L::NC, k);
     if (STRICT) {
         if (!wall) {
-            const double e_new = Energy::eval(prop, prop + L::NR, prop + L::NR + L::NC, p.consts);
+            const double e_new = Energy::eval(prop, prop + L::NR, prop + L::NR + L::NC, k);
             if (e_new != e_new) c.status |= ME_STATUS_ENERGY_NAN;
             accept = decide<STRICT>(e_new - c.e, d.u, p, tables, g.hot, g.k64, lt);
             if (accept) {
@@ -886,7 +893,7 @@ __device__ __forceinline__ bool finish_step(Chain<Lay<Cfg::NR, Cfg::NC>> &c, dou
         double e_new = 0.0, diff = 0.0;
         bool inside = false;
         if (!wall) {
-            e_new = Energy::eval(prop, prop + L::NR, prop + L::NR + L::NC, p.consts);
+            e_new = Energy::eval(prop, prop + L::NR, prop + L::NR + L::NC, k);
             diff = e_new - c.e;
             accept = diff <= (double)d.lo;
             inside = !accept && !(diff > (double)d.hi);
@@ -934,7 +941,18 @@ __device__ __forceinline__ bool finish_step(Chain<Lay<Cfg::NR, Cfg::NC>> &c, dou
  * (lo(g_lo), hi(g_lo), lo32(n), 0xFFFFFFFF) and key = seed, g_lo the global id of the lower rung's chain (step draws use
  * slots < 16).  Both lanes of a pair compute the test from the same operands, so they agree.  A swap exchanges the
  * configuration, the energy and the walker label; everything adapted to a temperature (widths, means, covariances and
- * factors, observable means, counters) stays with the rung. */
+ * factors, observable means, counters) stays with the rung.
+ *
+ * Hamiltonian ladders (identical in oracle/me_oracle_hladder.c, meo_run_hladder).  Rung r has temperature T_r and constant
+ * vector k_r[0..K), 1 <= K <= 16; every step evaluates the functor (eval and reject) with k_r of the chain's rung.  The
+ * swap uniform, the pairing schedule and what moves or stays are those above.  With a the lower and b the upper rung of a
+ * pair and E_a(x) rung a's functor with k_a at x, the pair swaps iff u <= exp(-D) with
+ *     D = (1/T_a) (E_a(x_b) - E_a(x_a)) + (1/T_b) (E_b(x_a) - E_b(x_b)),
+ * which both lanes evaluate from the same four energies in this operand order, so they agree bit for bit.  The pair does
+ * not swap if either cross-configuration is walled (reject(x_b; k_a) or reject(x_a; k_b)).  A NaN cross-energy refuses the
+ * swap and sets ME_STATUS_ENERGY_NAN on the lane that computed it (a lane that pairs and whose own wall passes its
+ * partner's configuration).  After a swap a chain holds its own rung's energy of the new configuration, E_a(x_b), not its
+ * partner's E.  Temperatures: finite and > 0 in any order with swaps (equal ones are the usual case), >= 0 without. */
 __device__ __forceinline__ double swap_uniform(const U4 &r) {
     const double d = __hiloint2double((int)(0x3ff00000u | (r.y >> 12)), (int)((r.y << 20) | (r.x >> 12)));
     return d - (1.0 - 0x1p-53);                                               /* exact */
@@ -954,9 +972,20 @@ __device__ __forceinline__ double swap_dbeta(const MeParams &p, int r, bool odd)
     return 1.0 / p.rung_temp[rlo] - 1.0 / p.rung_temp[rhi];
 }
 
-template <class L>
-__device__ __forceinline__ void swap_round(Chain<L> &c, int &walker, unsigned &swap_acc, bool odd, double dbeta,
-                                           long long n, unsigned long long gid, const MeParams &p) {
+/* 1/T of the rung a lane of rung r pairs with in an even / odd round (Hamiltonian ladders; its own 1/T when it sits out),
+   computed once per launch like swap_dbeta */
+__device__ __forceinline__ double swap_beta(const MeParams &p, int r, bool odd) {
+    return 1.0 / p.rung_temp[swap_partner(r, p.n_rungs, odd)];
+}
+
+/* One round.  Temperature ladders: dbeta = swap_dbeta.  Hamiltonian ladders: dbeta = swap_beta, beta = 1/T of the lane's
+   own rung, krung = its rung's constants. */
+template <class Cfg, int LM>
+__device__ __forceinline__ void swap_round(Chain<Lay<Cfg::NR, Cfg::NC>> &c, int &walker, unsigned &swap_acc, bool odd,
+                                           double dbeta, long long n, unsigned long long gid, const MeParams &p,
+                                           double beta = 0.0, const double *krung = nullptr) {
+    using L = Lay<Cfg::NR, Cfg::NC>;
+    using Energy = typename Cfg::Energy;
     const int R = p.n_rungs;
     const int lane = threadIdx.x & 31, r = lane & (R - 1);
     const int q = swap_partner(r, R, odd);
@@ -969,14 +998,32 @@ __device__ __forceinline__ void swap_round(Chain<L> &c, int &walker, unsigned &s
     const int wo = __shfl_sync(ME_FULL, walker, partner);
     const bool lower = q > r;
     const int rlo = lower ? r : q;
-    const double e_lo = lower ? c.e : eo, e_hi = lower ? eo : c.e;
-    const double delta = dbeta * (e_lo - e_hi);
+    double e_new = eo;
+    bool ok = pairs;
+    double delta;
+    if (LM == LADDER_HAM) {
+        /* own rung at the partner's configuration; the partner's rung at this one comes back by shuffle */
+        const bool wall = p.use_reject && Energy::reject(xo, xo + L::NR, xo + L::NR + L::NC, krung);
+        const double ec = Energy::eval(xo, xo + L::NR, xo + L::NR + L::NC, krung);
+        if (pairs && !wall && ec != ec) c.status |= ME_STATUS_ENERGY_NAN;
+        const double eco = __shfl_sync(ME_FULL, ec, partner);
+        const bool wall_o = __shfl_sync(ME_FULL, (int)wall, partner) != 0;
+        const double d_own = ec - c.e, d_other = eco - eo;
+        const double b_lo = lower ? beta : dbeta, b_hi = lower ? dbeta : beta;
+        const double d_lo = lower ? d_own : d_other, d_hi = lower ? d_other : d_own;
+        delta = -(b_lo * d_lo + b_hi * d_hi);
+        ok = ok && !wall && !wall_o;
+        e_new = ec;
+    } else {
+        const double e_lo = lower ? c.e : eo, e_hi = lower ? eo : c.e;
+        delta = dbeta * (e_lo - e_hi);
+    }
     const unsigned long long glo = gid - (unsigned long long)r + (unsigned long long)rlo;
     const U4 b = philox4x32((unsigned)glo, (unsigned)(glo >> 32), (unsigned)n, 0xFFFFFFFFu, p.rk);
-    const bool acc = pairs && swap_uniform(b) <= exp(delta);
+    const bool acc = ok && swap_uniform(b) <= exp(delta);
 #pragma unroll
     for (int i = 0; i < L::D; i++) c.x[i] = acc ? xo[i] : c.x[i];
-    c.e = acc ? eo : c.e;
+    c.e = acc ? e_new : c.e;
     walker = acc ? wo : walker;
     swap_acc += (acc && lower) ? 1u : 0u;
 }
@@ -994,13 +1041,17 @@ __device__ __forceinline__ double rung_sum(double v, int R) {
  * PT: instantiation for temperature ladders (MeParams::n_rungs ...): every chain runs at its rung's temperature, swaps
  * configurations with its neighbour rungs at the measures (swap_round) and pools its moments into its rung's row.  A ladder
  * with swaps is R <= 32 consecutive lanes of one warp, so a launch needs chain_offset and the chain count to be multiples
- * of R (me_set_ladder); the lanes without a chain then form whole ladders of their own. */
-template <class Cfg, bool MP = false, bool PT = false>
+ * of R (me_set_ladder); the lanes without a chain then form whole ladders of their own.
+ * LM selects the ladder mode: LADDER_TEMP is the PT instantiation above; LADDER_HAM (HX) is the same with each rung's
+ * functor constants (MeParams::rung_consts) held per lane for the whole launch, and a swap round that evaluates each
+ * rung's energy at its partner's configuration (swap_round). */
+template <class Cfg, bool MP = false, int LM = LADDER_NONE>
 __device__ __forceinline__ void run_body(const MeParams &p) {
     using L = Lay<Cfg::NR, Cfg::NC>;
     using Energy = typename Cfg::Energy;
     constexpr bool STRICT = Cfg::STRICT;
     constexpr int D = L::D;
+    constexpr bool PT = LM != LADDER_NONE, HAM = LM == LADDER_HAM;
     /* small problems keep running statistics and pooled accumulators in registers for the whole launch;
        larger ones touch them in global memory at measure time only */
 #ifndef ME_STATS_REG_MAX
@@ -1114,6 +1165,9 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     LaneTemp lane_temp;
     int walker = 0;
     unsigned swap_acc = 0u;
+    /* Hamiltonian ladders: the rung's constants in registers for the whole launch (the functor indexes them with
+       constants, so only the ones it reads stay live), zero beyond K as p.consts is */
+    double krung[HAM ? ME_MAX_CONSTS : 1];
     if (PT) {
         const long long rung = (long long)((p.chain_offset + (unsigned long long)ch) % (unsigned long long)p.n_rungs);
         lane_temp.temp = p.rung_temp[rung];
@@ -1121,8 +1175,14 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
         lane_temp.t_band = p.rung_window[2 * rung + 1];
         walker = __ldcg(p.walker + ch);
         swap_acc = __ldcg(p.swap_acc + ch);
+        if (HAM) {
+            const double *row = p.rung_consts + rung * p.n_consts;
+#pragma unroll
+            for (int i = 0; i < (HAM ? ME_MAX_CONSTS : 1); i++) krung[i] = i < p.n_consts ? row[i] : 0.0;
+        }
     }
     const LaneTemp *lt = PT ? &lane_temp : nullptr;
+    const double *kr = HAM ? krung : nullptr;
     const bool inject = STRICT && p.inj_delta != nullptr;
     const int group = p.group;
     /* under CUDA-graph replay the kernel parameters are frozen: the step index and the measure counter then come from
@@ -1134,13 +1194,19 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     /* ladders: measures left until the next swap round, and that round's parity */
     long long swap_in = 0;
     bool swap_odd = false;
-    double dbeta_even = 0.0, dbeta_odd = 0.0;
+    double dbeta_even = 0.0, dbeta_odd = 0.0, beta = 0.0;      /* Hamiltonian ladders: the partner's 1/T, and the own 1/T */
     if (PT && p.swap_every > 0) {
         swap_in = p.swap_every - n % p.swap_every;
         swap_odd = ((n / p.swap_every + 1) & 1) != 0;
         const int r = (int)(threadIdx.x & 31) & (p.n_rungs - 1);
-        dbeta_even = swap_dbeta(p, r, false);
-        dbeta_odd = swap_dbeta(p, r, true);
+        if (HAM) {
+            dbeta_even = swap_beta(p, r, false);
+            dbeta_odd = swap_beta(p, r, true);
+            beta = 1.0 / lane_temp.temp;
+        } else {
+            dbeta_even = swap_dbeta(p, r, false);
+            dbeta_odd = swap_dbeta(p, r, true);
+        }
     }
     const unsigned step_first = (unsigned)(step0 + (unsigned long long)(b_first * p.spm));
     long long s_local = 0;
@@ -1216,7 +1282,7 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
                 else propose_phases<L>(c, rng, step32, prop);
             }
         }
-        accept = finish_step<Cfg, Tab>(c, prop, use, g, p, tables, group, rng, step32, logtab, lt);
+        accept = finish_step<Cfg, Tab>(c, prop, use, g, p, tables, group, rng, step32, logtab, lt, kr);
         step32++;
     };
     const unsigned spm = (unsigned)p.spm;
@@ -1318,8 +1384,8 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
                     }
                 }
                 if (PT && p.swap_every > 0 && --swap_in == 0) {
-                    swap_round<L>(c, walker, swap_acc, swap_odd, swap_odd ? dbeta_odd : dbeta_even, n,
-                                  p.chain_offset + (unsigned long long)ch, p);
+                    swap_round<Cfg, LM>(c, walker, swap_acc, swap_odd, swap_odd ? dbeta_odd : dbeta_even, n,
+                                        p.chain_offset + (unsigned long long)ch, p, beta, kr);
                     swap_in = p.swap_every;
                     swap_odd = !swap_odd;
                 }
@@ -1422,7 +1488,14 @@ __device__ __forceinline__ void init_body(const MeParams &p) {
     for (int j = 0; j < NC; j++) s.obsm[NR + j] = hypot(c.x[NR + j], c.x[NR + NC + j]);
 #pragma unroll
     for (int i = 0; i < NR; i++) s.obsm[NR + NC + i] = c.x[i] * c.x[i];
-    c.e = p.have_e0 ? p.e_new[ch] : Energy::eval(c.x, c.x + NR, c.x + NR + NC, p.consts);
+    /* a Hamiltonian ladder's chain starts with its rung's energy */
+    double k[ME_MAX_CONSTS];
+    const bool rungs = p.rung_consts != nullptr;
+    const long long rung = rungs ? (long long)((p.chain_offset + (unsigned long long)ch) % (unsigned long long)p.n_rungs) : 0;
+#pragma unroll
+    for (int i = 0; i < ME_MAX_CONSTS; i++)
+        k[i] = rungs ? (i < p.n_consts ? p.rung_consts[rung * p.n_consts + i] : 0.0) : p.consts[i];
+    c.e = p.have_e0 ? p.e_new[ch] : Energy::eval(c.x, c.x + NR, c.x + NR + NC, k);
     c.nacc = 0.0;
     c.nacc_new = 0u;
     c.status = 0;

@@ -49,17 +49,33 @@ struct RunKernel<C, false> { static const void *get() { return (const void *)&k_
 /* temperature ladders (me_set_ladder): the same register policy as k_run_small / k_run */
 template <class C>
 __global__ void __maxnreg__(ME_SMALL_MAXNREG) k_run_pt_small(const __grid_constant__ MeParams p) {
-    run_body<C, false, true>(p);
+    run_body<C, false, LADDER_TEMP>(p);
 }
 #ifdef ME_BIG_MAXNREG
 template <class C>
 __global__ void __maxnreg__(ME_BIG_MAXNREG) k_run_pt(const __grid_constant__ MeParams p) {
-    run_body<C, false, true>(p);
+    run_body<C, false, LADDER_TEMP>(p);
 }
 #else
 template <class C>
 __global__ void __launch_bounds__(ME_MAX_BLOCK, 1) k_run_pt(const __grid_constant__ MeParams p) {
-    run_body<C, false, true>(p);
+    run_body<C, false, LADDER_TEMP>(p);
+}
+#endif
+/* Hamiltonian ladders (me_set_hamiltonian_ladder): the same register policy */
+template <class C>
+__global__ void __maxnreg__(ME_SMALL_MAXNREG) k_run_hx_small(const __grid_constant__ MeParams p) {
+    run_body<C, false, LADDER_HAM>(p);
+}
+#ifdef ME_BIG_MAXNREG
+template <class C>
+__global__ void __maxnreg__(ME_BIG_MAXNREG) k_run_hx(const __grid_constant__ MeParams p) {
+    run_body<C, false, LADDER_HAM>(p);
+}
+#else
+template <class C>
+__global__ void __launch_bounds__(ME_MAX_BLOCK, 1) k_run_hx(const __grid_constant__ MeParams p) {
+    run_body<C, false, LADDER_HAM>(p);
 }
 #endif
 #ifndef ME_NVRTC
@@ -72,6 +88,12 @@ template <class C>
 struct RunPtKernel<C, false, false> { static const void *get() { return (const void *)&k_run_pt<C>; } };
 template <class C, bool SMALL>
 struct RunPtKernel<C, SMALL, true> { static const void *get() { return nullptr; } };
+template <class C, bool SMALL = (C::NR + 2 * C::NC <= 4), bool EXT = IsExternal<C>::value>
+struct RunHxKernel { static const void *get() { return (const void *)&k_run_hx_small<C>; } };
+template <class C>
+struct RunHxKernel<C, false, false> { static const void *get() { return (const void *)&k_run_hx<C>; } };
+template <class C, bool SMALL>
+struct RunHxKernel<C, SMALL, true> { static const void *get() { return nullptr; } };
 #endif
 /* the instantiation that also performs the magnitude / phase complex moves (me_set_group 3, 4; SURVEY §8 row f4) */
 template <class C>
@@ -98,7 +120,7 @@ __global__ void __launch_bounds__(ME_MAX_BLOCK) k_energy(const __grid_constant__
 /* one ahead-of-time instantiation */
 struct MeAotEntry {
     int n_real, n_complex, energy_id, strict;
-    const void *run, *init, *propose, *accept, *run_mp, *energy, *run_pt;
+    const void *run, *init, *propose, *accept, *run_mp, *energy, *run_pt, *run_hx;
 };
 
 #define ME_AOT_ENTRY(NR, NC, ETMPL, EID, STRICT)                                                        \
@@ -108,7 +130,8 @@ struct MeAotEntry {
       (const void *)&me::k_accept<me::Cfg<NR, NC, ETMPL, STRICT>>,                                        \
       me::RunMpKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                             \
       (const void *)&me::k_energy<me::Cfg<NR, NC, ETMPL, STRICT>>,                                        \
-      me::RunPtKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get() }
+      me::RunPtKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                             \
+      me::RunHxKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get() }
 
 /* the shapes of BASELINE.json's configs plus the shapes of the golden fixtures */
 #define ME_AOT_TABLE(STRICT)                                                      \

@@ -5,7 +5,7 @@
 #ifndef ME_PARAMS_H
 #define ME_PARAMS_H
 
-#define ME_PARAMS_VERSION 11
+#define ME_PARAMS_VERSION 12
 #define ME_MAX_CONSTS 16
 
 /* status bits written to the per-chain STATUS word (SURVEY §5 "failure detection") */
@@ -79,6 +79,9 @@ struct MeParams {
     int *walker;                   /* [ld] walker label of the configuration a chain holds */
     unsigned *swap_acc;            /* [ld] accepted swaps between this chain's rung and the next one up
                                       (pooled moments of a ladder: n_rungs rows of POOLW words per CTA, rung-major) */
+    /* Hamiltonian ladder (me_set_hamiltonian_ladder; read by the HX instantiation of run_body and by init_body) */
+    const double *rung_consts;     /* [n_rungs][n_consts] functor constants of each rung (NULL: consts on every chain) */
+    int n_consts;                  /* K, 1 <= K <= ME_MAX_CONSTS */
 };
 
 #endif

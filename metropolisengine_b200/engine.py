@@ -88,14 +88,21 @@ class MetropolisEngine:
                       0 = a temperature sweep without swaps; k > 0 = parallel tempering, a replica-exchange round of
                       neighbour rungs (deterministic even/odd pairing) at every k-th measure.  Pooled attributes and
                       ``pooled_statistics()`` of a ladder engine gain a leading rung axis of length R.
+    rung_consts       [R, K] array: a Hamiltonian ladder.  Rung r (global chain g is rung g % R) runs the energy functor
+                      with the constants ``rung_consts[r]`` instead of the energy's own, at ``temp`` (a number: every rung)
+                      or ``temp[r]`` (a sequence of length R).  K must equal the number of constants the energy was given.
+                      With ``replica_exchange=k > 0`` neighbour rungs a < b swap configurations with probability
+                      min(1, exp(-D)), D = (E_a(x_b) - E_a(x_a)) / T_a + (E_b(x_a) - E_b(x_b)) / T_b, and a chain that
+                      takes a configuration takes its own rung's energy of it; 0 = a sweep over the constants in one
+                      launch.  Everything else is as for temperature ladders.
     """
 
     def __new__(cls, *args, adapt="per_chain", **kw):
         """One front door (SURVEY §5 config row): ``adapt="pooled"`` builds the shared-covariance engine (the proposal
         covariance of the complex block pooled over the ensemble, L.Z on the tensor cores) from the same arguments."""
         if adapt == "pooled" and cls is MetropolisEngine:
-            if np.ndim(kw.get("temp", args[9] if len(args) > 9 else 0)) > 0:
-                raise NotImplementedError("temperature ladders run with adapt='per_chain' only")
+            if np.ndim(kw.get("temp", args[9] if len(args) > 9 else 0)) > 0 or kw.get("rung_consts") is not None:
+                raise NotImplementedError("temperature and Hamiltonian ladders run with adapt='per_chain' only")
             from .engine_shared import SharedCovarianceEngine
             return SharedCovarianceEngine.from_reference_arguments(*args, **kw)
         if adapt not in ("per_chain", "pooled"):
@@ -107,7 +114,7 @@ class MetropolisEngine:
                  covariance_matrix_complex=None, params_names=None, target_acceptance=.3, temp=0,
                  complex_sample_method="multivariate-gaussian", *, n_chains=1, seed=0, device=None, strict=False,
                  record=True, callable_layout="chains_first", distributed=False, ts_chunk_bytes=1 << 30,
-                 graph_callable=False, adapt="per_chain", replica_exchange=0, _shard=None):
+                 graph_callable=False, adapt="per_chain", replica_exchange=0, rung_consts=None, _shard=None):
         if initial_real_params is None and initial_complex_params is None:
             raise ValueError("must give a list containing at least one value for initial real or complex "
                              "parameters")                                                   # ME:37-39
@@ -128,6 +135,18 @@ class MetropolisEngine:
             temp = float(temps[0])
         elif np.ndim(temp) > 1:
             raise ValueError("temp is a number or a 1-D sequence of temperatures")
+        self._rung_consts = None        # [R, K] functor constants of a Hamiltonian ladder's rungs
+        if rung_consts is not None:
+            rc = np.array(rung_consts, dtype=np.float64)
+            if rc.ndim != 2 or rc.shape[0] < 2 or rc.shape[1] < 1:
+                raise ValueError("rung_consts is an [R, K] array with R >= 2 rungs and K >= 1 constants")
+            if not np.all(np.isfinite(rc)):
+                raise ValueError("rung_consts must be finite")
+            if self._ladder is None:
+                self._ladder = np.full(rc.shape[0], temp, dtype=np.float64)
+            elif self._ladder.size != rc.shape[0]:
+                raise ValueError("temp has %d temperatures for %d rungs of rung_consts" % (self._ladder.size, rc.shape[0]))
+            self._rung_consts = rc
         if self._swap_every and self._ladder is None:
             raise ValueError("replica_exchange needs temp as a sequence of at least 2 temperatures")
         if temp is None or not temp >= 0:
@@ -218,8 +237,17 @@ class MetropolisEngine:
             self._walker = torch.arange(lo, hi, dtype=torch.int32, device=dev)
             self._swap_acc = torch.zeros(self.n_chains, dtype=torch.int32, device=dev)     # read as uint32 by the library
             temps = (ctypes.c_double * R)(*self._ladder.tolist())
-            self._check(self._lib.me_set_ladder(self._h, temps, R, self._swap_every, _ptr(self._walker),
-                                                _ptr(self._swap_acc)))
+            if self._rung_consts is None:
+                self._check(self._lib.me_set_ladder(self._h, temps, R, self._swap_every, _ptr(self._walker),
+                                                    _ptr(self._swap_acc)))
+            else:
+                K = self._rung_consts.shape[1]
+                n_energy = len(self._device_energy(energy_functions).consts)
+                if n_energy != K:
+                    raise ValueError("rung_consts has %d constants per rung, the energy takes %d" % (K, n_energy))
+                table = (ctypes.c_double * (R * K))(*self._rung_consts.ravel().tolist())
+                self._check(self._lib.me_set_hamiltonian_ladder(self._h, temps, table, K, R, self._swap_every,
+                                                                _ptr(self._walker), _ptr(self._swap_acc)))
             pw = pw * R if R <= 32 and R & (R - 1) == 0 else 0      # per-rung rows; see me_set_ladder
         self._lib.me_launch_dims(self._h, ctypes.byref(grid), ctypes.byref(block))
         self._grid, self._block = grid.value, block.value
@@ -318,11 +346,17 @@ class MetropolisEngine:
             self.state[self._lay.SIG].fill_(self._width_pair[0])
             self.state[self._lay.SIG + 1].fill_(self._width_pair[1])
 
-    def _install_energy(self, energy):
+    @staticmethod
+    def _device_energy(energy):
+        """A built-in name or (name, consts...) tuple as its BuiltinEnergy; anything else unchanged."""
         if isinstance(energy, str):
-            energy = BuiltinEnergy(energy)
-        elif isinstance(energy, tuple) and energy and isinstance(energy[0], str):
-            energy = BuiltinEnergy(energy[0], *energy[1:])
+            return BuiltinEnergy(energy)
+        if isinstance(energy, tuple) and energy and isinstance(energy[0], str):
+            return BuiltinEnergy(energy[0], *energy[1:])
+        return energy
+
+    def _install_energy(self, energy):
+        energy = self._device_energy(energy)
         if isinstance(energy, BuiltinEnergy):
             consts = (ctypes.c_double * max(len(energy.consts), 1))(*energy.consts)
             self._check(self._lib.me_set_energy_builtin(self._h, _lib.ENERGY_IDS[energy.name], consts,
@@ -351,6 +385,9 @@ class MetropolisEngine:
         self._energy_spec = energy
 
     def set_energy_function(self, energy_function):                                        # ME:136-140
+        if self._rung_consts is not None:
+            raise NotImplementedError("a Hamiltonian ladder's rung_consts belong to its energy functor; build a new engine "
+                                      "to change the functor")
         if self._ladder is not None:
             self._check_ladder_supported(energy_function, self.reject_condition, self.complex_sample_method)
         self._callable = self._terms = None
@@ -988,6 +1025,11 @@ class MetropolisEngine:
     def temperatures(self):
         """The temperatures, numpy [R] (R = 1 for a scalar ``temp``)."""
         return self._ladder.copy() if self._ladder is not None else np.array([float(self.temp)])
+
+    @property
+    def rung_consts(self):
+        """Functor constants of every rung of a Hamiltonian ladder, numpy [R, K] (None for other engines)."""
+        return None if self._rung_consts is None else self._rung_consts.copy()
 
     @property
     def rung_per_chain(self):
