@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define ME_ABI_VERSION 7
+#define ME_ABI_VERSION 8
 
 enum me_status_code {
     ME_OK = 0,
@@ -384,6 +384,42 @@ int me_statistical_inefficiency(const double *ts, int64_t rows, int64_t row0, in
 int me_detect_equilibration(const double *ts, int64_t rows, int32_t cols, int64_t ld, int32_t col, int64_t chain0,
                             int64_t n_sel, int64_t nskip, int32_t fast, double *scratch, int64_t scratch_doubles,
                             double *t_out, double *g_out, double *neff_out, void *stream);
+
+/* MBAR over recorded rows (Shirts & Chodera, J. Chem. Phys. 129, 124105, 2008; pymbar's MBAR): one pass of the
+ * multistate Bennett acceptance ratio over the time-series rows [row0, rows) of one storage chunk ts[row][TS_COLS][n_chains]
+ * of this handle, every stride-th row, every local chain.  Sample n = (row, chain) was drawn at rung
+ * (chain_offset + chain) % R (R = 1 for a handle without a ladder); every rung has the same count N = n_per_state (the
+ * global count: samples of all chunks and all ranks / R).  States: the R rungs (temps[r], the rung's constants, or the
+ * handle's constants on a temperature ladder; the handle's temp when R = 1) followed by n_target targets
+ * (target_temps[t], target_consts[t][K] with K the functor's constant count; target_consts = NULL: the handle's constants,
+ * not allowed on a Hamiltonian ladder); S = R + n_target <= 32.  u_s(x) = E(x; k_s) / T_s is re-evaluated from the stored
+ * x columns with the handle's device functor (wall first: a walled x has weight 0 in state s).  Given f[R] (device,
+ * reduced free energies of the rungs; the targets take f = 0):
+ *     L_n  = ln sum_k N exp(f_k - u_k(x_n)),   w_ns = exp(f_s - u_s(x_n) - L_n)
+ * and the pass writes (accumulate = 0) or adds (accumulate != 0: a series kept in several chunks is passed chunk by chunk)
+ * the fixed-order sums
+ *     sums[0] = sum_n L_n,  sums[1] = samples with a NaN energy or a non-finite L_n,  sums[2] = samples whose target
+ *     weight exceeds 1e140 (a target without overlap) — such samples enter no other sum;
+ *     then s[S] (s_s = sum_n w_ns), then G lower-packed (G_st = sum_n w_ns w_nt at s(s+1)/2 + t, t <= s),
+ *     then, with_obs != 0, per state s: sum_n w_ns [x_0..x_{D-1}, x_0^2..x_{D-1}^2, E_s(x_n), E_s(x_n)^2].
+ * me_mbar_words gives the length.  The sums are plain FP64 sums: across ranks they all-reduce as they are
+ * (me_comm_allreduce).  One pass is bit-identical from run to run on one device.
+ * Finishing the computation on the host (S x S algebra, what metropolisengine_b200/mbar.py does):
+ *     objective F(f) = sum L - N sum_k f_k (convex), gradient g_i = N (s_i - 1), Hessian H_ij = delta_ij N s_i - N^2 G_ij;
+ *     gauge f_0 = 0; Newton on f_1..f_{R-1} from f = 0 with a backtracking line search on F (one pass per trial point),
+ *     until max |s_i - 1| < tol; if the reduced Hessian is not positive definite, f_i <- f_i - ln s_i.
+ *     Targets: f_t = -ln s_t;  <a>_t = (sum_n w_nt a_t) / s_t.
+ *     Uncertainties (pymbar "svd-ew", uncorrelated samples: take stride ~ the statistical inefficiency of the E column):
+ *     G = V Sigma^2 V^T,  Theta = V Sigma (I - Sigma V^T diag(N_s) V Sigma)^+ Sigma V^T with N_s = 0 for targets,
+ *     d(f_j - f_i) = sqrt(Theta_ii + Theta_jj - 2 Theta_ij).
+ * ME_ERR_INVALID (with a message): more than 32 rungs or states, a rung or target temperature not finite or not > 0,
+ * non-finite constants, targets of a Hamiltonian ladder without target_consts, row0 outside [0, rows), stride < 1,
+ * n_per_state < 1, null pointers.  ME_ERR_UNSUPPORTED: D > 32, caller-evaluated energies, group / magnitude-phase modes.
+ * Arguments are checked before any device work. */
+int me_mbar_words(me_engine *eng, int32_t n_target, int32_t with_obs, int64_t *words);
+int me_mbar_pass(me_engine *eng, const double *ts, int64_t rows, int64_t row0, int64_t stride, const double *f,
+                 int64_t n_per_state, int32_t n_target, const double *target_temps, const double *target_consts,
+                 int32_t with_obs, double *sums, int32_t accumulate, void *stream);
 
 const char *me_last_error(me_engine *eng);   /* eng may be NULL: error of the last failing me_create */
 

@@ -42,7 +42,7 @@ struct KernelRef {
     bool valid() const { return rt != nullptr || drv != nullptr; }
 };
 struct KernelSet {
-    KernelRef run, init, propose, accept, energy, run_mp, run_pt, run_hx;
+    KernelRef run, init, propose, accept, energy, run_mp, run_pt, run_hx, mbar;
     bool valid() const { return run.valid(); }
 };
 
@@ -196,12 +196,14 @@ int nvrtc_compile(int n_real, int n_complex, int energy_id, const std::string &u
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_init(const __grid_constant__ MeParams p) { me::init_body<UserCfg>(p); }\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_propose(const __grid_constant__ MeParams p) { me::propose_body<UserCfg>(p); }\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_accept(const __grid_constant__ MeParams p) { me::accept_body<UserCfg>(p); }\n"
-           "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_energy(const __grid_constant__ MeParams p) { me::energy_body<UserCfg>(p); }\n";
-    const char *hdr_names[] = {"me_params.h", "me_math.cuh", "me_device.cuh", "me_energies.cuh", "me_kernels.cuh"};
+           "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_energy(const __grid_constant__ MeParams p) { me::energy_body<UserCfg>(p); }\n"
+           "extern \"C\" __global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) me_k_mbar(const __grid_constant__ MeMbarParams q) { me::mbar_pass_body<UserCfg>(q); }\n";
+    const char *hdr_names[] = {"me_params.h", "me_math.cuh", "me_device.cuh", "me_energies.cuh", "me_kernels.cuh",
+                               "me_mbar.cuh"};
     const char *hdr_src[] = {me_src_params_h, me_src_math_cuh, me_src_device_cuh, me_src_energies_cuh,
-                             me_src_kernels_cuh};
+                             me_src_kernels_cuh, me_src_mbar_cuh};
     nvrtcProgram prog = nullptr;
-    int rc = n.createProgram(&prog, src.c_str(), "me_user_kernels.cu", 5, hdr_src, hdr_names);
+    int rc = n.createProgram(&prog, src.c_str(), "me_user_kernels.cu", 6, hdr_src, hdr_names);
     if (rc != 0) { log = std::string("nvrtcCreateProgram: ") + n.getErrorString(rc); return ME_ERR_COMPILE; }
     std::string d_nr = "-DME_NR=" + std::to_string(n_real), d_nc = "-DME_NC=" + std::to_string(n_complex);
     std::string d_st = std::string("-DME_STRICT=") + (strict ? "1" : "0");
@@ -233,11 +235,11 @@ int me_rt_compile(const std::string &src, const char *name, const std::vector<st
     Nvrtc &n = nvrtc();
     if (!n.ok) { log = n.err; return ME_ERR_UNSUPPORTED; }
     const char *hdr_names[] = {"me_params.h", "me_math.cuh", "me_device.cuh", "me_energies.cuh", "me_kernels.cuh",
-                               "me_k4_device.cuh", "me_generic.cuh"};
+                               "me_k4_device.cuh", "me_generic.cuh", "me_mbar.cuh"};
     const char *hdr_src[] = {me_src_params_h, me_src_math_cuh, me_src_device_cuh, me_src_energies_cuh, me_src_kernels_cuh,
-                             me_src_k4_device_cuh, me_src_generic_cuh};
+                             me_src_k4_device_cuh, me_src_generic_cuh, me_src_mbar_cuh};
     nvrtcProgram prog = nullptr;
-    int rc = n.createProgram(&prog, src.c_str(), name, 7, hdr_src, hdr_names);
+    int rc = n.createProgram(&prog, src.c_str(), name, 8, hdr_src, hdr_names);
     if (rc != 0) { log = std::string("nvrtcCreateProgram: ") + n.getErrorString(rc); return ME_ERR_COMPILE; }
     std::vector<const char *> opts = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo", "-DME_NVRTC=1"};
     for (auto &o : extra) opts.push_back(o.c_str());
@@ -366,6 +368,9 @@ struct me_engine {
     /* Hamiltonian ladder (me_set_hamiltonian_ladder): rung_k > 0 runs the HX instantiation */
     double *rung_consts = nullptr;             /* [R][rung_k] functor constants of each rung, device memory */
     int rung_k = 0;
+    std::vector<double> rung_temps_host, rung_consts_host;   /* host copies: the states of an MBAR pass (me_mbar_pass) */
+    double *mbar_buf = nullptr;                /* MBAR pass: per-CTA partial rows, then the reduced row */
+    size_t mbar_cap = 0;                       /* doubles */
     std::string err;
 };
 
@@ -647,7 +652,7 @@ int resolve_kernels(me_engine *e, int energy_id, const std::string &user_src) {
             if (t[i].n_real == nr && t[i].n_complex == nc && t[i].energy_id == energy_id) {
                 e->ks.run.rt = t[i].run; e->ks.init.rt = t[i].init; e->ks.run_mp.rt = t[i].run_mp;
                 e->ks.propose.rt = t[i].propose; e->ks.accept.rt = t[i].accept; e->ks.energy.rt = t[i].energy;
-                e->ks.run_pt.rt = t[i].run_pt; e->ks.run_hx.rt = t[i].run_hx;
+                e->ks.run_pt.rt = t[i].run_pt; e->ks.run_hx.rt = t[i].run_hx; e->ks.mbar.rt = t[i].mbar;
                 return ME_OK;
             }
     }
@@ -681,6 +686,7 @@ int resolve_kernels(me_engine *e, int energy_id, const std::string &user_src) {
         d.moduleGetFunction(&ks.energy.drv, mod, "me_k_energy") != CUDA_SUCCESS ||
         d.moduleGetFunction(&ks.run_pt.drv, mod, "me_k_run_pt") != CUDA_SUCCESS ||
         d.moduleGetFunction(&ks.run_hx.drv, mod, "me_k_run_hx") != CUDA_SUCCESS ||
+        d.moduleGetFunction(&ks.mbar.drv, mod, "me_k_mbar") != CUDA_SUCCESS ||
         (e->cfg.n_complex > 0 && d.moduleGetFunction(&ks.run_mp.drv, mod, "me_k_run_mp") != CUDA_SUCCESS))
         return fail(e, ME_ERR_CUDA, "cuModuleGetFunction failed on the runtime-compiled module");
     g_cache[key] = ks;
@@ -856,6 +862,79 @@ __global__ void k_equil_pick(const double *g_t, const double *neff_t, long long 
     neff_out[t_id] = bn;
 }
 
+/* Geometry of an MBAR pass (me_mbar.cuh): the 8-row blocks of the staged rows, the tile list in the order k_mbar_unpack
+ * reads it — [s: (W_i, ONE)] [G: (W_i, W_j), j <= i] and with observables [(WE_i, ONE)] [(WE2_i, ONE)] [(W_i, XX_j)] —
+ * and the length of the documented sums vector (me_b200.h, me_mbar_pass). */
+struct MbarLayout {
+    int S, nb, nx, n_tiles, z_rows, rw;
+    long long words;
+    unsigned char ta[ME_MBAR_MAX_TILES], tb[ME_MBAR_MAX_TILES];
+};
+void mbar_layout(int d, int n_states, int obs, MbarLayout &m) {
+    m.S = n_states;
+    m.nb = (n_states + 7) / 8;
+    m.nx = obs ? (2 * d + 7) / 8 : 0;
+    const int nb = m.nb;
+    int t = 0;
+    auto add = [&](int a, int b) { m.ta[t] = (unsigned char)a; m.tb[t] = (unsigned char)b; t++; };
+    for (int i = 0; i < nb; i++) add(i, nb);
+    for (int i = 0; i < nb; i++)
+        for (int j = 0; j <= i; j++) add(i, j);
+    if (obs) {
+        for (int i = 0; i < nb; i++) add(nb + 1 + i, nb);
+        for (int i = 0; i < nb; i++) add(2 * nb + 1 + i, nb);
+        for (int i = 0; i < nb; i++)
+            for (int j = 0; j < m.nx; j++) add(i, 3 * nb + 1 + j);
+    }
+    m.n_tiles = t;
+    m.z_rows = 8 * (obs ? 3 * nb + 1 + m.nx : 2 * nb + 1);
+    m.rw = 3 + 64 * t;
+    m.words = 3 + n_states + (long long)n_states * (n_states + 1) / 2 + (obs ? (long long)n_states * (2 * d + 2) : 0);
+}
+
+/* reduced partial row [sum L, n_nan, n_overflow, tiles[n_tiles][8][8]] -> the sums vector of me_mbar_pass
+   (sums = that, or sums += that) */
+__global__ void k_mbar_unpack(const double *raw, double *sums, int S, int nb, int nx, int d, long long words, int accumulate) {
+    const long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= words) return;
+    const double *tile = raw + 3;
+    const int we0 = nb + nb * (nb + 1) / 2, we20 = we0 + nb, xx0 = we20 + nb;
+    long long o = w - 3;
+    double v;
+    if (w < 3) {
+        v = raw[w];
+    } else if (o < S) {
+        v = tile[(o / 8) * 64 + (o % 8) * 8];
+    } else if ((o -= S) < (long long)S * (S + 1) / 2) {
+        int s = 0;
+        while ((long long)(s + 1) * (s + 2) / 2 <= o) s++;
+        const int t = (int)(o - (long long)s * (s + 1) / 2), i = s / 8, j = t / 8;
+        v = tile[(nb + i * (i + 1) / 2 + j) * 64 + (s % 8) * 8 + t % 8];
+    } else {
+        o -= (long long)S * (S + 1) / 2;
+        const int s = (int)(o / (2 * d + 2)), a = (int)(o % (2 * d + 2));
+        if (a < 2 * d) v = tile[(xx0 + (s / 8) * nx + a / 8) * 64 + (s % 8) * 8 + a % 8];
+        else v = tile[((a == 2 * d ? we0 : we20) + s / 8) * 64 + (s % 8) * 8];
+    }
+    sums[w] = accumulate ? sums[w] + v : v;
+}
+
+/* the checks me_mbar_words and me_mbar_pass share: shape, functor, mode and state count */
+int mbar_check(me_engine *e, int n_target) {
+    if (e->generic) return fail(e, ME_ERR_UNSUPPORTED, "MBAR passes need a fused shape (n_real + 2 n_complex <= 32)");
+    if (e->energy_id == ME_ENERGY_EXTERNAL)
+        return fail(e, ME_ERR_UNSUPPORTED, "MBAR passes re-evaluate a device energy functor; this handle's energies are "
+                                           "evaluated by the caller");
+    if (e->group != 0)
+        return fail(e, ME_ERR_UNSUPPORTED, "MBAR passes serve handles that step all parameters (group 0), not group-wise or "
+                                           "magnitude-phase modes");
+    if (e->energy_id < 0) return fail(e, ME_ERR_STATE, "no energy functor registered (call me_set_energy_* first)");
+    if (e->n_rungs > ME_MBAR_MAX_STATES) return fail(e, ME_ERR_INVALID, "MBAR passes take at most 32 rungs");
+    if (n_target < 0 || e->n_rungs + n_target > ME_MBAR_MAX_STATES)
+        return fail(e, ME_ERR_INVALID, "MBAR passes take at most 32 states (rungs + targets) and n_target >= 0");
+    return ME_OK;
+}
+
 }  // namespace
 
 /* ========================================================================================= C ABI */
@@ -910,8 +989,9 @@ int me_create(const me_config *cfg, me_engine **out) {
 }
 
 int me_destroy(me_engine *e) {
-    if (e && (e->seg_flags || e->ctr_dev || e->pool_partial || e->ladder_dev || e->rung_consts)) {
+    if (e && (e->seg_flags || e->ctr_dev || e->pool_partial || e->ladder_dev || e->rung_consts || e->mbar_buf)) {
         DeviceGuard g(e->cfg.device);
+        if (e->mbar_buf) cudaFree(e->mbar_buf);
         if (e->ladder_dev) cudaFree(e->ladder_dev);
         if (e->rung_consts) cudaFree(e->rung_consts);
         if (e->seg_flags) cudaFree(e->seg_flags);
@@ -1040,6 +1120,8 @@ int me_set_hamiltonian_ladder(me_engine *e, const double *temps, const double *c
         return fail(e, ME_ERR_CUDA, "allocating the ladder failed");
     }
     e->rung_k = ham ? n_consts : 0;
+    e->rung_temps_host.assign(temps, temps + n_rungs);
+    e->rung_consts_host.assign(consts ? consts : temps, consts ? consts + R * n_consts : temps);
     e->n_rungs = n_rungs;
     e->swap_every = swap_every;
     e->walker = walker;
@@ -1663,6 +1745,113 @@ int me_detect_equilibration(const double *ts, int64_t rows, int32_t cols, int64_
                                                           g_t, neff_t);
     k_equil_pick<<<gx, block, 0, (cudaStream_t)stream>>>(g_t, neff_t, n_cand, n_sel, nskip, t_out, g_out, neff_out);
     if (cudaGetLastError() != cudaSuccess) return ME_ERR_CUDA;
+    return ME_OK;
+}
+
+int me_mbar_words(me_engine *e, int32_t n_target, int32_t with_obs, int64_t *words) {
+    if (!e || !words) return ME_ERR_INVALID;
+    const int rc = mbar_check(e, n_target);
+    if (rc != ME_OK) return rc;
+    MbarLayout m;
+    mbar_layout(e->lay.D, e->n_rungs + n_target, with_obs ? 1 : 0, m);
+    *words = m.words;
+    return ME_OK;
+}
+
+int me_mbar_pass(me_engine *e, const double *ts, int64_t rows, int64_t row0, int64_t stride, const double *f,
+                 int64_t n_per_state, int32_t n_target, const double *target_temps, const double *target_consts,
+                 int32_t with_obs, double *sums, int32_t accumulate, void *stream) {
+    if (!e) return ME_ERR_INVALID;
+    int rc = mbar_check(e, n_target);
+    if (rc != ME_OK) return rc;
+    if (!ts || !f || !sums) return fail(e, ME_ERR_INVALID, "ts, f and sums are required");
+    if (n_target > 0 && !target_temps) return fail(e, ME_ERR_INVALID, "target_temps is required when n_target > 0");
+    if (rows < 1 || row0 < 0 || row0 >= rows) return fail(e, ME_ERR_INVALID, "row0 must lie in [0, rows)");
+    if (stride < 1) return fail(e, ME_ERR_INVALID, "stride must be >= 1");
+    if (n_per_state < 1) return fail(e, ME_ERR_INVALID, "n_per_state must be >= 1");
+    const int R = e->n_rungs, S = R + n_target;
+    const bool ham = e->rung_k > 0;
+    const int K = ham ? e->rung_k : e->n_consts;
+    if (n_target > 0 && ham && !target_consts)
+        return fail(e, ME_ERR_INVALID, "targets of a Hamiltonian ladder need their constants (target_consts)");
+    MeMbarParams q;
+    memset(&q, 0, sizeof(q));
+    for (int s = 0; s < S; s++) {
+        const double t = s < R ? (R > 1 ? e->rung_temps_host[s] : e->cfg.temp) : target_temps[s - R];
+        if (!std::isfinite(t) || !(t > 0))
+            return fail(e, ME_ERR_INVALID, std::string(s < R ? "every rung temperature" : "every target temperature") +
+                                               " must be finite and > 0 for MBAR");
+        q.inv_temp[s] = 1.0 / t;
+        for (int i = 0; i < ME_MAX_CONSTS; i++) {
+            double k = e->consts[i];
+            if (s < R && ham) k = i < K ? e->rung_consts_host[(size_t)s * K + i] : 0.0;
+            if (s >= R && target_consts) k = i < K ? target_consts[(size_t)(s - R) * K + i] : 0.0;
+            if (!std::isfinite(k)) return fail(e, ME_ERR_INVALID, "MBAR state constants must be finite");
+            q.consts[s][i] = k;
+        }
+    }
+    if (!e->ks.mbar.valid()) return fail(e, ME_ERR_STATE, "no MBAR kernel for this engine (device functors only)");
+    MbarLayout m;
+    mbar_layout(e->lay.D, S, with_obs ? 1 : 0, m);
+    const long long ld = e->cfg.n_chains, n_rows = (rows - row0 + stride - 1) / stride;
+    q.ts = ts; q.ld = ld; q.row0 = row0; q.stride = stride; q.n_samples = n_rows * ld;
+    q.ts_cols = e->lay.TS_COLS;
+    q.n_rungs = R; q.n_states = S; q.use_reject = e->use_reject;
+    q.nb = m.nb; q.nx = m.nx; q.n_tiles = m.n_tiles; q.z_rows = m.z_rows; q.rw = m.rw;
+    q.n_per_state = (double)n_per_state; q.log_n = std::log((double)n_per_state);
+    q.f = f;
+    memcpy(q.tile_a, m.ta, sizeof(m.ta));
+    memcpy(q.tile_b, m.tb, sizeof(m.tb));
+    /* CTAs of up to 4 warps inside the default 48 KB of shared memory; shapes whose one warp needs more opt in */
+    const int per_warp = (m.n_tiles * 64 + m.z_rows * ME_MBAR_LD) * 8, head = ME_MBAR_HEAD * 8;
+    int nw = (48 * 1024 - head) / per_warp;
+    nw = nw < 1 ? 1 : (nw > ME_MBAR_MAX_WARPS ? ME_MBAR_MAX_WARPS : nw);
+    const int smem = head + nw * per_warp;
+    const long long want = (q.n_samples + 32LL * nw - 1) / (32LL * nw);
+    const int grid = (int)(want < 8LL * e->n_sm ? want : 8LL * e->n_sm);
+    DeviceGuard g(e->cfg.device);
+    const size_t need = (size_t)(grid + 1) * m.rw;
+    if (need > e->mbar_cap) {
+        if (e->mbar_buf) cudaFree(e->mbar_buf);
+        e->mbar_buf = nullptr;
+        e->mbar_cap = 0;
+        if (cudaMalloc((void **)&e->mbar_buf, need * sizeof(double)) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(e, ME_ERR_CUDA, "allocating the MBAR partial rows failed");
+        }
+        e->mbar_cap = need;
+    }
+    q.partial = e->mbar_buf;
+    double *raw = e->mbar_buf + (size_t)grid * m.rw;
+    cudaStream_t st = (cudaStream_t)stream;
+    void *args[] = {&q};
+    const KernelRef &k = e->ks.mbar;
+    if (k.rt) {
+        if (smem > 48 * 1024 &&
+            cudaFuncSetAttribute(k.rt, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(e, ME_ERR_CUDA, "MBAR pass: cannot raise the kernel's shared-memory limit");
+        }
+        cudaError_t ce = cudaLaunchKernel(k.rt, dim3(grid), dim3(32 * nw), args, (size_t)smem, st);
+        if (ce != cudaSuccess) return fail(e, ME_ERR_CUDA, std::string("cudaLaunchKernel: ") + cudaGetErrorString(ce));
+    } else {
+        Driver &d = driver();
+        if (smem > 48 * 1024 &&
+            (!d.funcSetAttribute ||
+             d.funcSetAttribute(k.drv, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, smem) != CUDA_SUCCESS))
+            return fail(e, ME_ERR_CUDA, "MBAR pass: cannot raise the kernel's shared-memory limit");
+        CUresult r = d.launchKernel(k.drv, grid, 1, 1, 32 * nw, 1, 1, smem, (CUstream)st, args, nullptr);
+        if (r != CUDA_SUCCESS) {
+            const char *s = nullptr;
+            d.getErrorString(r, &s);
+            return fail(e, ME_ERR_CUDA, std::string("cuLaunchKernel: ") + (s ? s : "?"));
+        }
+    }
+    k_pool_reduce<<<m.rw, 256, 0, st>>>(q.partial, raw, grid, m.rw, 0);
+    k_mbar_unpack<<<(unsigned)((m.words + 127) / 128), 128, 0, st>>>(raw, sums, S, m.nb, m.nx, e->lay.D, m.words,
+                                                                    accumulate ? 1 : 0);
+    cudaError_t ce = cudaGetLastError();
+    if (ce != cudaSuccess) return fail(e, ME_ERR_CUDA, std::string("MBAR pass: ") + cudaGetErrorString(ce));
     return ME_OK;
 }
 

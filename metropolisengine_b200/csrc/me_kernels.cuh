@@ -5,6 +5,7 @@
 
 #include "me_device.cuh"
 #include "me_energies.cuh"
+#include "me_mbar.cuh"
 
 namespace me {
 
@@ -114,13 +115,24 @@ template <class C>
 __global__ void __launch_bounds__(ME_MAX_BLOCK) k_accept(const __grid_constant__ MeParams p) { accept_body<C>(p); }
 template <class C>
 __global__ void __launch_bounds__(ME_MAX_BLOCK) k_energy(const __grid_constant__ MeParams p) { energy_body<C>(p); }
+/* one MBAR pass over recorded rows (me_mbar_pass); CTAs of at most ME_MBAR_MAX_WARPS warps */
+template <class C>
+__global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) k_mbar(const __grid_constant__ MeMbarParams q) {
+    mbar_pass_body<C>(q);
+}
+#ifndef ME_NVRTC
+template <class C, bool EXT = IsExternal<C>::value>
+struct MbarKernel { static const void *get() { return (const void *)&k_mbar<C>; } };
+template <class C>
+struct MbarKernel<C, true> { static const void *get() { return nullptr; } };
+#endif
 
 }  // namespace me
 
 /* one ahead-of-time instantiation */
 struct MeAotEntry {
     int n_real, n_complex, energy_id, strict;
-    const void *run, *init, *propose, *accept, *run_mp, *energy, *run_pt, *run_hx;
+    const void *run, *init, *propose, *accept, *run_mp, *energy, *run_pt, *run_hx, *mbar;
 };
 
 #define ME_AOT_ENTRY(NR, NC, ETMPL, EID, STRICT)                                                        \
@@ -131,7 +143,8 @@ struct MeAotEntry {
       me::RunMpKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                             \
       (const void *)&me::k_energy<me::Cfg<NR, NC, ETMPL, STRICT>>,                                        \
       me::RunPtKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                             \
-      me::RunHxKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get() }
+      me::RunHxKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                             \
+      me::MbarKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get() }
 
 /* the shapes of BASELINE.json's configs plus the shapes of the golden fixtures */
 #define ME_AOT_TABLE(STRICT)                                                      \

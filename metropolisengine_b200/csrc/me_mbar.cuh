@@ -1,0 +1,176 @@
+/* me_mbar.cuh — one MBAR pass (Shirts & Chodera, J. Chem. Phys. 129, 124105, 2008) over recorded time-series rows
+ * (DESIGN §3 "MBAR over recorded ladder rows").
+ *
+ * Given the rungs' reduced free energies f[R], every sample x_n (one recorded row of one chain) contributes
+ *     L_n  = ln sum_k N_k exp(f_k - u_k(x_n))                 (k over the R rungs, max-shifted log-sum-exp)
+ *     w_ns = exp(f_s - u_s(x_n) - L_n)                        (s over the S output states; f = 0 for the targets)
+ * with u_s(x) = E(x; k_s) / T_s re-evaluated from the stored x columns (the stored E column is not read) and u_s = +inf
+ * where the functor's wall rejects x under k_s.  A pass returns the fixed-order sums
+ *     sum_n L_n,  s_s = sum_n w_ns,  G_st = sum_n w_ns w_nt,  sum_n w_ns [x, x^2, E_s, E_s^2]  (the latter optional)
+ * and the counts of samples with a NaN energy or a non-finite L_n, and of samples whose target weight exceeds 1e140
+ * (a target without overlap); such samples enter no sum.
+ *
+ * One thread per sample, chain-fastest, so the loads of each x column coalesce as the rows were written.  The energies
+ * and weights of a warp's 32 samples are staged column-wise in shared memory (z[row][lane], one column per lane), and all
+ * sums over samples are products with the 32 samples as the K dimension on the FP64 tensor cores (mma.m8n8k4, as
+ * pool_mma_update): tile (a, b) accumulates Z_a Z_b^T of two 8-row blocks of z.  Row blocks of z:
+ *     [0, nb)            w_s           (rows s < S; the rest stay 0)
+ *     nb                 ONE           (row 0 = 1, rows 1..7 = 0: a product with it is a plain sum over the samples)
+ *     [nb+1, 2nb+1)      E_s, then w_s E_s
+ *     [2nb+1, 3nb+1)     w_s E_s^2                            (observables only)
+ *     [3nb+1, 3nb+1+nx)  x_0..x_{D-1}, x_0^2..x_{D-1}^2      (observables only)
+ * Each warp adds its tile products to its own rows of shared memory after every 32 samples; at the end the CTA sums its
+ * warps in order and writes one partial row [sum L, n_nan, n_overflow, tiles[n_tiles][8][8]], which the host reduces
+ * with the fixed-order k_pool_reduce.  Every sum therefore has a fixed order for a given (samples, grid, block): a pass
+ * is bit-identical from run to run on one device. */
+#ifndef ME_MBAR_CUH
+#define ME_MBAR_CUH
+
+#include "me_device.cuh"
+
+#define ME_MBAR_LD 36                /* doubles per staged row: 32 samples + 4 of padding (fragment reads: two wavefronts) */
+#define ME_MBAR_HEAD 64              /* f[32], then [ME_MBAR_MAX_WARPS][4] per-warp scalar sums */
+#define ME_MBAR_MAX_WARPS 4
+#define ME_MBAR_OVERFLOW 1e140       /* w^2 summed over 10^10 samples stays finite */
+
+namespace me {
+
+template <class C>
+__device__ __forceinline__ void mbar_pass_body(const MeMbarParams &q) {
+    using L = Lay<C::NR, C::NC>;
+    using Energy = typename C::Energy;
+    constexpr int D = L::D, NR = L::NR, NC = L::NC;
+    extern __shared__ __align__(16) double me_mbar_smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    const int r8 = lane >> 2, k4 = lane & 3;
+    const int S = q.n_states, R = q.n_rungs, nb = q.nb;
+    double *fs = me_mbar_smem, *scal = me_mbar_smem + 32;
+    double *acc = me_mbar_smem + ME_MBAR_HEAD + (long long)warp * q.n_tiles * 64;
+    double(*z)[ME_MBAR_LD] =
+        reinterpret_cast<double(*)[ME_MBAR_LD]>(me_mbar_smem + ME_MBAR_HEAD + (long long)nw * q.n_tiles * 64) +
+        (long long)warp * q.z_rows;
+    const int W0 = 0, ONE = 8 * nb, E0 = 8 * (nb + 1), E20 = 8 * (2 * nb + 1), X0 = 8 * (3 * nb + 1);
+    const bool obs = q.nx > 0;
+
+    for (int i = threadIdx.x; i < 32; i += blockDim.x) fs[i] = i < R ? q.f[i] : 0.0;
+    for (int i = lane; i < q.n_tiles * 64; i += 32) acc[i] = 0.0;
+    for (int r = 0; r < q.z_rows; r++) z[r][lane] = r == ONE ? 1.0 : 0.0;
+    __syncthreads();
+
+    const long long per = (q.n_samples + gridDim.x - 1) / gridDim.x;
+    const long long lo = (long long)blockIdx.x * per;
+    const long long hi = lo + per < q.n_samples ? lo + per : q.n_samples;
+    double sum_l = 0.0, n_bad = 0.0, n_ovf = 0.0;
+    for (long long base = lo + 32LL * warp; base < hi; base += 32LL * nw) {   /* warp-uniform trip count */
+        const long long n = base + lane;
+        bool live = n < hi;
+        double x[D];
+        if (live) {
+            const long long i = n / q.ld, ch = n - i * q.ld;
+            const double *xp = q.ts + (q.row0 + i * q.stride) * (long long)q.ts_cols * q.ld + ch;
+#pragma unroll
+            for (int d = 0; d < D; d++) x[d] = xp[(long long)d * q.ld];
+        } else {
+#pragma unroll
+            for (int d = 0; d < D; d++) x[d] = 0.0;
+        }
+        /* energies of every output state (wall first, as in the step), staged in this lane's column */
+        bool bad = false;
+        unsigned walled = 0u;
+        if (live) {
+            for (int s = 0; s < S; s++) {
+                const double *k = q.consts[s];
+                const bool w = q.use_reject && Energy::reject(x, x + NR, x + NR + NC, k);
+                const double e = w ? 0.0 : Energy::eval(x, x + NR, x + NR + NC, k);
+                bad = bad || e != e;
+                walled |= (unsigned)w << s;
+                z[E0 + s][lane] = e;
+            }
+        }
+        /* L_n = ln N + m + ln sum_k exp(a_k - m),  a_k = f_k - u_k */
+        double m = -__longlong_as_double(0x7ff0000000000000LL);   /* -inf */
+        if (live && !bad)
+            for (int k = 0; k < R; k++)
+                if (!((walled >> k) & 1u)) m = fmax(m, fs[k] - z[E0 + k][lane] * q.inv_temp[k]);
+        double sum = 0.0;
+        if (live && !bad)
+            for (int k = 0; k < R; k++) {
+                const double ek = ((walled >> k) & 1u) ? 0.0 : exp(fs[k] - z[E0 + k][lane] * q.inv_temp[k] - m);
+                z[W0 + k][lane] = ek;
+                sum += ek;
+            }
+        const double l = q.log_n + m + log(sum);
+        if (live && !bad && !(fabs(l) <= 1.79e308)) bad = true;   /* every rung walled, or an infinite energy */
+        bool ovf = false;
+        if (live && !bad) {
+            const double sc = 1.0 / (q.n_per_state * sum);
+            for (int s = 0; s < S; s++) {
+                double w;
+                if (s < R) w = z[W0 + s][lane] * sc;
+                else w = ((walled >> s) & 1u) ? 0.0 : exp(-z[E0 + s][lane] * q.inv_temp[s] - l);
+                if (!(w <= ME_MBAR_OVERFLOW)) ovf = true;
+                z[W0 + s][lane] = w;
+            }
+        }
+        live = live && !bad && !ovf;
+        if (live) {
+            sum_l += l;
+            for (int s = 0; s < S; s++) {
+                const double w = z[W0 + s][lane], e = z[E0 + s][lane];
+                z[E0 + s][lane] = w * e;
+                if (obs) z[E20 + s][lane] = (w * e) * e;
+            }
+            if (obs) {
+#pragma unroll
+                for (int d = 0; d < D; d++) {
+                    z[X0 + d][lane] = x[d];
+                    z[X0 + D + d][lane] = x[d] * x[d];
+                }
+            }
+        } else {
+            n_bad += bad ? 1.0 : 0.0;
+            n_ovf += (!bad && ovf) ? 1.0 : 0.0;
+            for (int s = 0; s < S; s++) {
+                z[W0 + s][lane] = 0.0;
+                z[E0 + s][lane] = 0.0;
+                if (obs) z[E20 + s][lane] = 0.0;
+            }
+            if (obs)
+                for (int d = 0; d < 2 * D; d++) z[X0 + d][lane] = 0.0;
+        }
+        __syncwarp();
+        for (int t = 0; t < q.n_tiles; t++) {
+            const int ra = 8 * q.tile_a[t] + r8, rb = 8 * q.tile_b[t] + r8;
+            double c0 = 0.0, c1 = 0.0;
+#pragma unroll
+            for (int kk = 0; kk < 8; kk++) dmma_8x8x4(c0, c1, z[ra][4 * kk + k4], z[rb][4 * kk + k4]);
+            acc[t * 64 + 2 * lane] += c0;            /* C[r8][2 k4 + i] at r8 * 8 + 2 k4 + i: tiles are row-major */
+            acc[t * 64 + 2 * lane + 1] += c1;
+        }
+        __syncwarp();
+    }
+    sum_l = warp_sum(sum_l);
+    n_bad = warp_sum(n_bad);
+    n_ovf = warp_sum(n_ovf);
+    if (lane == 0) {
+        scal[4 * warp] = sum_l;
+        scal[4 * warp + 1] = n_bad;
+        scal[4 * warp + 2] = n_ovf;
+    }
+    __syncthreads();
+    double *row = q.partial + (long long)blockIdx.x * q.rw;
+    for (int w = threadIdx.x; w < q.rw; w += blockDim.x) {
+        double v = 0.0;
+        if (w < 3) {
+            for (int j = 0; j < nw; j++) v += scal[4 * j + w];
+        } else {
+            const double *a0 = me_mbar_smem + ME_MBAR_HEAD + (w - 3);
+            for (int j = 0; j < nw; j++) v += a0[(long long)j * q.n_tiles * 64];
+        }
+        row[w] = v;
+    }
+}
+
+}  // namespace me
+
+#endif

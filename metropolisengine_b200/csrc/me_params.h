@@ -5,7 +5,7 @@
 #ifndef ME_PARAMS_H
 #define ME_PARAMS_H
 
-#define ME_PARAMS_VERSION 12
+#define ME_PARAMS_VERSION 13
 #define ME_MAX_CONSTS 16
 
 /* status bits written to the per-chain STATUS word (SURVEY §5 "failure detection") */
@@ -82,6 +82,29 @@ struct MeParams {
     /* Hamiltonian ladder (me_set_hamiltonian_ladder; read by the HX instantiation of run_body and by init_body) */
     const double *rung_consts;     /* [n_rungs][n_consts] functor constants of each rung (NULL: consts on every chain) */
     int n_consts;                  /* K, 1 <= K <= ME_MAX_CONSTS */
+};
+
+/* One MBAR pass over recorded rows (me_mbar.cuh, me_mbar_pass).  A struct of its own so that MeParams, and with it the
+ * SASS of the step kernels, does not depend on the analysis.  The host fills the state table and the tile list. */
+#define ME_MBAR_MAX_STATES 32
+#define ME_MBAR_MAX_TILES 64
+struct MeMbarParams {
+    const double *ts;              /* [row][ts_cols][ld] time-series block of one storage chunk */
+    long long ld;                  /* chains per row (the handle's n_chains) */
+    long long row0, stride;        /* sample rows row0 + i stride, i < n_rows */
+    long long n_samples;           /* n_rows x ld; sample n = (row index n / ld, chain n % ld) */
+    int ts_cols;
+    int n_rungs, n_states;         /* R sampled states (the rungs), S = R + targets output states */
+    int use_reject;
+    int nb, nx, n_tiles, z_rows;   /* 8-row blocks of the weights and of [x, x^2]; tiles; staged rows per warp */
+    int rw;                        /* words of a partial row: 3 + 64 n_tiles */
+    double n_per_state;            /* N_k, the same for every rung */
+    double log_n;                  /* ln N_k */
+    const double *f;               /* [R] device: the rungs' reduced free energies */
+    double *partial;               /* [gridDim.x][rw] one row per CTA */
+    unsigned char tile_a[ME_MBAR_MAX_TILES], tile_b[ME_MBAR_MAX_TILES];   /* 8-row blocks of the staged rows */
+    double inv_temp[ME_MBAR_MAX_STATES];
+    double consts[ME_MBAR_MAX_STATES][ME_MAX_CONSTS];
 };
 
 #endif

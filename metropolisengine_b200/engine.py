@@ -1203,6 +1203,85 @@ class MetropolisEngine:
             raise ValueError("bad arguments to me_statistical_inefficiency")
         return g
 
+    # ------------------------------------------------------------------ MBAR over the recorded rows
+    def _mbar_sums(self, f, temps, consts, with_obs, row0, stride):
+        """One device pass (``me_mbar_pass``) over the recorded rows row0, row0 + stride, ... of every local chain,
+        storage chunk by storage chunk, summed over the ranks; returns the unpacked sums (``mbar.unpack``)."""
+        from . import mbar as _mbar
+        R, n_t = self.temperatures.size, int(np.size(temps))
+        n_rows = len(range(row0, self._ts_rows, stride))
+        n_per = n_rows * (self.n_chains_total // R)
+        words = ctypes.c_int64()
+        self._check(self._lib.me_mbar_words(self._h, n_t, int(with_obs), ctypes.byref(words)))
+        sums = torch.zeros(words.value, dtype=torch.float64, device=self.device)
+        f_dev = torch.tensor(np.asarray(f, dtype=np.float64), device=self.device)
+        tt = (ctypes.c_double * max(n_t, 1))(*np.asarray(temps, dtype=np.float64).ravel().tolist())
+        kk = None
+        if consts is not None:
+            arr = np.ascontiguousarray(consts, dtype=np.float64)
+            K = len(self._energy_spec.consts)
+            if arr.ndim != 2 or arr.shape != (n_t, K):
+                raise ValueError("target constants must be [n_target, %d] (the energy's constant count)" % K)
+            kk = ctypes.cast((ctypes.c_double * arr.size)(*arr.ravel().tolist()), ctypes.c_void_p)
+        g0, first = 0, True
+        for t, used in self._ts_chunks:
+            if not used:
+                continue
+            lo = max(row0, g0)
+            lo += (-(lo - row0)) % stride                  # first sampled row of this chunk
+            if lo < g0 + used:
+                self._launch(self._lib.me_mbar_pass(self._h, _ptr(t), used, lo - g0, stride, _ptr(f_dev), n_per, n_t,
+                                                    ctypes.cast(tt, ctypes.c_void_p), kk, int(with_obs), _ptr(sums),
+                                                    0 if first else 1, self._stream()))
+                first = False
+            g0 += used
+        if self._distributed:
+            comm = self._library_comm()
+            if comm is not None:
+                if self._lib.me_comm_allreduce(comm, _ptr(sums), sums.numel(), self._stream()) != _lib.ME_OK:
+                    raise _lib.MeError("MBAR all-reduce: " + self._lib.me_comm_last_error().decode(errors="replace"))
+            else:
+                parallel.allreduce_sum_(sums, self._group)
+        out = _mbar.unpack(sums.cpu().numpy(), R + n_t, self._d, with_obs)
+        if out["n_nan"]:
+            raise RuntimeError("MBAR pass: %d samples have a NaN energy or no finite log-sum over the rungs "
+                               "(status ME_STATUS_ENERGY_NAN)" % out["n_nan"])
+        if out["n_overflow"]:
+            raise RuntimeError("MBAR pass: a target state's weight overflowed on %d samples: the target has no "
+                               "overlap with the rungs" % out["n_overflow"])
+        return out
+
+    def mbar(self, burn_in=0.2, stride=1, tol=1e-10, max_iter=100):
+        """Reduced free energies of the rungs by MBAR (Shirts & Chodera 2008; pymbar's ``MBAR``) from the recorded rows,
+        evaluated on the device: every pass re-evaluates the energy functor with every rung's temperature and constants
+        from the stored parameters.  The first ``burn_in`` fraction of the rows is discarded, then every ``stride``-th
+        row of every chain is one sample.  The error estimate assumes uncorrelated samples: use ``stride`` of about the
+        statistical inefficiency of the energy column (``statistical_inefficiency(column=D)``).  Returns an
+        ``mbar.MBARResult`` (``free_energies`` with f_0 = 0, ``free_energy_errors``, ``n_iterations``, ``converged``;
+        ``evaluate()`` reweights to other temperatures or constants).  A scalar-``temp`` engine is a ladder of one rung."""
+        from . import mbar as _mbar
+        if self._d > 32:
+            raise NotImplementedError("MBAR needs n_real + 2 n_complex <= 32 (fused shapes)")
+        if self._callable is not None:
+            raise NotImplementedError("MBAR re-evaluates a device energy functor (BuiltinEnergy / CudaEnergy)")
+        if self.complex_sample_method == "magnitude-phase":
+            raise NotImplementedError("MBAR serves engines that step all parameters jointly, not magnitude-phase moves")
+        if not self.record:
+            raise RuntimeError("MBAR needs recorded rows: build the engine with record=True")
+        stride = int(stride)
+        if stride < 1:
+            raise ValueError("stride must be >= 1")
+        if not 0 <= burn_in < 1:
+            raise ValueError("burn_in is a fraction in [0, 1)")
+        row0 = int(self._ts_rows * burn_in)
+        if row0 >= self._ts_rows:
+            raise RuntimeError("MBAR: no recorded rows left after burn-in")
+        R = self.temperatures.size
+        n_per = len(range(row0, self._ts_rows, stride)) * (self.n_chains_total // R)
+        f, sums, it, conv = _mbar.solve(lambda f: self._mbar_sums(f, np.zeros(0), None, False, row0, stride), R, n_per,
+                                        tol, max_iter)
+        return _mbar.MBARResult(self, f, sums, it, conv, n_per, (row0, stride))
+
     def _equilibration_kernel(self, block, col, n_sel, nskip, fast=True):
         """(t0, g, Neff_max) tensors [n_sel] for column ``col`` of a block [rows, cols, ld] on the device."""
         rows, cols, ld = block.shape

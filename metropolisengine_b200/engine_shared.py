@@ -45,6 +45,10 @@ class SharedEnergy:
 
 
 class SharedCovarianceEngine:
+    def mbar(self, *args, **kwargs):
+        """MBAR passes run on the per-chain engine's fused shapes only (``MetropolisEngine.mbar``)."""
+        raise NotImplementedError("MBAR is not available for shared-covariance engines")
+
     def __init__(self, energy_consts=(10.0, -1.0, 0.05, 1.0), reject_condition=True, initial_real_params=None,
                  initial_complex_params=None, sampling_width=0.05, covariance_matrix_real=None,
                  covariance_matrix_complex=None, params_names=None, target_acceptance=.3, temp=0, *, n_chains=128,
