@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define ME_ABI_VERSION 8
+#define ME_ABI_VERSION 9
 
 enum me_status_code {
     ME_OK = 0,
@@ -420,6 +420,41 @@ int me_mbar_words(me_engine *eng, int32_t n_target, int32_t with_obs, int64_t *w
 int me_mbar_pass(me_engine *eng, const double *ts, int64_t rows, int64_t row0, int64_t stride, const double *f,
                  int64_t n_per_state, int32_t n_target, const double *target_temps, const double *target_consts,
                  int32_t with_obs, double *sums, int32_t accumulate, void *stream);
+
+/* MBAR free-energy profiles (pymbar's histogram FES: pymbar 4 FES, pymbar 3 computePMF): one histogram pass over the
+ * samples of me_mbar_pass (rows [row0, rows) of one storage chunk, every stride-th row, every local chain) with its
+ * weights at the rungs' f[R] (device):
+ *     L_n = ln sum_k N exp(f_k - u_k(x_n)),  w_nt = exp(-u_t(x_n) - L_n),  w_nk = exp(f_k - u_k(x_n) - L_n)
+ * for one target state t = (target_temp, target_consts[K]; NULL: the handle's constants, not allowed on a Hamiltonian
+ * ladder).  A walled x has u = +inf.  Samples with a NaN energy or a non-finite L_n count in n_nan, samples whose
+ * target weight exceeds 1e140 in n_overflow; neither enters a sum.
+ * Coordinates: n_axes in {1, 2}; axis a is stored parameter column coord_index[a] in [0, D) (order real, Re c, Im c)
+ * when coord_kind[a] = 0, or the modulus |c_j| = sqrt(Re c_j^2 + Im c_j^2) of complex parameter j = coord_index[a] in
+ * [0, n_complex) when coord_kind[a] = 1.  Uniform bins on [lo[a], hi[a]) (finite, hi > lo), n_bins[a] >= 1:
+ *     i = floor((c - lo) * inv_w),  inv_w = n / (hi - lo) rounded once;  in range iff lo <= c < hi (NaN is not);
+ *     i = n becomes n - 1;  bin b = i_0 n_bins[1] + i_1 in 2-D;  B = prod n_bins.
+ * The coordinate, modulus and index are computed with round-to-nearest operations (no FMA contraction), so every
+ * sample falls in the same bin in both builds and in a restatement in IEEE FP64.
+ * Sums (accumulate = 0: written; != 0: added), words = 4 + B (R + 2) (me_mbar_hist_words):
+ *     sums[0] = n_nan, sums[1] = n_overflow, sums[2] = w_out = sum of w_nt over out-of-range samples, sums[3] = their
+ *     count, then per bin b: h_b = sum_{n in b} w_nt, q_b = sum_{n in b} w_nt^2, c_bk = sum_{n in b} w_nt w_nk (k < R).
+ * Plain FP64 sums: chunks accumulate and ranks all-reduce them as they are.  A pass is bit-identical from run to run on
+ * one device.  B (R + 2) <= 24576.
+ * Finishing on the host (metropolisengine_b200/mbar.py, pmf): f_b = -ln h_b reported as f_b - f_ref;
+ * p_b = h_b / (sum h + w_out); uncertainties from Theta (me_mbar_pass) of the augmented Gram matrix over the R rungs
+ * and the non-empty bins: G_RR = the rungs' G at the solution, G_bk = c_bk / h_b, G_bb = q_b / h_b^2, G_bb' = 0, with
+ * N = [N .. N, 0 .. 0]: df_b = sqrt(Theta_bb + Theta_rr - 2 Theta_br) against the reference bin r (the lowest f, or a
+ * given bin).  An empty bin has f = +inf and df = NaN and stays out of Theta.
+ * ME_ERR_INVALID (with a message): n_axes not 1 or 2, an unknown coord_kind, a column outside [0, D) or a modulus index
+ * outside [0, n_complex), non-finite lo or hi or hi <= lo, n_bins < 1 or B (R + 2) > 24576, a target temperature not
+ * finite or not > 0, non-finite constants, no target_consts on a Hamiltonian ladder, the row0 / stride / n_per_state
+ * rules and null pointers of me_mbar_pass.  ME_ERR_UNSUPPORTED as me_mbar_pass.  Arguments are checked before any
+ * device work. */
+int me_mbar_hist_words(me_engine *eng, int32_t n_axes, const int32_t *n_bins, int64_t *words);
+int me_mbar_hist_pass(me_engine *eng, const double *ts, int64_t rows, int64_t row0, int64_t stride, const double *f,
+                      int64_t n_per_state, double target_temp, const double *target_consts, int32_t n_axes,
+                      const int32_t *coord_kind, const int32_t *coord_index, const double *lo, const double *hi,
+                      const int32_t *n_bins, double *sums, int32_t accumulate, void *stream);
 
 const char *me_last_error(me_engine *eng);   /* eng may be NULL: error of the last failing me_create */
 

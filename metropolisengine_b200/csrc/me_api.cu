@@ -42,7 +42,7 @@ struct KernelRef {
     bool valid() const { return rt != nullptr || drv != nullptr; }
 };
 struct KernelSet {
-    KernelRef run, init, propose, accept, energy, run_mp, run_pt, run_hx, mbar;
+    KernelRef run, init, propose, accept, energy, run_mp, run_pt, run_hx, mbar, mbar_hist;
     bool valid() const { return run.valid(); }
 };
 
@@ -197,7 +197,8 @@ int nvrtc_compile(int n_real, int n_complex, int energy_id, const std::string &u
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_propose(const __grid_constant__ MeParams p) { me::propose_body<UserCfg>(p); }\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_accept(const __grid_constant__ MeParams p) { me::accept_body<UserCfg>(p); }\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_energy(const __grid_constant__ MeParams p) { me::energy_body<UserCfg>(p); }\n"
-           "extern \"C\" __global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) me_k_mbar(const __grid_constant__ MeMbarParams q) { me::mbar_pass_body<UserCfg>(q); }\n";
+           "extern \"C\" __global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) me_k_mbar(const __grid_constant__ MeMbarParams q) { me::mbar_pass_body<UserCfg>(q); }\n"
+           "extern \"C\" __global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) me_k_mbar_hist(const __grid_constant__ MeMbarParams q) { me::mbar_hist_body<UserCfg>(q); }\n";
     const char *hdr_names[] = {"me_params.h", "me_math.cuh", "me_device.cuh", "me_energies.cuh", "me_kernels.cuh",
                                "me_mbar.cuh"};
     const char *hdr_src[] = {me_src_params_h, me_src_math_cuh, me_src_device_cuh, me_src_energies_cuh,
@@ -653,6 +654,7 @@ int resolve_kernels(me_engine *e, int energy_id, const std::string &user_src) {
                 e->ks.run.rt = t[i].run; e->ks.init.rt = t[i].init; e->ks.run_mp.rt = t[i].run_mp;
                 e->ks.propose.rt = t[i].propose; e->ks.accept.rt = t[i].accept; e->ks.energy.rt = t[i].energy;
                 e->ks.run_pt.rt = t[i].run_pt; e->ks.run_hx.rt = t[i].run_hx; e->ks.mbar.rt = t[i].mbar;
+                e->ks.mbar_hist.rt = t[i].mbar_hist;
                 return ME_OK;
             }
     }
@@ -687,6 +689,7 @@ int resolve_kernels(me_engine *e, int energy_id, const std::string &user_src) {
         d.moduleGetFunction(&ks.run_pt.drv, mod, "me_k_run_pt") != CUDA_SUCCESS ||
         d.moduleGetFunction(&ks.run_hx.drv, mod, "me_k_run_hx") != CUDA_SUCCESS ||
         d.moduleGetFunction(&ks.mbar.drv, mod, "me_k_mbar") != CUDA_SUCCESS ||
+        d.moduleGetFunction(&ks.mbar_hist.drv, mod, "me_k_mbar_hist") != CUDA_SUCCESS ||
         (e->cfg.n_complex > 0 && d.moduleGetFunction(&ks.run_mp.drv, mod, "me_k_run_mp") != CUDA_SUCCESS))
         return fail(e, ME_ERR_CUDA, "cuModuleGetFunction failed on the runtime-compiled module");
     g_cache[key] = ks;
@@ -932,6 +935,102 @@ int mbar_check(me_engine *e, int n_target) {
     if (e->n_rungs > ME_MBAR_MAX_STATES) return fail(e, ME_ERR_INVALID, "MBAR passes take at most 32 rungs");
     if (n_target < 0 || e->n_rungs + n_target > ME_MBAR_MAX_STATES)
         return fail(e, ME_ERR_INVALID, "MBAR passes take at most 32 states (rungs + targets) and n_target >= 0");
+    return ME_OK;
+}
+
+/* 1 / T and the functor constants [ME_MAX_CONSTS] of one MBAR state: rung r >= 0 (its temperature, and its constants on
+   a Hamiltonian ladder), or, r < 0, a target at temperature t with constants tk[K] (NULL: the handle's constants) */
+int mbar_state(me_engine *e, int r, double t, const double *tk, double &inv_temp, double *consts) {
+    const int R = e->n_rungs;
+    const bool ham = e->rung_k > 0;
+    const int K = ham ? e->rung_k : e->n_consts;
+    if (r >= 0) t = R > 1 ? e->rung_temps_host[r] : e->cfg.temp;
+    if (!std::isfinite(t) || !(t > 0))
+        return fail(e, ME_ERR_INVALID, std::string(r >= 0 ? "every rung temperature" : "every target temperature") +
+                                           " must be finite and > 0 for MBAR");
+    inv_temp = 1.0 / t;
+    for (int i = 0; i < ME_MAX_CONSTS; i++) {
+        double k = e->consts[i];
+        if (r >= 0 && ham) k = i < K ? e->rung_consts_host[(size_t)r * K + i] : 0.0;
+        if (r < 0 && tk) k = i < K ? tk[i] : 0.0;
+        if (!std::isfinite(k)) return fail(e, ME_ERR_INVALID, "MBAR state constants must be finite");
+        consts[i] = k;
+    }
+    return ME_OK;
+}
+
+/* Launch one MBAR-type pass kernel over q.n_samples samples and reduce its per-CTA rows of q.rw words in fixed order
+   into raw[q.rw] (device, inside the handle's buffer).  CTAs of up to 4 warps inside the default 48 KB of shared
+   memory; shapes whose one warp needs more (per_warp bytes) opt in.  At most 8 CTAs per SM; resident_only: no more than fit
+   the SMs' shared memory at once, so that wide partial rows (histograms) stay as few as can run together. */
+int mbar_launch(me_engine *e, const KernelRef &k, MeMbarParams &q, int per_warp, bool resident_only, cudaStream_t st,
+                double *&raw) {
+    const int head = ME_MBAR_HEAD * 8;
+    int nw = (48 * 1024 - head) / per_warp;
+    nw = nw < 1 ? 1 : (nw > ME_MBAR_MAX_WARPS ? ME_MBAR_MAX_WARPS : nw);
+    const int smem = head + nw * per_warp;
+    const long long want = (q.n_samples + 32LL * nw - 1) / (32LL * nw);
+    long long per_sm = 8;
+    if (resident_only && 233472 / (smem + 1024) < per_sm) per_sm = std::max(1, 233472 / (smem + 1024));
+    const long long cap = per_sm * e->n_sm;
+    const int grid = (int)(want < cap ? want : cap);
+    DeviceGuard g(e->cfg.device);
+    const size_t need = (size_t)(grid + 1) * q.rw;
+    if (need > e->mbar_cap) {
+        if (e->mbar_buf) cudaFree(e->mbar_buf);
+        e->mbar_buf = nullptr;
+        e->mbar_cap = 0;
+        if (cudaMalloc((void **)&e->mbar_buf, need * sizeof(double)) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(e, ME_ERR_CUDA, "allocating the MBAR partial rows failed");
+        }
+        e->mbar_cap = need;
+    }
+    q.partial = e->mbar_buf;
+    raw = e->mbar_buf + (size_t)grid * q.rw;
+    void *args[] = {&q};
+    if (k.rt) {
+        if (smem > 48 * 1024 &&
+            cudaFuncSetAttribute(k.rt, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(e, ME_ERR_CUDA, "MBAR pass: cannot raise the kernel's shared-memory limit");
+        }
+        cudaError_t ce = cudaLaunchKernel(k.rt, dim3(grid), dim3(32 * nw), args, (size_t)smem, st);
+        if (ce != cudaSuccess) return fail(e, ME_ERR_CUDA, std::string("cudaLaunchKernel: ") + cudaGetErrorString(ce));
+    } else {
+        Driver &d = driver();
+        if (smem > 48 * 1024 &&
+            (!d.funcSetAttribute ||
+             d.funcSetAttribute(k.drv, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, smem) != CUDA_SUCCESS))
+            return fail(e, ME_ERR_CUDA, "MBAR pass: cannot raise the kernel's shared-memory limit");
+        CUresult r = d.launchKernel(k.drv, grid, 1, 1, 32 * nw, 1, 1, smem, (CUstream)st, args, nullptr);
+        if (r != CUDA_SUCCESS) {
+            const char *s = nullptr;
+            d.getErrorString(r, &s);
+            return fail(e, ME_ERR_CUDA, std::string("cuLaunchKernel: ") + (s ? s : "?"));
+        }
+    }
+    k_pool_reduce<<<q.rw, 256, 0, st>>>(q.partial, raw, grid, q.rw, 0);
+    return ME_OK;
+}
+
+/* histogram pass: the reduced row already has the layout of the sums vector (me_mbar_hist_pass) */
+__global__ void k_mbar_hist_unpack(const double *raw, double *sums, long long words, int accumulate) {
+    const long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (w < words) sums[w] = accumulate ? sums[w] + raw[w] : raw[w];
+}
+
+/* bins of a histogram pass: B = prod n_bins over 1 or 2 axes, with B (R + 2) <= ME_MBAR_HIST_MAX_WORDS */
+int mbar_hist_bins(me_engine *e, int n_axes, const int32_t *n_bins, long long &B) {
+    if (n_axes != 1 && n_axes != 2) return fail(e, ME_ERR_INVALID, "n_axes must be 1 or 2");
+    if (!n_bins) return fail(e, ME_ERR_INVALID, "n_bins is required");
+    B = 1;
+    for (int a = 0; a < n_axes; a++) {
+        if (n_bins[a] < 1) return fail(e, ME_ERR_INVALID, "n_bins must be >= 1 on every axis");
+        B *= n_bins[a];
+        if (B * (e->n_rungs + 2) > ME_MBAR_HIST_MAX_WORDS)
+            return fail(e, ME_ERR_INVALID, "histogram too large: bins x (rungs + 2) must not exceed 24576 doubles");
+    }
     return ME_OK;
 }
 
@@ -1777,18 +1876,10 @@ int me_mbar_pass(me_engine *e, const double *ts, int64_t rows, int64_t row0, int
     MeMbarParams q;
     memset(&q, 0, sizeof(q));
     for (int s = 0; s < S; s++) {
-        const double t = s < R ? (R > 1 ? e->rung_temps_host[s] : e->cfg.temp) : target_temps[s - R];
-        if (!std::isfinite(t) || !(t > 0))
-            return fail(e, ME_ERR_INVALID, std::string(s < R ? "every rung temperature" : "every target temperature") +
-                                               " must be finite and > 0 for MBAR");
-        q.inv_temp[s] = 1.0 / t;
-        for (int i = 0; i < ME_MAX_CONSTS; i++) {
-            double k = e->consts[i];
-            if (s < R && ham) k = i < K ? e->rung_consts_host[(size_t)s * K + i] : 0.0;
-            if (s >= R && target_consts) k = i < K ? target_consts[(size_t)(s - R) * K + i] : 0.0;
-            if (!std::isfinite(k)) return fail(e, ME_ERR_INVALID, "MBAR state constants must be finite");
-            q.consts[s][i] = k;
-        }
+        const double *tk = target_consts && s >= R ? target_consts + (size_t)(s - R) * K : nullptr;
+        rc = s < R ? mbar_state(e, s, 0.0, nullptr, q.inv_temp[s], q.consts[s])
+                   : mbar_state(e, -1, target_temps[s - R], tk, q.inv_temp[s], q.consts[s]);
+        if (rc != ME_OK) return rc;
     }
     if (!e->ks.mbar.valid()) return fail(e, ME_ERR_STATE, "no MBAR kernel for this engine (device functors only)");
     MbarLayout m;
@@ -1802,56 +1893,94 @@ int me_mbar_pass(me_engine *e, const double *ts, int64_t rows, int64_t row0, int
     q.f = f;
     memcpy(q.tile_a, m.ta, sizeof(m.ta));
     memcpy(q.tile_b, m.tb, sizeof(m.tb));
-    /* CTAs of up to 4 warps inside the default 48 KB of shared memory; shapes whose one warp needs more opt in */
-    const int per_warp = (m.n_tiles * 64 + m.z_rows * ME_MBAR_LD) * 8, head = ME_MBAR_HEAD * 8;
-    int nw = (48 * 1024 - head) / per_warp;
-    nw = nw < 1 ? 1 : (nw > ME_MBAR_MAX_WARPS ? ME_MBAR_MAX_WARPS : nw);
-    const int smem = head + nw * per_warp;
-    const long long want = (q.n_samples + 32LL * nw - 1) / (32LL * nw);
-    const int grid = (int)(want < 8LL * e->n_sm ? want : 8LL * e->n_sm);
-    DeviceGuard g(e->cfg.device);
-    const size_t need = (size_t)(grid + 1) * m.rw;
-    if (need > e->mbar_cap) {
-        if (e->mbar_buf) cudaFree(e->mbar_buf);
-        e->mbar_buf = nullptr;
-        e->mbar_cap = 0;
-        if (cudaMalloc((void **)&e->mbar_buf, need * sizeof(double)) != cudaSuccess) {
-            cudaGetLastError();
-            return fail(e, ME_ERR_CUDA, "allocating the MBAR partial rows failed");
-        }
-        e->mbar_cap = need;
-    }
-    q.partial = e->mbar_buf;
-    double *raw = e->mbar_buf + (size_t)grid * m.rw;
+    double *raw = nullptr;
+    rc = mbar_launch(e, e->ks.mbar, q, (m.n_tiles * 64 + m.z_rows * ME_MBAR_LD) * 8, false, (cudaStream_t)stream,
+                     raw);
+    if (rc != ME_OK) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    void *args[] = {&q};
-    const KernelRef &k = e->ks.mbar;
-    if (k.rt) {
-        if (smem > 48 * 1024 &&
-            cudaFuncSetAttribute(k.rt, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) {
-            cudaGetLastError();
-            return fail(e, ME_ERR_CUDA, "MBAR pass: cannot raise the kernel's shared-memory limit");
-        }
-        cudaError_t ce = cudaLaunchKernel(k.rt, dim3(grid), dim3(32 * nw), args, (size_t)smem, st);
-        if (ce != cudaSuccess) return fail(e, ME_ERR_CUDA, std::string("cudaLaunchKernel: ") + cudaGetErrorString(ce));
-    } else {
-        Driver &d = driver();
-        if (smem > 48 * 1024 &&
-            (!d.funcSetAttribute ||
-             d.funcSetAttribute(k.drv, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, smem) != CUDA_SUCCESS))
-            return fail(e, ME_ERR_CUDA, "MBAR pass: cannot raise the kernel's shared-memory limit");
-        CUresult r = d.launchKernel(k.drv, grid, 1, 1, 32 * nw, 1, 1, smem, (CUstream)st, args, nullptr);
-        if (r != CUDA_SUCCESS) {
-            const char *s = nullptr;
-            d.getErrorString(r, &s);
-            return fail(e, ME_ERR_CUDA, std::string("cuLaunchKernel: ") + (s ? s : "?"));
-        }
-    }
-    k_pool_reduce<<<m.rw, 256, 0, st>>>(q.partial, raw, grid, m.rw, 0);
     k_mbar_unpack<<<(unsigned)((m.words + 127) / 128), 128, 0, st>>>(raw, sums, S, m.nb, m.nx, e->lay.D, m.words,
                                                                     accumulate ? 1 : 0);
     cudaError_t ce = cudaGetLastError();
     if (ce != cudaSuccess) return fail(e, ME_ERR_CUDA, std::string("MBAR pass: ") + cudaGetErrorString(ce));
+    return ME_OK;
+}
+
+int me_mbar_hist_words(me_engine *e, int32_t n_axes, const int32_t *n_bins, int64_t *words) {
+    if (!e || !words) return ME_ERR_INVALID;
+    int rc = mbar_check(e, 0);
+    if (rc != ME_OK) return rc;
+    long long B = 0;
+    rc = mbar_hist_bins(e, n_axes, n_bins, B);
+    if (rc != ME_OK) return rc;
+    *words = 4 + B * (e->n_rungs + 2);
+    return ME_OK;
+}
+
+int me_mbar_hist_pass(me_engine *e, const double *ts, int64_t rows, int64_t row0, int64_t stride, const double *f,
+                      int64_t n_per_state, double target_temp, const double *target_consts, int32_t n_axes,
+                      const int32_t *coord_kind, const int32_t *coord_index, const double *lo, const double *hi,
+                      const int32_t *n_bins, double *sums, int32_t accumulate, void *stream) {
+    if (!e) return ME_ERR_INVALID;
+    int rc = mbar_check(e, 0);
+    if (rc != ME_OK) return rc;
+    if (!ts || !f || !sums) return fail(e, ME_ERR_INVALID, "ts, f and sums are required");
+    if (!coord_kind || !coord_index || !lo || !hi)
+        return fail(e, ME_ERR_INVALID, "coord_kind, coord_index, lo and hi are required");
+    long long B = 0;
+    rc = mbar_hist_bins(e, n_axes, n_bins, B);
+    if (rc != ME_OK) return rc;
+    MeMbarParams q;
+    memset(&q, 0, sizeof(q));
+    for (int a = 0; a < n_axes; a++) {
+        if (coord_kind[a] == 0) {
+            if (coord_index[a] < 0 || coord_index[a] >= e->lay.D)
+                return fail(e, ME_ERR_INVALID, "a column coordinate must lie in [0, D)");
+        } else if (coord_kind[a] == 1) {
+            if (coord_index[a] < 0 || coord_index[a] >= e->cfg.n_complex)
+                return fail(e, ME_ERR_INVALID, "a modulus coordinate must name a complex parameter in [0, n_complex)");
+        } else {
+            return fail(e, ME_ERR_INVALID, "coord_kind must be 0 (column) or 1 (modulus of a complex parameter)");
+        }
+        if (!std::isfinite(lo[a]) || !std::isfinite(hi[a]) || !(hi[a] > lo[a]))
+            return fail(e, ME_ERR_INVALID, "every axis needs finite lo and hi with hi > lo");
+        q.axis_kind[a] = coord_kind[a];
+        q.axis_index[a] = coord_index[a];
+        q.axis_lo[a] = lo[a];
+        q.axis_hi[a] = hi[a];
+        q.axis_inv_w[a] = (double)n_bins[a] / (hi[a] - lo[a]);
+        q.n_bins[a] = n_bins[a];
+    }
+    if (rows < 1 || row0 < 0 || row0 >= rows) return fail(e, ME_ERR_INVALID, "row0 must lie in [0, rows)");
+    if (stride < 1) return fail(e, ME_ERR_INVALID, "stride must be >= 1");
+    if (n_per_state < 1) return fail(e, ME_ERR_INVALID, "n_per_state must be >= 1");
+    const int R = e->n_rungs;
+    const bool ham = e->rung_k > 0;
+    if (ham && !target_consts)
+        return fail(e, ME_ERR_INVALID, "the target of a Hamiltonian ladder needs its constants (target_consts)");
+    for (int s = 0; s < R; s++) {
+        rc = mbar_state(e, s, 0.0, nullptr, q.inv_temp[s], q.consts[s]);
+        if (rc != ME_OK) return rc;
+    }
+    rc = mbar_state(e, -1, target_temp, target_consts, q.t_inv_temp, q.t_consts);
+    if (rc != ME_OK) return rc;
+    if (!e->ks.mbar_hist.valid()) return fail(e, ME_ERR_STATE, "no MBAR kernel for this engine (device functors only)");
+    const long long ld = e->cfg.n_chains, n_rows = (rows - row0 + stride - 1) / stride;
+    q.ts = ts; q.ld = ld; q.row0 = row0; q.stride = stride; q.n_samples = n_rows * ld;
+    q.ts_cols = e->lay.TS_COLS;
+    q.n_rungs = R; q.n_states = R + 1; q.use_reject = e->use_reject;
+    q.n_axes = n_axes;
+    q.hw = (int)(B * (R + 2));
+    q.z_rows = 2 * (R + 1);
+    q.rw = 4 + q.hw;
+    q.n_per_state = (double)n_per_state; q.log_n = std::log((double)n_per_state);
+    q.f = f;
+    double *raw = nullptr;
+    rc = mbar_launch(e, e->ks.mbar_hist, q, (q.hw + q.z_rows * ME_MBAR_LD) * 8, true, (cudaStream_t)stream, raw);
+    if (rc != ME_OK) return rc;
+    k_mbar_hist_unpack<<<(unsigned)((q.rw + 127) / 128), 128, 0, (cudaStream_t)stream>>>(raw, sums, q.rw,
+                                                                                         accumulate ? 1 : 0);
+    cudaError_t ce = cudaGetLastError();
+    if (ce != cudaSuccess) return fail(e, ME_ERR_CUDA, std::string("MBAR histogram pass: ") + cudaGetErrorString(ce));
     return ME_OK;
 }
 

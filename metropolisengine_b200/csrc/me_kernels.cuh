@@ -120,11 +120,22 @@ template <class C>
 __global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) k_mbar(const __grid_constant__ MeMbarParams q) {
     mbar_pass_body<C>(q);
 }
+/* the histogram pass of free-energy profiles over the same rows (me_mbar_hist_pass) */
+template <class C>
+__global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) k_mbar_hist(const __grid_constant__ MeMbarParams q) {
+    mbar_hist_body<C>(q);
+}
 #ifndef ME_NVRTC
 template <class C, bool EXT = IsExternal<C>::value>
-struct MbarKernel { static const void *get() { return (const void *)&k_mbar<C>; } };
+struct MbarKernel {
+    static const void *get() { return (const void *)&k_mbar<C>; }
+    static const void *hist() { return (const void *)&k_mbar_hist<C>; }
+};
 template <class C>
-struct MbarKernel<C, true> { static const void *get() { return nullptr; } };
+struct MbarKernel<C, true> {
+    static const void *get() { return nullptr; }
+    static const void *hist() { return nullptr; }
+};
 #endif
 
 }  // namespace me
@@ -132,7 +143,7 @@ struct MbarKernel<C, true> { static const void *get() { return nullptr; } };
 /* one ahead-of-time instantiation */
 struct MeAotEntry {
     int n_real, n_complex, energy_id, strict;
-    const void *run, *init, *propose, *accept, *run_mp, *energy, *run_pt, *run_hx, *mbar;
+    const void *run, *init, *propose, *accept, *run_mp, *energy, *run_pt, *run_hx, *mbar, *mbar_hist;
 };
 
 #define ME_AOT_ENTRY(NR, NC, ETMPL, EID, STRICT)                                                        \
@@ -144,7 +155,8 @@ struct MeAotEntry {
       (const void *)&me::k_energy<me::Cfg<NR, NC, ETMPL, STRICT>>,                                        \
       me::RunPtKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                             \
       me::RunHxKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                             \
-      me::MbarKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get() }
+      me::MbarKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                              \
+      me::MbarKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::hist() }
 
 /* the shapes of BASELINE.json's configs plus the shapes of the golden fixtures */
 #define ME_AOT_TABLE(STRICT)                                                      \

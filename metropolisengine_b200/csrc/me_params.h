@@ -5,7 +5,7 @@
 #ifndef ME_PARAMS_H
 #define ME_PARAMS_H
 
-#define ME_PARAMS_VERSION 13
+#define ME_PARAMS_VERSION 14
 #define ME_MAX_CONSTS 16
 
 /* status bits written to the per-chain STATUS word (SURVEY §5 "failure detection") */
@@ -105,6 +105,15 @@ struct MeMbarParams {
     unsigned char tile_a[ME_MBAR_MAX_TILES], tile_b[ME_MBAR_MAX_TILES];   /* 8-row blocks of the staged rows */
     double inv_temp[ME_MBAR_MAX_STATES];
     double consts[ME_MBAR_MAX_STATES][ME_MAX_CONSTS];
+    /* histogram pass (me_mbar_hist_pass; appended so the fields above keep their offsets): n_states = R + 1, the
+     * target is the last state; bins b = i_0 n_bins[1] + i_1 over n_axes axes; hw = B (R + 2) words per histogram */
+    double t_inv_temp;             /* 1 / T_t of the target */
+    double t_consts[ME_MAX_CONSTS];
+    double axis_lo[2], axis_hi[2], axis_inv_w[2];   /* inv_w = n / (hi - lo), rounded once on the host */
+    int n_axes, hw;
+    int axis_kind[2];              /* 0: stored column axis_index; 1: modulus of complex parameter axis_index */
+    int axis_index[2], n_bins[2];
 };
+#define ME_MBAR_HIST_MAX_WORDS 24576   /* B (R + 2) doubles: one warp's histogram and staging fit the 227 KB opt-in */
 
 #endif

@@ -1223,6 +1223,16 @@ class MetropolisEngine:
             if arr.ndim != 2 or arr.shape != (n_t, K):
                 raise ValueError("target constants must be [n_target, %d] (the energy's constant count)" % K)
             kk = ctypes.cast((ctypes.c_double * arr.size)(*arr.ravel().tolist()), ctypes.c_void_p)
+        self._mbar_chunks(lambda t, used, lo, acc: self._lib.me_mbar_pass(
+            self._h, _ptr(t), used, lo, stride, _ptr(f_dev), n_per, n_t, ctypes.cast(tt, ctypes.c_void_p), kk,
+            int(with_obs), _ptr(sums), acc, self._stream()), sums, row0, stride)
+        out = _mbar.unpack(sums.cpu().numpy(), R + n_t, self._d, with_obs)
+        self._mbar_refuse(out)
+        return out
+
+    def _mbar_chunks(self, launch, sums, row0, stride):
+        """Run ``launch(chunk, rows used, first sampled row in the chunk, accumulate)`` over the storage chunks that
+        hold sampled rows (the first writes ``sums``, the rest add to it), then sum ``sums`` over the ranks."""
         g0, first = 0, True
         for t, used in self._ts_chunks:
             if not used:
@@ -1230,9 +1240,7 @@ class MetropolisEngine:
             lo = max(row0, g0)
             lo += (-(lo - row0)) % stride                  # first sampled row of this chunk
             if lo < g0 + used:
-                self._launch(self._lib.me_mbar_pass(self._h, _ptr(t), used, lo - g0, stride, _ptr(f_dev), n_per, n_t,
-                                                    ctypes.cast(tt, ctypes.c_void_p), kk, int(with_obs), _ptr(sums),
-                                                    0 if first else 1, self._stream()))
+                self._launch(launch(t, used, lo - g0, 0 if first else 1))
                 first = False
             g0 += used
         if self._distributed:
@@ -1242,13 +1250,43 @@ class MetropolisEngine:
                     raise _lib.MeError("MBAR all-reduce: " + self._lib.me_comm_last_error().decode(errors="replace"))
             else:
                 parallel.allreduce_sum_(sums, self._group)
-        out = _mbar.unpack(sums.cpu().numpy(), R + n_t, self._d, with_obs)
+
+    @staticmethod
+    def _mbar_refuse(out):
         if out["n_nan"]:
             raise RuntimeError("MBAR pass: %d samples have a NaN energy or no finite log-sum over the rungs "
                                "(status ME_STATUS_ENERGY_NAN)" % out["n_nan"])
         if out["n_overflow"]:
             raise RuntimeError("MBAR pass: a target state's weight overflowed on %d samples: the target has no "
                                "overlap with the rungs" % out["n_overflow"])
+
+    def _mbar_hist_sums(self, f, temp, consts, kinds, index, lo, hi, n_bins, row0, stride):
+        """One histogram pass (``me_mbar_hist_pass``) of the target (temp, consts [K] or None) over the rows row0,
+        row0 + stride, ... of every local chain, chunk by chunk, summed over the ranks; returns ``mbar.unpack_hist``."""
+        from . import mbar as _mbar
+        R, n_ax = self.temperatures.size, len(kinds)
+        n_per = len(range(row0, self._ts_rows, stride)) * (self.n_chains_total // R)
+        i32 = ctypes.c_int32 * n_ax
+        f64 = ctypes.c_double * n_ax
+        nb, kd, ix = i32(*n_bins), i32(*kinds), i32(*index)
+        lo_c, hi_c = f64(*np.asarray(lo, dtype=np.float64).tolist()), f64(*np.asarray(hi, dtype=np.float64).tolist())
+        words = ctypes.c_int64()
+        self._check(self._lib.me_mbar_hist_words(self._h, n_ax, ctypes.cast(nb, ctypes.c_void_p), ctypes.byref(words)))
+        kk = None
+        if consts is not None:
+            arr = np.ascontiguousarray(consts, dtype=np.float64).ravel()
+            K = len(self._energy_spec.consts)
+            if arr.size != K:
+                raise ValueError("target constants must be [%d] (the energy's constant count)" % K)
+            kk = ctypes.cast((ctypes.c_double * K)(*arr.tolist()), ctypes.c_void_p)
+        sums = torch.zeros(words.value, dtype=torch.float64, device=self.device)
+        f_dev = torch.tensor(np.asarray(f, dtype=np.float64), device=self.device)
+        vp = lambda a: ctypes.cast(a, ctypes.c_void_p)
+        self._mbar_chunks(lambda t, used, lo0, acc: self._lib.me_mbar_hist_pass(
+            self._h, _ptr(t), used, lo0, stride, _ptr(f_dev), n_per, float(temp), kk, n_ax, vp(kd), vp(ix), vp(lo_c),
+            vp(hi_c), vp(nb), _ptr(sums), acc, self._stream()), sums, row0, stride)
+        out = _mbar.unpack_hist(sums.cpu().numpy(), R, n_bins)
+        self._mbar_refuse(out)
         return out
 
     def mbar(self, burn_in=0.2, stride=1, tol=1e-10, max_iter=100):

@@ -8,7 +8,10 @@ free energies f; everything here is S x S algebra on those sums (S <= 32 states)
   line search on F (one pass per trial point) and the self-consistent step f_i <- f_i - ln s_i when the reduced Hessian
   is not positive definite;
 * pymbar's ``svd-ew`` asymptotic covariance Theta from the Gram matrix G of the weights;
-* target states: f_t = -ln s_t and <a>_t = sum_n w_nt a_t / s_t.
+* target states: f_t = -ln s_t and <a>_t = sum_n w_nt a_t / s_t;
+* free-energy profiles (pymbar's histogram FES): the histogram pass (``me_mbar_hist_pass``) sums a target's weights per
+  bin of one or two coordinates, and ``profile`` turns them into f_b, p_b and their errors by Theta over the rungs plus
+  one state per non-empty bin.
 
 The covariance assumes uncorrelated samples: pass ``stride`` of about the statistical inefficiency g of the energy
 column (``MetropolisEngine.statistical_inefficiency``).
@@ -44,6 +47,55 @@ def differences(th):
     """d(f_j - f_i) = sqrt(Theta_ii + Theta_jj - 2 Theta_ij), [S, S]."""
     dg = np.diag(th)
     return np.sqrt(np.clip(dg[:, None] + dg[None, :] - 2.0 * th, 0.0, None))
+
+
+def unpack_hist(sums, n_rungs, n_bins):
+    """The sums vector of ``me_mbar_hist_pass`` as a dict: ``n_nan``, ``n_overflow``, ``w_out``, ``n_out``, and per flat
+    bin ``h`` [B], ``q`` [B] and ``c`` [B, R]."""
+    R, B = n_rungs, int(np.prod(n_bins))
+    sums = np.asarray(sums, dtype=np.float64)
+    body = sums[4:4 + B * (R + 2)].reshape(B, R + 2)
+    return dict(n_nan=int(sums[0]), n_overflow=int(sums[1]), w_out=float(sums[2]), n_out=int(sums[3]),
+                h=body[:, 0].copy(), q=body[:, 1].copy(), c=body[:, 2:].copy())
+
+
+def profile(h, q, c, w_out, G, n_per_state, reference="lowest"):
+    """pymbar's histogram free-energy surface from the per-bin sums of one target (flat bins).
+
+    f_b = -ln h_b, reported as f_b - f_ref; p_b = h_b / (sum h + w_out).  Errors: Theta of the augmented Gram matrix
+    over the R rungs (G, the rung Gram matrix at the MBAR solution) and the non-empty bins, G_bk = c_bk / h_b,
+    G_bb = q_b / h_b^2, G_bb' = 0, with N = 0 for the bins; df_b = sqrt(Theta_bb + Theta_rr - 2 Theta_br).  reference:
+    "lowest" (the bin of smallest f) or a flat bin index.  Empty bins: f = +inf, df = NaN.  Returns (f, df, p)."""
+    h, q, c = np.asarray(h, dtype=np.float64), np.asarray(q, dtype=np.float64), np.asarray(c, dtype=np.float64)
+    R, B = G.shape[0], h.size
+    full = np.flatnonzero(h > 0)
+    f = np.full(B, np.inf)
+    f[full] = -np.log(h[full])
+    p = h / (h.sum() + w_out)
+    if isinstance(reference, str):
+        if reference != "lowest":
+            raise ValueError('reference is "lowest" or a bin index')
+        if full.size == 0:
+            raise ValueError("every bin is empty: the range holds none of the target's weight")
+        ref = int(full[np.argmin(f[full])])
+    else:
+        ref = int(reference)
+        if not 0 <= ref < B:
+            raise ValueError("the reference bin lies outside the bins")
+        if not h[ref] > 0:
+            raise ValueError("the reference bin is empty")
+    nb = full.size
+    Ga = np.zeros((R + nb, R + nb))
+    Ga[:R, :R] = G
+    gbk = c[full] / h[full, None]
+    Ga[R:, :R] = gbk
+    Ga[:R, R:] = gbk.T
+    Ga[np.arange(R, R + nb), np.arange(R, R + nb)] = q[full] / (h[full] * h[full])
+    th = theta(Ga, np.concatenate([np.full(R, float(n_per_state)), np.zeros(nb)]))
+    j = R + int(np.searchsorted(full, ref))
+    df = np.full(B, np.nan)
+    df[full] = np.sqrt(np.clip(np.diag(th)[R:] + th[j, j] - 2.0 * th[R:, j], 0.0, None))
+    return f - f[ref], df, p
 
 
 def solve(pass_fn, n_rungs, n_per_state, tol=1e-10, max_iter=100):
@@ -101,6 +153,7 @@ class MBARResult:
         self._sample = sample                 # (burn-in row, stride) of the solve
         self._n = float(n_per_state)
         R = f.size
+        self._G = sums["G"][:R, :R].copy()    # rung Gram matrix at the solution (profile errors)
         self.free_energies = f.copy()
         self.free_energy_errors = differences(theta(sums["G"][:R, :R], np.full(R, self._n)))
         self.n_iterations = int(n_iterations)
@@ -150,3 +203,69 @@ class MBARResult:
         sel = slice(R, S) if n_t else slice(0, R)
         return dict(f=f_all[sel].copy(), df=df_all[sel].copy(), x_mean=ob[sel, :d].copy(), x2_mean=ob[sel, d:2 * d].copy(),
                     E_mean=ob[sel, 2 * d].copy(), E2_mean=ob[sel, 2 * d + 1].copy())
+
+    def pmf(self, coords, bins, range, temp=None, consts=None, reference="lowest"):
+        """Free-energy profile of one target state along one or two coordinates (pymbar's histogram FES), from a device
+        histogram pass over the rows of the solve.
+
+        coords     an int (stored parameter column, order real, Re c, Im c), ("abs", j) (the modulus of complex
+                   parameter j), or a pair of those for a 2-D profile
+        bins       an int, or a pair (one per axis)
+        range      (lo, hi), or a pair of those; a sample counts iff lo <= c < hi on every axis
+        temp, consts  the target state, with the rules of ``evaluate``: consts is one [K] vector; both None: rung 0 (its
+                   temperature, and its constants on a Hamiltonian ladder)
+        reference  "lowest" (the bin of smallest f, pymbar's from-lowest) or a bin index (a pair in 2-D)
+
+        Returns a dict of numpy arrays: ``f`` and ``df`` shaped [n] or [n_x, n_y] (reduced free energy against the
+        reference bin and its standard error; empty bins: f = +inf, df = NaN), ``p`` (bin probabilities), ``edges``
+        (one array per axis) and ``weight_outside`` (the target's probability outside the range)."""
+        eng = self._engine
+        one = isinstance(coords, (int, np.integer)) or (isinstance(coords, (tuple, list)) and len(coords) == 2
+                                                        and isinstance(coords[0], str))
+        axes = [coords] if one else list(coords)
+        if not 1 <= len(axes) <= 2:
+            raise ValueError("coords names one or two axes")
+        n_ax = len(axes)
+        kinds, idx = [], []
+        for a in axes:
+            if isinstance(a, (int, np.integer)) and not isinstance(a, bool):
+                kinds.append(0)
+                idx.append(int(a))
+            elif isinstance(a, (tuple, list)) and len(a) == 2 and a[0] == "abs" and isinstance(a[1], (int, np.integer)):
+                kinds.append(1)
+                idx.append(int(a[1]))
+            else:
+                raise ValueError('a coordinate is a column index or ("abs", j), got %r' % (a,))
+        nb = [bins] if n_ax == 1 and np.ndim(bins) == 0 else list(np.ravel(bins))
+        rg = np.asarray(range, dtype=np.float64)
+        rg = rg.reshape(1, -1) if n_ax == 1 and rg.ndim == 1 else rg
+        if len(nb) != n_ax or rg.shape != (n_ax, 2):
+            raise ValueError("bins and range need one entry per axis")
+        if any(not isinstance(n, (int, np.integer)) or isinstance(n, bool) for n in nb):
+            raise ValueError("bins are integers")
+        nb = [int(n) for n in nb]
+        if temp is None and consts is None:
+            temp = eng.temperatures[0]
+            kt = None if eng.rung_consts is None else eng.rung_consts[0]
+        else:
+            if temp is None:
+                if eng.rung_consts is None and np.unique(eng.temperatures).size != 1:
+                    raise ValueError("give temp for the target of a temperature ladder")
+                temp = eng.temperatures[0]
+            kt = None if consts is None else np.asarray(consts, dtype=np.float64)
+        if np.size(temp) != 1 or (kt is not None and kt.ndim != 1):
+            raise ValueError("pmf takes one target state: a scalar temp and one [K] constant vector")
+        sums = eng._mbar_hist_sums(self.free_energies, float(np.asarray(temp).ravel()[0]), kt, kinds, idx, rg[:, 0],
+                                   rg[:, 1], nb, *self._sample)
+        if isinstance(reference, str):
+            ref = reference
+        else:
+            r = np.ravel(reference)
+            if r.size != n_ax or np.any(r < 0) or np.any(r >= np.array(nb)):
+                raise ValueError("the reference bin lies outside the bins")
+            ref = int(np.ravel_multi_index(tuple(int(v) for v in r), nb))
+        f, df, p = profile(sums["h"], sums["q"], sums["c"], sums["w_out"], self._G, self._n, ref)
+        shape = tuple(nb)
+        return dict(f=f.reshape(shape), df=df.reshape(shape), p=p.reshape(shape),
+                    edges=[np.linspace(rg[a, 0], rg[a, 1], nb[a] + 1) for a in np.arange(n_ax)],
+                    weight_outside=sums["w_out"] / (sums["h"].sum() + sums["w_out"]))
