@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define ME_ABI_VERSION 9
+#define ME_ABI_VERSION 10
 
 enum me_status_code {
     ME_OK = 0,
@@ -455,6 +455,38 @@ int me_mbar_hist_pass(me_engine *eng, const double *ts, int64_t rows, int64_t ro
                       int64_t n_per_state, double target_temp, const double *target_consts, int32_t n_axes,
                       const int32_t *coord_kind, const int32_t *coord_index, const double *lo, const double *hi,
                       const int32_t *n_bins, double *sums, int32_t accumulate, void *stream);
+
+/* MBAR expectation uncertainties (pymbar's compute_expectations covariance): one covariance pass over the samples and
+ * weights of me_mbar_pass (the same rows, rungs, targets, f[R] and S = R + n_target <= 32 states)
+ *     w_ns = exp(f_s - u_s(x_n) - L_n)
+ * for the covered states s in [cov_first, cov_first + cov_count) of those S.  The observables of state s are the ones
+ * me_mbar_pass averages, a_s = [x_0..x_{D-1}, x_0^2..x_{D-1}^2, E_s, E_s^2] (m = 2D + 2), taken about host-given
+ * centres: a~ = a_s - c_s with centers[c][m] (device) for covered state c = s - cov_first.  Samples with a NaN energy or
+ * a non-finite L_n count in n_nan, samples whose target weight exceeds 1e140 in n_overflow; neither enters a sum.
+ * Sums (accumulate = 0: written; != 0: added), words = 2 + cov_count (m + m (R + 1) + m (m + 1) / 2)
+ * (me_mbar_cov_words):
+ *     sums[0] = n_nan, sums[1] = n_overflow, then per covered state s:
+ *     o[m]          o_a = sum_n w_ns a~_a
+ *     C[m][R + 1]   C_ak = sum_n w_ns a~_a w_nk for the rungs k < R, then C_a* = sum_n w_ns^2 a~_a
+ *     Q[m(m+1)/2]   Q_ab = sum_n w_ns^2 a~_a a~_b, b <= a, lower-packed at a (a + 1) / 2 + b.
+ * Plain FP64 sums: chunks accumulate and ranks all-reduce them as they are.  A pass is bit-identical from run to run on
+ * one device.
+ * Finishing on the host (metropolisengine_b200/mbar.py, expectation_covariance), with s_s and G from me_mbar_pass at the
+ * same f: delta_a = o_a / s_s, <a>_s = c_a + delta_a; the centred column v_a = w_s (a - <a>_s) / s_s has the Gram entries
+ *     G(v_a, k)   = (C_ak - delta_a G_sk) / s_s
+ *     G(v_a, v_b) = (Q_ab - delta_a C_b* - delta_b C_a* + delta_a delta_b G_ss) / s_s^2
+ * and Theta (me_mbar_pass) over [the R rungs, v_0 .. v_{m-1}] with N = [N .. N, 0 .. 0] gives
+ * Cov(<a>_s, <b>_s) = Theta(v_a, v_b), for any centres (they only keep Q from cancelling when |<a>| >> std(a)).
+ * Uncorrelated samples are assumed, as for the free-energy errors.
+ * ME_ERR_INVALID (with a message): the rules of me_mbar_pass; cov_count < 1 or a range outside [0, S); null centers;
+ * a range whose tiles and staging for one warp exceed the 227 KB of shared memory (a single state always fits, so
+ * callers split the covered states into passes: me_mbar_cov_words applies the same check).  ME_ERR_UNSUPPORTED as
+ * me_mbar_pass.  Arguments are checked before any device work. */
+int me_mbar_cov_words(me_engine *eng, int32_t n_target, int32_t cov_first, int32_t cov_count, int64_t *words);
+int me_mbar_cov_pass(me_engine *eng, const double *ts, int64_t rows, int64_t row0, int64_t stride, const double *f,
+                     int64_t n_per_state, int32_t n_target, const double *target_temps, const double *target_consts,
+                     int32_t cov_first, int32_t cov_count, const double *centers, double *sums, int32_t accumulate,
+                     void *stream);
 
 const char *me_last_error(me_engine *eng);   /* eng may be NULL: error of the last failing me_create */
 

@@ -9,7 +9,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("ME_B200_LIB") or os.path.join(HERE, "lib", "libme_b200.so")   # override: kernel experiments
 
-ME_ABI_VERSION = 9
+ME_ABI_VERSION = 10
 
 ME_OK, ME_ERR_INVALID, ME_ERR_CUDA, ME_ERR_COMPILE, ME_ERR_UNSUPPORTED, ME_ERR_STATE = range(6)
 
@@ -116,6 +116,9 @@ SIGNATURES = {
     "me_mbar_hist_words": (ctypes.c_int, [_vp, _i32, _vp, ctypes.POINTER(_i64)]),
     "me_mbar_hist_pass": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _vp, _i64, ctypes.c_double, _vp, _i32, _vp, _vp,
                                          _vp, _vp, _vp, _vp, _i32, _vp]),
+    "me_mbar_cov_words": (ctypes.c_int, [_vp, _i32, _i32, _i32, ctypes.POINTER(_i64)]),
+    "me_mbar_cov_pass": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _vp, _i64, _i32, _vp, _vp, _i32, _i32, _vp, _vp,
+                                        _i32, _vp]),
     "me_last_error": (_cp, [_vp]),
 }
 

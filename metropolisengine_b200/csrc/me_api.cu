@@ -42,7 +42,7 @@ struct KernelRef {
     bool valid() const { return rt != nullptr || drv != nullptr; }
 };
 struct KernelSet {
-    KernelRef run, init, propose, accept, energy, run_mp, run_pt, run_hx, mbar, mbar_hist;
+    KernelRef run, init, propose, accept, energy, run_mp, run_pt, run_hx, mbar, mbar_hist, mbar_cov;
     bool valid() const { return run.valid(); }
 };
 
@@ -198,7 +198,8 @@ int nvrtc_compile(int n_real, int n_complex, int energy_id, const std::string &u
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_accept(const __grid_constant__ MeParams p) { me::accept_body<UserCfg>(p); }\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_energy(const __grid_constant__ MeParams p) { me::energy_body<UserCfg>(p); }\n"
            "extern \"C\" __global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) me_k_mbar(const __grid_constant__ MeMbarParams q) { me::mbar_pass_body<UserCfg>(q); }\n"
-           "extern \"C\" __global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) me_k_mbar_hist(const __grid_constant__ MeMbarParams q) { me::mbar_hist_body<UserCfg>(q); }\n";
+           "extern \"C\" __global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) me_k_mbar_hist(const __grid_constant__ MeMbarParams q) { me::mbar_hist_body<UserCfg>(q); }\n"
+           "extern \"C\" __global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) me_k_mbar_cov(const __grid_constant__ MeMbarParams q) { me::mbar_cov_body<UserCfg>(q); }\n";
     const char *hdr_names[] = {"me_params.h", "me_math.cuh", "me_device.cuh", "me_energies.cuh", "me_kernels.cuh",
                                "me_mbar.cuh"};
     const char *hdr_src[] = {me_src_params_h, me_src_math_cuh, me_src_device_cuh, me_src_energies_cuh,
@@ -654,7 +655,7 @@ int resolve_kernels(me_engine *e, int energy_id, const std::string &user_src) {
                 e->ks.run.rt = t[i].run; e->ks.init.rt = t[i].init; e->ks.run_mp.rt = t[i].run_mp;
                 e->ks.propose.rt = t[i].propose; e->ks.accept.rt = t[i].accept; e->ks.energy.rt = t[i].energy;
                 e->ks.run_pt.rt = t[i].run_pt; e->ks.run_hx.rt = t[i].run_hx; e->ks.mbar.rt = t[i].mbar;
-                e->ks.mbar_hist.rt = t[i].mbar_hist;
+                e->ks.mbar_hist.rt = t[i].mbar_hist; e->ks.mbar_cov.rt = t[i].mbar_cov;
                 return ME_OK;
             }
     }
@@ -690,6 +691,7 @@ int resolve_kernels(me_engine *e, int energy_id, const std::string &user_src) {
         d.moduleGetFunction(&ks.run_hx.drv, mod, "me_k_run_hx") != CUDA_SUCCESS ||
         d.moduleGetFunction(&ks.mbar.drv, mod, "me_k_mbar") != CUDA_SUCCESS ||
         d.moduleGetFunction(&ks.mbar_hist.drv, mod, "me_k_mbar_hist") != CUDA_SUCCESS ||
+        d.moduleGetFunction(&ks.mbar_cov.drv, mod, "me_k_mbar_cov") != CUDA_SUCCESS ||
         (e->cfg.n_complex > 0 && d.moduleGetFunction(&ks.run_mp.drv, mod, "me_k_run_mp") != CUDA_SUCCESS))
         return fail(e, ME_ERR_CUDA, "cuModuleGetFunction failed on the runtime-compiled module");
     g_cache[key] = ks;
@@ -1031,6 +1033,122 @@ int mbar_hist_bins(me_engine *e, int n_axes, const int32_t *n_bins, long long &B
         if (B * (e->n_rungs + 2) > ME_MBAR_HIST_MAX_WORDS)
             return fail(e, ME_ERR_INVALID, "histogram too large: bins x (rungs + 2) must not exceed 24576 doubles");
     }
+    return ME_OK;
+}
+
+/* the samples of an MBAR-type pass (rows [row0, rows) of one storage chunk, every stride-th row, every local chain) and
+   the fields every pass shares: q.n_rungs and the sample range (row0 / stride / n_per_state checks) */
+int mbar_samples(me_engine *e, const double *ts, int64_t rows, int64_t row0, int64_t stride, const double *f,
+                 int64_t n_per_state, MeMbarParams &q) {
+    if (rows < 1 || row0 < 0 || row0 >= rows) return fail(e, ME_ERR_INVALID, "row0 must lie in [0, rows)");
+    if (stride < 1) return fail(e, ME_ERR_INVALID, "stride must be >= 1");
+    if (n_per_state < 1) return fail(e, ME_ERR_INVALID, "n_per_state must be >= 1");
+    const long long ld = e->cfg.n_chains, n_rows = (rows - row0 + stride - 1) / stride;
+    q.ts = ts; q.ld = ld; q.row0 = row0; q.stride = stride; q.n_samples = n_rows * ld;
+    q.ts_cols = e->lay.TS_COLS;
+    q.n_rungs = e->n_rungs; q.use_reject = e->use_reject;
+    q.n_per_state = (double)n_per_state; q.log_n = std::log((double)n_per_state);
+    q.f = f;
+    return ME_OK;
+}
+
+/* the state table of me_mbar_pass and me_mbar_cov_pass: the R rungs, then n_target targets (target_temps[t],
+   target_consts[t][K] or the handle's constants); sets q.n_states = R + n_target */
+int mbar_states(me_engine *e, int n_target, const double *target_temps, const double *target_consts, MeMbarParams &q) {
+    if (n_target > 0 && !target_temps) return fail(e, ME_ERR_INVALID, "target_temps is required when n_target > 0");
+    const int R = e->n_rungs, S = R + n_target;
+    const bool ham = e->rung_k > 0;
+    const int K = ham ? e->rung_k : e->n_consts;
+    if (n_target > 0 && ham && !target_consts)
+        return fail(e, ME_ERR_INVALID, "targets of a Hamiltonian ladder need their constants (target_consts)");
+    for (int s = 0; s < S; s++) {
+        const double *tk = target_consts && s >= R ? target_consts + (size_t)(s - R) * K : nullptr;
+        const int rc = s < R ? mbar_state(e, s, 0.0, nullptr, q.inv_temp[s], q.consts[s])
+                             : mbar_state(e, -1, target_temps[s - R], tk, q.inv_temp[s], q.consts[s]);
+        if (rc != ME_OK) return rc;
+    }
+    q.n_states = S;
+    return ME_OK;
+}
+
+/* Geometry of a covariance pass (me_mbar.cuh, mbar_cov_body) over the covered states [first, first + count) of S
+ * states: nb 8-row blocks of weights, mb blocks per covered state's m = 2D + 2 observables, and per covered state c the
+ * tile list [(V_ci, ONE), (V_ci, W_j) j < nb] for i < mb, then [(V_ci, V_cj), j <= i], which k_mbar_cov_unpack reads.
+ * fits: the tiles fit the list and one warp's accumulators and staging fit the 227 KB shared-memory opt-in. */
+struct MbarCovLayout {
+    int nb, mb, m, n_tiles, z_rows, rw, per_warp;
+    long long words;
+    bool fits;
+    unsigned char ta[ME_MBAR_COV_MAX_TILES], tb[ME_MBAR_COV_MAX_TILES];
+};
+void mbar_cov_layout(int d, int n_states, int n_rungs, int count, MbarCovLayout &m) {
+    m.nb = (n_states + 7) / 8;
+    m.m = 2 * d + 2;
+    m.mb = (m.m + 7) / 8;
+    const int nb = m.nb, mb = m.mb, per = mb * (nb + 1) + mb * (mb + 1) / 2;
+    m.n_tiles = count * per;
+    m.z_rows = 8 * (2 * nb + 1 + count * mb);
+    m.rw = 2 + 64 * m.n_tiles;
+    m.per_warp = (m.n_tiles * 64 + m.z_rows * ME_MBAR_LD) * 8;
+    m.words = 2 + (long long)count * (m.m + (long long)m.m * (n_rungs + 1) + (long long)m.m * (m.m + 1) / 2);
+    m.fits = m.n_tiles <= ME_MBAR_COV_MAX_TILES && ME_MBAR_HEAD * 8 + m.per_warp <= ME_MBAR_SMEM_OPTIN;
+    if (!m.fits) return;
+    int t = 0;
+    for (int c = 0; c < count; c++) {
+        const int v0 = 2 * nb + 1 + c * mb;
+        for (int i = 0; i < mb; i++) {
+            m.ta[t] = (unsigned char)(v0 + i); m.tb[t++] = (unsigned char)nb;
+            for (int j = 0; j < nb; j++) { m.ta[t] = (unsigned char)(v0 + i); m.tb[t++] = (unsigned char)j; }
+        }
+        for (int i = 0; i < mb; i++)
+            for (int j = 0; j <= i; j++) { m.ta[t] = (unsigned char)(v0 + i); m.tb[t++] = (unsigned char)(v0 + j); }
+    }
+}
+
+/* reduced partial row [n_nan, n_overflow, tiles[n_tiles][8][8]] -> the sums vector of me_mbar_cov_pass: per covered
+   state o[m], C[m][R + 1] (the last column is C_a*), Q[m (m + 1) / 2] (sums = that, or sums += that) */
+__global__ void k_mbar_cov_unpack(const double *raw, double *sums, int R, int nb, int mb, int m, int first, long long words,
+                                  int accumulate) {
+    const long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= words) return;
+    const double *tile = raw + 2;
+    const long long per = m + (long long)m * (R + 1) + (long long)m * (m + 1) / 2;
+    const long long tc = mb * (nb + 1) + mb * (mb + 1) / 2;
+    double v;
+    if (w < 2) {
+        v = raw[w];
+    } else {
+        const long long c = (w - 2) / per;
+        long long r = (w - 2) % per;
+        const double *tt = tile + c * tc * 64;
+        if (r < m) {
+            v = tt[(r / 8) * (nb + 1) * 64 + (r % 8) * 8];
+        } else if ((r -= m) < (long long)m * (R + 1)) {
+            const int a = (int)(r / (R + 1)), k = (int)(r % (R + 1)), col = k < R ? k : first + (int)c;
+            v = tt[((a / 8) * (nb + 1) + 1 + col / 8) * 64 + (a % 8) * 8 + col % 8];
+        } else {
+            r -= (long long)m * (R + 1);
+            int a = 0;
+            while ((long long)(a + 1) * (a + 2) / 2 <= r) a++;
+            const int b = (int)(r - (long long)a * (a + 1) / 2), i = a / 8, j = b / 8;
+            v = tt[(mb * (nb + 1) + i * (i + 1) / 2 + j) * 64 + (a % 8) * 8 + b % 8];
+        }
+    }
+    sums[w] = accumulate ? sums[w] + v : v;
+}
+
+/* the checks me_mbar_cov_words and me_mbar_cov_pass share: those of me_mbar_pass, the covered range and the fit */
+int mbar_cov_check(me_engine *e, int n_target, int cov_first, int cov_count, MbarCovLayout &m) {
+    const int rc = mbar_check(e, n_target);
+    if (rc != ME_OK) return rc;
+    const int S = e->n_rungs + n_target;
+    if (cov_count < 1 || cov_first < 0 || cov_first > S - cov_count)
+        return fail(e, ME_ERR_INVALID, "the covered states [cov_first, cov_first + cov_count) must be a non-empty range "
+                                       "inside [0, rungs + targets)");
+    mbar_cov_layout(e->lay.D, S, e->n_rungs, cov_count, m);
+    if (!m.fits)
+        return fail(e, ME_ERR_INVALID, "too many covered states for one pass: one warp's tiles and staging exceed the "
+                                       "227 KB of shared memory (cover fewer states per pass)");
     return ME_OK;
 }
 
@@ -1864,33 +1982,17 @@ int me_mbar_pass(me_engine *e, const double *ts, int64_t rows, int64_t row0, int
     int rc = mbar_check(e, n_target);
     if (rc != ME_OK) return rc;
     if (!ts || !f || !sums) return fail(e, ME_ERR_INVALID, "ts, f and sums are required");
-    if (n_target > 0 && !target_temps) return fail(e, ME_ERR_INVALID, "target_temps is required when n_target > 0");
-    if (rows < 1 || row0 < 0 || row0 >= rows) return fail(e, ME_ERR_INVALID, "row0 must lie in [0, rows)");
-    if (stride < 1) return fail(e, ME_ERR_INVALID, "stride must be >= 1");
-    if (n_per_state < 1) return fail(e, ME_ERR_INVALID, "n_per_state must be >= 1");
-    const int R = e->n_rungs, S = R + n_target;
-    const bool ham = e->rung_k > 0;
-    const int K = ham ? e->rung_k : e->n_consts;
-    if (n_target > 0 && ham && !target_consts)
-        return fail(e, ME_ERR_INVALID, "targets of a Hamiltonian ladder need their constants (target_consts)");
     MeMbarParams q;
     memset(&q, 0, sizeof(q));
-    for (int s = 0; s < S; s++) {
-        const double *tk = target_consts && s >= R ? target_consts + (size_t)(s - R) * K : nullptr;
-        rc = s < R ? mbar_state(e, s, 0.0, nullptr, q.inv_temp[s], q.consts[s])
-                   : mbar_state(e, -1, target_temps[s - R], tk, q.inv_temp[s], q.consts[s]);
-        if (rc != ME_OK) return rc;
-    }
+    rc = mbar_samples(e, ts, rows, row0, stride, f, n_per_state, q);
+    if (rc != ME_OK) return rc;
+    rc = mbar_states(e, n_target, target_temps, target_consts, q);
+    if (rc != ME_OK) return rc;
     if (!e->ks.mbar.valid()) return fail(e, ME_ERR_STATE, "no MBAR kernel for this engine (device functors only)");
+    const int S = q.n_states;
     MbarLayout m;
     mbar_layout(e->lay.D, S, with_obs ? 1 : 0, m);
-    const long long ld = e->cfg.n_chains, n_rows = (rows - row0 + stride - 1) / stride;
-    q.ts = ts; q.ld = ld; q.row0 = row0; q.stride = stride; q.n_samples = n_rows * ld;
-    q.ts_cols = e->lay.TS_COLS;
-    q.n_rungs = R; q.n_states = S; q.use_reject = e->use_reject;
     q.nb = m.nb; q.nx = m.nx; q.n_tiles = m.n_tiles; q.z_rows = m.z_rows; q.rw = m.rw;
-    q.n_per_state = (double)n_per_state; q.log_n = std::log((double)n_per_state);
-    q.f = f;
     memcpy(q.tile_a, m.ta, sizeof(m.ta));
     memcpy(q.tile_b, m.tb, sizeof(m.tb));
     double *raw = nullptr;
@@ -1950,30 +2052,21 @@ int me_mbar_hist_pass(me_engine *e, const double *ts, int64_t rows, int64_t row0
         q.axis_inv_w[a] = (double)n_bins[a] / (hi[a] - lo[a]);
         q.n_bins[a] = n_bins[a];
     }
-    if (rows < 1 || row0 < 0 || row0 >= rows) return fail(e, ME_ERR_INVALID, "row0 must lie in [0, rows)");
-    if (stride < 1) return fail(e, ME_ERR_INVALID, "stride must be >= 1");
-    if (n_per_state < 1) return fail(e, ME_ERR_INVALID, "n_per_state must be >= 1");
+    rc = mbar_samples(e, ts, rows, row0, stride, f, n_per_state, q);
+    if (rc != ME_OK) return rc;
     const int R = e->n_rungs;
-    const bool ham = e->rung_k > 0;
-    if (ham && !target_consts)
+    if (e->rung_k > 0 && !target_consts)
         return fail(e, ME_ERR_INVALID, "the target of a Hamiltonian ladder needs its constants (target_consts)");
-    for (int s = 0; s < R; s++) {
-        rc = mbar_state(e, s, 0.0, nullptr, q.inv_temp[s], q.consts[s]);
-        if (rc != ME_OK) return rc;
-    }
+    rc = mbar_states(e, 0, nullptr, nullptr, q);
+    if (rc != ME_OK) return rc;
     rc = mbar_state(e, -1, target_temp, target_consts, q.t_inv_temp, q.t_consts);
     if (rc != ME_OK) return rc;
     if (!e->ks.mbar_hist.valid()) return fail(e, ME_ERR_STATE, "no MBAR kernel for this engine (device functors only)");
-    const long long ld = e->cfg.n_chains, n_rows = (rows - row0 + stride - 1) / stride;
-    q.ts = ts; q.ld = ld; q.row0 = row0; q.stride = stride; q.n_samples = n_rows * ld;
-    q.ts_cols = e->lay.TS_COLS;
-    q.n_rungs = R; q.n_states = R + 1; q.use_reject = e->use_reject;
+    q.n_states = R + 1;
     q.n_axes = n_axes;
     q.hw = (int)(B * (R + 2));
     q.z_rows = 2 * (R + 1);
     q.rw = 4 + q.hw;
-    q.n_per_state = (double)n_per_state; q.log_n = std::log((double)n_per_state);
-    q.f = f;
     double *raw = nullptr;
     rc = mbar_launch(e, e->ks.mbar_hist, q, (q.hw + q.z_rows * ME_MBAR_LD) * 8, true, (cudaStream_t)stream, raw);
     if (rc != ME_OK) return rc;
@@ -1981,6 +2074,46 @@ int me_mbar_hist_pass(me_engine *e, const double *ts, int64_t rows, int64_t row0
                                                                                          accumulate ? 1 : 0);
     cudaError_t ce = cudaGetLastError();
     if (ce != cudaSuccess) return fail(e, ME_ERR_CUDA, std::string("MBAR histogram pass: ") + cudaGetErrorString(ce));
+    return ME_OK;
+}
+
+int me_mbar_cov_words(me_engine *e, int32_t n_target, int32_t cov_first, int32_t cov_count, int64_t *words) {
+    if (!e || !words) return ME_ERR_INVALID;
+    MbarCovLayout m;
+    const int rc = mbar_cov_check(e, n_target, cov_first, cov_count, m);
+    if (rc != ME_OK) return rc;
+    *words = m.words;
+    return ME_OK;
+}
+
+int me_mbar_cov_pass(me_engine *e, const double *ts, int64_t rows, int64_t row0, int64_t stride, const double *f,
+                     int64_t n_per_state, int32_t n_target, const double *target_temps, const double *target_consts,
+                     int32_t cov_first, int32_t cov_count, const double *centers, double *sums, int32_t accumulate,
+                     void *stream) {
+    if (!e) return ME_ERR_INVALID;
+    MbarCovLayout m;
+    int rc = mbar_cov_check(e, n_target, cov_first, cov_count, m);
+    if (rc != ME_OK) return rc;
+    if (!ts || !f || !sums) return fail(e, ME_ERR_INVALID, "ts, f and sums are required");
+    if (!centers) return fail(e, ME_ERR_INVALID, "centers is required");
+    MeMbarParams q;
+    memset(&q, 0, sizeof(q));
+    rc = mbar_samples(e, ts, rows, row0, stride, f, n_per_state, q);
+    if (rc != ME_OK) return rc;
+    rc = mbar_states(e, n_target, target_temps, target_consts, q);
+    if (rc != ME_OK) return rc;
+    if (!e->ks.mbar_cov.valid()) return fail(e, ME_ERR_STATE, "no MBAR kernel for this engine (device functors only)");
+    q.nb = m.nb; q.n_tiles = m.n_tiles; q.z_rows = m.z_rows; q.rw = m.rw;
+    q.centers = centers; q.cov_first = cov_first; q.n_cov = cov_count; q.cov_mb = m.mb;
+    memcpy(q.cov_tile_a, m.ta, sizeof(m.ta));
+    memcpy(q.cov_tile_b, m.tb, sizeof(m.tb));
+    double *raw = nullptr;
+    rc = mbar_launch(e, e->ks.mbar_cov, q, m.per_warp, false, (cudaStream_t)stream, raw);
+    if (rc != ME_OK) return rc;
+    k_mbar_cov_unpack<<<(unsigned)((m.words + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+        raw, sums, e->n_rungs, m.nb, m.mb, m.m, cov_first, m.words, accumulate ? 1 : 0);
+    cudaError_t ce = cudaGetLastError();
+    if (ce != cudaSuccess) return fail(e, ME_ERR_CUDA, std::string("MBAR covariance pass: ") + cudaGetErrorString(ce));
     return ME_OK;
 }
 

@@ -125,16 +125,23 @@ template <class C>
 __global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) k_mbar_hist(const __grid_constant__ MeMbarParams q) {
     mbar_hist_body<C>(q);
 }
+/* the covariance pass of expectation uncertainties over the same rows (me_mbar_cov_pass) */
+template <class C>
+__global__ void __launch_bounds__(32 * ME_MBAR_MAX_WARPS, 1) k_mbar_cov(const __grid_constant__ MeMbarParams q) {
+    mbar_cov_body<C>(q);
+}
 #ifndef ME_NVRTC
 template <class C, bool EXT = IsExternal<C>::value>
 struct MbarKernel {
     static const void *get() { return (const void *)&k_mbar<C>; }
     static const void *hist() { return (const void *)&k_mbar_hist<C>; }
+    static const void *cov() { return (const void *)&k_mbar_cov<C>; }
 };
 template <class C>
 struct MbarKernel<C, true> {
     static const void *get() { return nullptr; }
     static const void *hist() { return nullptr; }
+    static const void *cov() { return nullptr; }
 };
 #endif
 
@@ -143,7 +150,7 @@ struct MbarKernel<C, true> {
 /* one ahead-of-time instantiation */
 struct MeAotEntry {
     int n_real, n_complex, energy_id, strict;
-    const void *run, *init, *propose, *accept, *run_mp, *energy, *run_pt, *run_hx, *mbar, *mbar_hist;
+    const void *run, *init, *propose, *accept, *run_mp, *energy, *run_pt, *run_hx, *mbar, *mbar_hist, *mbar_cov;
 };
 
 #define ME_AOT_ENTRY(NR, NC, ETMPL, EID, STRICT)                                                        \
@@ -156,7 +163,8 @@ struct MeAotEntry {
       me::RunPtKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                             \
       me::RunHxKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                             \
       me::MbarKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::get(),                                              \
-      me::MbarKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::hist() }
+      me::MbarKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::hist(),                                             \
+      me::MbarKernel<me::Cfg<NR, NC, ETMPL, STRICT>>::cov() }
 
 /* the shapes of BASELINE.json's configs plus the shapes of the golden fixtures */
 #define ME_AOT_TABLE(STRICT)                                                      \

@@ -25,7 +25,8 @@
  * is bit-identical from run to run on one device.
  *
  * mbar_hist_body (k_mbar_hist, me_mbar_hist_pass) is the histogram pass of free-energy profiles over the same samples
- * and weights; mbar_sample is the per-sample evaluation both passes share. */
+ * and weights, mbar_cov_body (k_mbar_cov, me_mbar_cov_pass) the covariance pass of expectation uncertainties; mbar_sample
+ * is the per-sample evaluation all three passes share. */
 #ifndef ME_MBAR_CUH
 #define ME_MBAR_CUH
 
@@ -302,6 +303,101 @@ __device__ __forceinline__ void mbar_hist_body(const MeMbarParams &q) {
         } else {
             const double *a0 = me_mbar_smem + ME_MBAR_HEAD + (w - 4);
             for (int j = 0; j < nw; j++) v += a0[(long long)j * q.hw];
+        }
+        row[w] = v;
+    }
+}
+
+/* Covariance pass (me_mbar_cov_pass, DESIGN §3 "Uncertainties of reweighted expectations"): the samples and weights of
+ * mbar_pass_body with the same R rungs and targets, and for each covered state s = cov_first + c (c < n_cov) the centred
+ * observables a~ = a_s - c_s, a_s = [x_0..x_{D-1}, x_0^2..x_{D-1}^2, E_s, E_s^2] (m = 2D + 2).  Row blocks of z:
+ *     [0, nb)                 w_s           (rows s < S; the rest stay 0)
+ *     nb                      ONE
+ *     [nb+1, 2nb+1)           E_s           (mbar_sample's staging only)
+ *     2nb+1 + c mb + [0, mb)  w_s a~        (rows a < m of covered state c; mb = ceil(m / 8) blocks, padding rows 0)
+ * The host's tile list (me_api.cu, mbar_cov_layout) pairs each covered state's blocks with ONE (o_a), with every w block
+ * (C_ak against the rungs and the self column C_a* = sum w_s^2 a~) and with each other (Q_ab, b <= a).  Tiles accumulate
+ * per warp in shared memory as in mbar_pass_body; the CTA writes [n_nan, n_overflow, tiles[n_tiles][8][8]] and
+ * k_pool_reduce sums the rows in fixed order, so a pass is bit-identical from run to run on one device.
+ * Shared memory: 512 + 512 n_tiles + 288 z_rows bytes for one warp, at most the 227 KB opt-in (the host refuses larger
+ * ranges).  One covered state always fits: at D = 32 and S = 32 it takes 90 tiles and 144 rows, 88 KB. */
+template <class C>
+__device__ __forceinline__ void mbar_cov_body(const MeMbarParams &q) {
+    constexpr int D = Lay<C::NR, C::NC>::D, M = 2 * D + 2;
+    extern __shared__ __align__(16) double me_mbar_smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    const int r8 = lane >> 2, k4 = lane & 3;
+    const int S = q.n_states, R = q.n_rungs, nb = q.nb, mb = q.cov_mb;
+    double *fs = me_mbar_smem, *scal = me_mbar_smem + 32;
+    double *acc = me_mbar_smem + ME_MBAR_HEAD + (long long)warp * q.n_tiles * 64;
+    double(*z)[ME_MBAR_LD] =
+        reinterpret_cast<double(*)[ME_MBAR_LD]>(me_mbar_smem + ME_MBAR_HEAD + (long long)nw * q.n_tiles * 64) +
+        (long long)warp * q.z_rows;
+    const int W0 = 0, ONE = 8 * nb, E0 = 8 * (nb + 1), V0 = 8 * (2 * nb + 1);
+
+    for (int i = threadIdx.x; i < 32; i += blockDim.x) fs[i] = i < R ? q.f[i] : 0.0;
+    for (int i = lane; i < q.n_tiles * 64; i += 32) acc[i] = 0.0;
+    for (int r = 0; r < q.z_rows; r++) z[r][lane] = r == ONE ? 1.0 : 0.0;
+    __syncthreads();
+
+    const long long per = (q.n_samples + gridDim.x - 1) / gridDim.x;
+    const long long lo = (long long)blockIdx.x * per;
+    const long long hi = lo + per < q.n_samples ? lo + per : q.n_samples;
+    double n_bad = 0.0, n_ovf = 0.0;
+    for (long long base = lo + 32LL * warp; base < hi; base += 32LL * nw) {   /* warp-uniform trip count */
+        const long long n = base + lane;
+        double x[D];
+        bool live, bad, ovf;
+        double l;
+        mbar_sample<C, false>(q, fs, z, W0, E0, lane, n, hi, x, live, bad, ovf, l);
+        live = live && !bad && !ovf;
+        if (live) {
+            for (int c = 0; c < q.n_cov; c++) {
+                const int s = q.cov_first + c;
+                const double w = z[W0 + s][lane], e = z[E0 + s][lane];
+                const double *ce = q.centers + (long long)c * M;
+                double *v = &z[V0 + 8 * mb * c][0] + lane;
+#pragma unroll
+                for (int d = 0; d < D; d++) {
+                    v[d * ME_MBAR_LD] = w * (x[d] - ce[d]);
+                    v[(D + d) * ME_MBAR_LD] = w * (x[d] * x[d] - ce[D + d]);
+                }
+                v[2 * D * ME_MBAR_LD] = w * (e - ce[2 * D]);
+                v[(2 * D + 1) * ME_MBAR_LD] = w * (e * e - ce[2 * D + 1]);
+            }
+        } else {
+            n_bad += bad ? 1.0 : 0.0;
+            n_ovf += (!bad && ovf) ? 1.0 : 0.0;
+            for (int s = 0; s < S; s++) z[W0 + s][lane] = 0.0;
+            for (int c = 0; c < q.n_cov; c++)
+                for (int a = 0; a < M; a++) z[V0 + 8 * mb * c + a][lane] = 0.0;
+        }
+        __syncwarp();
+        for (int t = 0; t < q.n_tiles; t++) {
+            const int ra = 8 * q.cov_tile_a[t] + r8, rb = 8 * q.cov_tile_b[t] + r8;
+            double c0 = 0.0, c1 = 0.0;
+#pragma unroll
+            for (int kk = 0; kk < 8; kk++) dmma_8x8x4(c0, c1, z[ra][4 * kk + k4], z[rb][4 * kk + k4]);
+            acc[t * 64 + 2 * lane] += c0;
+            acc[t * 64 + 2 * lane + 1] += c1;
+        }
+        __syncwarp();
+    }
+    n_bad = warp_sum(n_bad);
+    n_ovf = warp_sum(n_ovf);
+    if (lane == 0) {
+        scal[4 * warp] = n_bad;
+        scal[4 * warp + 1] = n_ovf;
+    }
+    __syncthreads();
+    double *row = q.partial + (long long)blockIdx.x * q.rw;
+    for (int w = threadIdx.x; w < q.rw; w += blockDim.x) {
+        double v = 0.0;
+        if (w < 2) {
+            for (int j = 0; j < nw; j++) v += scal[4 * j + w];
+        } else {
+            const double *a0 = me_mbar_smem + ME_MBAR_HEAD + (w - 2);
+            for (int j = 0; j < nw; j++) v += a0[(long long)j * q.n_tiles * 64];
         }
         row[w] = v;
     }

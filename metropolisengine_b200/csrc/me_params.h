@@ -5,7 +5,7 @@
 #ifndef ME_PARAMS_H
 #define ME_PARAMS_H
 
-#define ME_PARAMS_VERSION 14
+#define ME_PARAMS_VERSION 15
 #define ME_MAX_CONSTS 16
 
 /* status bits written to the per-chain STATUS word (SURVEY §5 "failure detection") */
@@ -88,6 +88,7 @@ struct MeParams {
  * SASS of the step kernels, does not depend on the analysis.  The host fills the state table and the tile list. */
 #define ME_MBAR_MAX_STATES 32
 #define ME_MBAR_MAX_TILES 64
+#define ME_MBAR_COV_MAX_TILES 448     /* 448 tiles of 512 bytes fill the 227 KB opt-in */
 struct MeMbarParams {
     const double *ts;              /* [row][ts_cols][ld] time-series block of one storage chunk */
     long long ld;                  /* chains per row (the handle's n_chains) */
@@ -113,7 +114,13 @@ struct MeMbarParams {
     int n_axes, hw;
     int axis_kind[2];              /* 0: stored column axis_index; 1: modulus of complex parameter axis_index */
     int axis_index[2], n_bins[2];
+    /* covariance pass (me_mbar_cov_pass; appended): covered states [cov_first, cov_first + n_cov), each with m = 2D + 2
+     * centred observables in cov_mb 8-row blocks; n_tiles counts the tiles of cov_tile_a / cov_tile_b */
+    const double *centers;         /* [n_cov][m] device: the centres c_s subtracted from the observables */
+    int cov_first, n_cov, cov_mb;
+    unsigned char cov_tile_a[ME_MBAR_COV_MAX_TILES], cov_tile_b[ME_MBAR_COV_MAX_TILES];
 };
 #define ME_MBAR_HIST_MAX_WORDS 24576   /* B (R + 2) doubles: one warp's histogram and staging fit the 227 KB opt-in */
+#define ME_MBAR_SMEM_OPTIN 232448      /* 227 KB: the most dynamic shared memory one CTA may opt in to */
 
 #endif

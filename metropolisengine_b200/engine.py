@@ -1215,6 +1215,17 @@ class MetropolisEngine:
         self._check(self._lib.me_mbar_words(self._h, n_t, int(with_obs), ctypes.byref(words)))
         sums = torch.zeros(words.value, dtype=torch.float64, device=self.device)
         f_dev = torch.tensor(np.asarray(f, dtype=np.float64), device=self.device)
+        tt, kk = self._mbar_targets(temps, consts)
+        self._mbar_chunks(lambda t, used, lo, acc: self._lib.me_mbar_pass(
+            self._h, _ptr(t), used, lo, stride, _ptr(f_dev), n_per, n_t, tt, kk,
+            int(with_obs), _ptr(sums), acc, self._stream()), sums, row0, stride)
+        out = _mbar.unpack(sums.cpu().numpy(), R + n_t, self._d, with_obs)
+        self._mbar_refuse(out)
+        return out
+
+    def _mbar_targets(self, temps, consts):
+        """The target temperatures and constants of a pass as C arrays (constants: [n_target, K] or None)."""
+        n_t = int(np.size(temps))
         tt = (ctypes.c_double * max(n_t, 1))(*np.asarray(temps, dtype=np.float64).ravel().tolist())
         kk = None
         if consts is not None:
@@ -1223,11 +1234,38 @@ class MetropolisEngine:
             if arr.ndim != 2 or arr.shape != (n_t, K):
                 raise ValueError("target constants must be [n_target, %d] (the energy's constant count)" % K)
             kk = ctypes.cast((ctypes.c_double * arr.size)(*arr.ravel().tolist()), ctypes.c_void_p)
-        self._mbar_chunks(lambda t, used, lo, acc: self._lib.me_mbar_pass(
-            self._h, _ptr(t), used, lo, stride, _ptr(f_dev), n_per, n_t, ctypes.cast(tt, ctypes.c_void_p), kk,
-            int(with_obs), _ptr(sums), acc, self._stream()), sums, row0, stride)
-        out = _mbar.unpack(sums.cpu().numpy(), R + n_t, self._d, with_obs)
-        self._mbar_refuse(out)
+        return ctypes.cast(tt, ctypes.c_void_p), kk
+
+    def _mbar_cov_sums(self, f, temps, consts, first, count, centers, row0, stride):
+        """The covariance sums (``me_mbar_cov_pass``) of the states [first, first + count) of the rungs and the targets
+        (temps, consts) about centers [count, 2D + 2], over the rows row0, row0 + stride, ... of every local chain.  The
+        states are split into as few passes as the library accepts (the largest range that fits each time); each pass
+        runs chunk by chunk and is summed over the ranks.  Returns ``mbar.unpack_cov`` of all covered states, with
+        ``passes``, the (first, count) of each pass."""
+        from . import mbar as _mbar
+        R, n_t, m = self.temperatures.size, int(np.size(temps)), 2 * self._d + 2
+        n_per = len(range(row0, self._ts_rows, stride)) * (self.n_chains_total // R)
+        f_dev = torch.tensor(np.asarray(f, dtype=np.float64), device=self.device)
+        c_dev = torch.tensor(np.ascontiguousarray(centers, dtype=np.float64).reshape(count, m), device=self.device)
+        tt, kk = self._mbar_targets(temps, consts)
+        words = ctypes.c_int64()
+        parts, lo = [], first
+        while lo < first + count:
+            n = first + count - lo
+            while n > 1 and self._lib.me_mbar_cov_words(self._h, n_t, lo, n, ctypes.byref(words)) != _lib.ME_OK:
+                n -= 1
+            self._check(self._lib.me_mbar_cov_words(self._h, n_t, lo, n, ctypes.byref(words)))
+            sums = torch.zeros(words.value, dtype=torch.float64, device=self.device)
+            cen = c_dev[lo - first:lo - first + n]
+            self._mbar_chunks(lambda t, used, r0, acc: self._lib.me_mbar_cov_pass(
+                self._h, _ptr(t), used, r0, stride, _ptr(f_dev), n_per, n_t, tt, kk, lo, n, _ptr(cen), _ptr(sums), acc,
+                self._stream()), sums, row0, stride)
+            part = _mbar.unpack_cov(sums.cpu().numpy(), n, m, R)
+            self._mbar_refuse(part)
+            parts.append((lo, n, part))
+            lo += n
+        out = {k: np.concatenate([p[k] for _, _, p in parts]) for k in ("o", "C", "Q")}
+        out.update(n_nan=0, n_overflow=0, passes=[(a, n) for a, n, _ in parts])
         return out
 
     def _mbar_chunks(self, launch, sums, row0, stride):

@@ -11,7 +11,10 @@ free energies f; everything here is S x S algebra on those sums (S <= 32 states)
 * target states: f_t = -ln s_t and <a>_t = sum_n w_nt a_t / s_t;
 * free-energy profiles (pymbar's histogram FES): the histogram pass (``me_mbar_hist_pass``) sums a target's weights per
   bin of one or two coordinates, and ``profile`` turns them into f_b, p_b and their errors by Theta over the rungs plus
-  one state per non-empty bin.
+  one state per non-empty bin;
+* uncertainties of expectations (pymbar's ``compute_expectations`` covariance): the covariance pass
+  (``me_mbar_cov_pass``) sums products of the centred observables with the weights, and ``expectation_covariance``
+  turns them into the covariance of a state's means by Theta over the rungs plus one centred column per observable.
 
 The covariance assumes uncorrelated samples: pass ``stride`` of about the statistical inefficiency g of the energy
 column (``MetropolisEngine.statistical_inefficiency``).
@@ -98,6 +101,49 @@ def profile(h, q, c, w_out, G, n_per_state, reference="lowest"):
     return f - f[ref], df, p
 
 
+def unpack_cov(sums, n_cov, m, n_rungs):
+    """The sums vector of ``me_mbar_cov_pass`` as a dict: ``n_nan``, ``n_overflow``, and per covered state ``o`` [n, m]
+    (sum w a~), ``C`` [n, m, R + 1] (sum w a~ w_k, then the self column sum w^2 a~) and ``Q`` [n, m, m] (sum w^2 a~ a~,
+    symmetric)."""
+    sums = np.asarray(sums, dtype=np.float64)
+    R, p = n_rungs, m * (m + 1) // 2
+    body = sums[2:2 + n_cov * (m + m * (R + 1) + p)].reshape(n_cov, -1)
+    Q = np.zeros((n_cov, m, m))
+    Q[:, np.tril_indices(m)[0], np.tril_indices(m)[1]] = body[:, m + m * (R + 1):]
+    Q = Q + np.tril(Q, -1).transpose(0, 2, 1)
+    return dict(n_nan=int(sums[0]), n_overflow=int(sums[1]), o=body[:, :m].copy(),
+                C=body[:, m:m + m * (R + 1)].reshape(n_cov, m, R + 1), Q=Q)
+
+
+def expectation_covariance(G, s, state, o, C, Q, n_per_state):
+    """Covariance [m, m] of the means <a>_s of one state from its covariance sums (o [m], C [m, R + 1], Q [m, m], about
+    any centres) and the plain pass's s [S] and G [S, S] (R = C.shape[1] - 1 rungs first) at the same f.
+
+    delta = o / s_s; the centred column v_a = w_s (a - <a>_s) / s_s has G(v_a, k) = (C_ak - delta_a G_sk) / s_s and
+    G(v_a, v_b) = (Q_ab - delta_a C_b* - delta_b C_a* + delta_a delta_b G_ss) / s_s^2; Theta over [rungs, v] with
+    N = [N .. N, 0 .. 0] gives Cov(<a>_s, <b>_s) = Theta(v_a, v_b).  This is pymbar's compute_expectations covariance
+    A_i A_j (Theta_AiAj - Theta_Ai,s - Theta_s,Aj + Theta_ss) with its shifted, normalised columns A: Theta is bilinear
+    in the columns."""
+    R, m = C.shape[1] - 1, o.size
+    ss = s[state]
+    d = o / ss
+    gvk = (C[:, :R] - d[:, None] * G[state, :R][None, :]) / ss
+    cs = C[:, R]
+    gvv = (Q - np.outer(d, cs) - np.outer(cs, d) + np.outer(d, d) * G[state, state]) / (ss * ss)
+    Ga = np.block([[G[:R, :R], gvk.T], [gvk, gvv]])
+    th = theta(Ga, np.concatenate([np.full(R, float(n_per_state)), np.zeros(m)]))
+    return th[R:, R:]
+
+
+def heat_capacity(E, E2, cov, T):
+    """C = (<E^2> - <E>^2) / T^2 (k_B = 1) and its standard error by the delta method over the (E, E^2) block cov
+    [..., 2, 2] of the means, gradient [-2 <E>, 1] / T^2."""
+    E, E2, T = np.asarray(E, dtype=np.float64), np.asarray(E2, dtype=np.float64), np.asarray(T, dtype=np.float64)
+    g = np.stack([-2.0 * E, np.ones_like(E)], axis=-1) / (T * T)[..., None]
+    var = np.einsum("...i,...ij,...j->...", g, cov, g)
+    return (E2 - E * E) / (T * T), np.sqrt(np.clip(var, 0.0, None))
+
+
 def solve(pass_fn, n_rungs, n_per_state, tol=1e-10, max_iter=100):
     """Newton on F(f) = sum L - N sum_k f_k with f_0 = 0.  ``pass_fn(f)`` returns the unpacked sums of one pass at f.
     Returns (f, sums at f, iterations, converged)."""
@@ -159,7 +205,7 @@ class MBARResult:
         self.n_iterations = int(n_iterations)
         self.converged = bool(converged)
 
-    def evaluate(self, temp=None, consts=None):
+    def evaluate(self, temp=None, consts=None, uncertainty=False):
         """Free energies and expectations at target states, or at the rungs when both arguments are None.
 
         temp    one temperature or a sequence (one per target); None: the rungs' own temperatures when consts names
@@ -169,7 +215,15 @@ class MBARResult:
 
         Returns a dict of numpy arrays over the requested states (Q of them): ``f`` [Q] (reduced, same gauge as
         ``free_energies``), ``df`` [Q] (standard error of f - f_0), ``x_mean`` [Q, D], ``x2_mean`` [Q, D] (parameters
-        in the order real, Re c, Im c), ``E_mean`` [Q], ``E2_mean`` [Q] (the energy with the state's constants)."""
+        in the order real, Re c, Im c), ``E_mean`` [Q], ``E2_mean`` [Q] (the energy with the state's constants).
+
+        uncertainty=True adds the errors of the means (pymbar's compute_expectations covariance) from device covariance
+        passes over the same rows, as many as the shared-memory bound needs; the keys above are the same bits as
+        without it.  Added: ``dx_mean`` [Q, D], ``dx2_mean`` [Q, D], ``dE_mean`` [Q], ``dE2_mean`` [Q] (standard
+        errors), ``obs_cov`` [Q, m, m] (covariance of the m = 2D + 2 means in the order x, x^2, E, E^2), and
+        ``heat_capacity`` [Q] = (<E^2> - <E>^2) / T^2 (k_B = 1, the functor's energy units) with ``dheat_capacity``
+        [Q] (delta method).  Like ``df`` these errors assume uncorrelated samples: they are only as good as the
+        ``stride`` of ``MetropolisEngine.mbar`` (about the statistical inefficiency of the energy column)."""
         eng = self._engine
         R = self.free_energies.size
         if temp is None and consts is None:
@@ -201,8 +255,20 @@ class MBARResult:
         df_all = differences(th)[0]
         ob = sums["obs"] / s[:, None]
         sel = slice(R, S) if n_t else slice(0, R)
-        return dict(f=f_all[sel].copy(), df=df_all[sel].copy(), x_mean=ob[sel, :d].copy(), x2_mean=ob[sel, d:2 * d].copy(),
-                    E_mean=ob[sel, 2 * d].copy(), E2_mean=ob[sel, 2 * d + 1].copy())
+        out = dict(f=f_all[sel].copy(), df=df_all[sel].copy(), x_mean=ob[sel, :d].copy(), x2_mean=ob[sel, d:2 * d].copy(),
+                   E_mean=ob[sel, 2 * d].copy(), E2_mean=ob[sel, 2 * d + 1].copy())
+        if not uncertainty:
+            return out
+        first, q = (R, n_t) if n_t else (0, R)
+        cs = eng._mbar_cov_sums(self.free_energies, temps, kt, first, q, ob[sel], *self._sample)
+        cov = np.stack([expectation_covariance(sums["G"], s, first + i, cs["o"][i], cs["C"][i], cs["Q"][i], self._n)
+                        for i in range(q)])
+        se = np.sqrt(np.clip(np.diagonal(cov, axis1=1, axis2=2), 0.0, None))
+        t_states = temps if n_t else np.broadcast_to(np.asarray(eng.temperatures, dtype=np.float64), (R,))
+        c, dc = heat_capacity(out["E_mean"], out["E2_mean"], cov[:, 2 * d:, 2 * d:], t_states)
+        out.update(dx_mean=se[:, :d].copy(), dx2_mean=se[:, d:2 * d].copy(), dE_mean=se[:, 2 * d].copy(),
+                   dE2_mean=se[:, 2 * d + 1].copy(), obs_cov=cov, heat_capacity=c, dheat_capacity=dc)
+        return out
 
     def pmf(self, coords, bins, range, temp=None, consts=None, reference="lowest"):
         """Free-energy profile of one target state along one or two coordinates (pymbar's histogram FES), from a device
