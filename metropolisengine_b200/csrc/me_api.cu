@@ -174,19 +174,19 @@ int nvrtc_compile(int n_real, int n_complex, int energy_id, const std::string &u
         src += "};\n}\n";
     }
     src += std::string("typedef me::Cfg<ME_NR, ME_NC, ") + tmpl + ", (ME_STRICT != 0)> UserCfg;\n";
-    /* same register policy as the ahead-of-time kernels (me_kernels.cuh): small shapes at most 160 registers */
+    /* same register policy as the ahead-of-time kernels (me_kernels.cuh): small shapes at most ME_SMALL_MAXNREG registers */
     src += "#if ME_NR + 2 * ME_NC <= 4\n"
-           "extern \"C\" __global__ void __maxnreg__(160) me_k_run(const __grid_constant__ MeParams p) { me::run_body<UserCfg>(p); }\n"
+           "extern \"C\" __global__ void __maxnreg__(ME_SMALL_MAXNREG) me_k_run(const __grid_constant__ MeParams p) { me::run_body<UserCfg>(p); }\n"
            "#else\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run(const __grid_constant__ MeParams p) { me::run_body<UserCfg>(p); }\n"
            "#endif\n"
            "#if ME_NR + 2 * ME_NC <= 4\n"
-           "extern \"C\" __global__ void __maxnreg__(160) me_k_run_pt(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, me::LADDER_TEMP>(p); }\n"
+           "extern \"C\" __global__ void __maxnreg__(ME_SMALL_MAXNREG) me_k_run_pt(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, me::LADDER_TEMP>(p); }\n"
            "#else\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run_pt(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, me::LADDER_TEMP>(p); }\n"
            "#endif\n"
            "#if ME_NR + 2 * ME_NC <= 4\n"
-           "extern \"C\" __global__ void __maxnreg__(160) me_k_run_hx(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, me::LADDER_HAM>(p); }\n"
+           "extern \"C\" __global__ void __maxnreg__(ME_SMALL_MAXNREG) me_k_run_hx(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, me::LADDER_HAM>(p); }\n"
            "#else\n"
            "extern \"C\" __global__ void __launch_bounds__(ME_MAX_BLOCK) me_k_run_hx(const __grid_constant__ MeParams p) { me::run_body<UserCfg, false, me::LADDER_HAM>(p); }\n"
            "#endif\n"
@@ -583,14 +583,11 @@ int plan_segments(me_engine *e, const KernelRef &k, long long n_blocks, long lon
 void choose_dims(me_engine *e) {
     const long long n = e->cfg.n_chains;
     int block = 128;
-    if (const char *env = getenv("ME_BLOCK")) block = atoi(env);
-    else if (n <= (long long)e->n_sm * 32 * 16) block = 32;     /* up to four warps per sub-partition: finest balance; beyond
+    if (n <= (long long)e->n_sm * 32 * 16) block = 32;          /* up to four warps per sub-partition: finest balance; beyond
                                                                    that 64-thread CTAs halve the per-CTA fixed cost, which
                                                                    short launches feel (tests/scripts/c5_launch_probe.py:
                                                                    131,072 chains x 100 steps, 106.6 -> 100.8 us) */
     else if (n <= (long long)e->n_sm * 32 * 64) block = 64;
-    if (block < 32) block = 32;
-    if (block > ME_MAX_BLOCK) block = ME_MAX_BLOCK;
     {   /* shapes whose pooled moments run on the FP64 tensor cores stage them per warp in static shared memory sized for
            me_pool_mma_max_block(D) threads (run_body in me_device.cuh: POOL_MMA) */
         const int d = e->cfg.n_real + 2 * e->cfg.n_complex;
@@ -598,7 +595,6 @@ void choose_dims(me_engine *e) {
         if (me::me_pool_mma_shape(d, poolw) && poolw <= ME_MAX_POOLW && block > me::me_pool_mma_max_block(d))
             block = me::me_pool_mma_max_block(d);
     }
-    block = (block / 32) * 32;
     e->block = block;
     e->grid = (int)((n + block - 1) / block);
 }

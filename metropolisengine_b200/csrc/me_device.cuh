@@ -25,19 +25,13 @@
 #include "me_math.cuh"
 
 #define ME_MAX_BLOCK 256
-#ifndef ME_PAIR_BIG
-#define ME_PAIR_BIG 0          /* shapes with D > 4: 1 = process the steps in pairs too (see run_body) */
-#endif
-#ifndef ME_BIG_LOOKAHEAD
-#define ME_BIG_LOOKAHEAD 0     /* shapes with D > 4: 1 = generate the draws of step s+1 during step s (costs D+2 doubles of
-                                  registers).  Measured on the 3r+4c shape, 262,144 chains: pairs + look-ahead 1.51e10,
-                                  single steps + look-ahead 1.55e10, single steps without look-ahead 1.70e10 chain-steps/s
-                                  (ceil(D/2) independent generator calls per step already give the warp its ILP; the
-                                  27 KB pair-unrolled loop stalls on instruction fetch) */
-#endif
 #define ME_FULL 0xffffffffu
 #define ME_SEG_MAX_D 4         /* shapes up to this D = n_real + 2 n_complex support work-queue time segmentation */
 #define ME_MAX_POOLW 600
+/* small problems keep running statistics (up to this many words) and pooled accumulators (up to this many) in registers
+   for the whole launch; larger ones touch them in global memory at measure time only */
+#define ME_STATS_REG_MAX 12
+#define ME_POOL_REG_MAX 9
 
 namespace me {
 
@@ -757,8 +751,8 @@ __device__ __forceinline__ double warp_sum(double v) {
  * and the B fragment of a thread are the same word when the row block equals the column block — and issues
  * 8 x NBX (NBX + 1) / 2 DMMAs (C3: 24); the observable sums are a second product against a unit vector.  No shuffles and
  * no CTA barrier: the 87 warp_sum reductions of the 3r+4c shape (870 SHFL + two __syncthreads per measure) were 39 % of
- * that kernel's time (tests/scripts/c3_probe.py: 13.9 ms with them, 8.5 ms without).  Each accumulator element belongs to
- * one thread, which adds it to its word of the warp's row of pooled sums (pw). */
+ * that kernel's time (profiles/r02_c3_probe_pooling_and_register_caps.txt: 13.9 ms with them, 8.5 ms without).  Each
+ * accumulator element belongs to one thread, which adds it to its word of the warp's row of pooled sums (pw). */
 #define ME_YB_LD 20            /* doubles per staged row: 16 chains + 4 of padding (fragment reads take two wavefronts) */
 /* staging rows (a multiple of 8 holding [x - s, 1]) and the CTA size that keeps the per-warp staging + the warp's row of sums
    + the math tables inside the 48 KB of static shared memory: D <= 15 -> 16 rows, 128 threads; D <= 23 -> 24 rows, 64
@@ -1052,24 +1046,13 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     constexpr bool STRICT = Cfg::STRICT;
     constexpr int D = L::D;
     constexpr bool PT = LM != LADDER_NONE, HAM = LM == LADDER_HAM;
-    /* small problems keep running statistics and pooled accumulators in registers for the whole launch;
-       larger ones touch them in global memory at measure time only */
-#ifndef ME_STATS_REG_MAX
-#define ME_STATS_REG_MAX 12      /* build-time experiment knobs (tests/scripts/nreg_probe.py) */
-#endif
-#ifndef ME_POOL_REG_MAX
-#define ME_POOL_REG_MAX 9
-#endif
     constexpr bool STATS_REG = (L::D + L::NCOVR + L::NCOVC + L::NOBS) <= ME_STATS_REG_MAX;
     constexpr bool POOL_REG = L::POOLW <= ME_POOL_REG_MAX;
     constexpr bool POOL_OK = L::POOLW <= ME_MAX_POOLW;        /* static shared-memory budget */
     constexpr int PW = POOL_OK ? L::POOLW : 1;
-#ifndef ME_POOL_MMA
-#define ME_POOL_MMA 1            /* build-time experiment knob: 0 = warp_sum reductions for every shape beyond POOL_REG */
-#endif
     /* mid-sized shapes: pooled moments on the FP64 tensor cores (pool_mma_update); their CTAs are at most
        me_pool_mma_max_block(D) threads (choose_dims in me_api.cu follows the same rule) */
-    constexpr bool POOL_MMA = !PT && ME_POOL_MMA && !POOL_REG && POOL_OK && me_pool_mma_shape(L::D, L::POOLW);
+    constexpr bool POOL_MMA = !PT && !POOL_REG && POOL_OK && me_pool_mma_shape(L::D, L::POOLW);
     constexpr int POOL_MMA_BLOCK = me_pool_mma_max_block(L::D), YB_ROWS = POOL_MMA ? me_pool_mma_rows(L::D) : 1;
     constexpr int POOL_WARPS = (POOL_MMA ? POOL_MMA_BLOCK : ME_MAX_BLOCK) / 32;
     /* ladders stage nothing in shared memory (it would cost one-warp CTAs occupancy): register-pooled shapes add their rung
@@ -1145,10 +1128,7 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
 #pragma unroll
         for (int w = 0; w < L::POOLW; w++) pacc[w] = 0.0;
     }
-#ifndef ME_EXPERIMENT_NO_POOL
-#define ME_EXPERIMENT_NO_POOL 0   /* build-time experiment knob (tests/scripts/c3_probe.py): what the pooled moments cost */
-#endif
-    const bool pooling = POOL_OK && p.pool != nullptr && p.do_measure && !ME_EXPERIMENT_NO_POOL;
+    const bool pooling = POOL_OK && p.pool != nullptr && p.do_measure;
     if (POOL_MMA && blockDim.x > POOL_MMA_BLOCK) __trap();       /* the host never launches this (choose_dims) */
     if (pooling && POOL_MMA) {
         for (int w = threadIdx.x; w < POOL_WARPS * PW; w += blockDim.x) (&pool_warp[0][0])[w] = 0.0;
@@ -1219,9 +1199,9 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
        counts is how many independent dependency chains one warp has in flight.  Small shapes run THREE stages per
        iteration — Philox rounds of step s+2 (10 dependent IMAD.WIDE/LOP3 rounds, ~180 cycles), Box-Muller of step
        s+1 (log -> rsqrt -> multiply, ~200 cycles), state update of step s (~190 cycles); larger shapes already
-       have ceil(D/2) independent generator calls per step and keep two stages (registers). */
+       have ceil(D/2) independent generator calls per step and generate each step's draws in that step (see the step
+       loop below). */
     constexpr bool DEEP = L::D <= 4;
-    constexpr bool AHEAD = DEEP || (ME_BIG_LOOKAHEAD != 0);
     Draws<L> cur;
     Raw<L> raw_a, raw_b;
     const Pins pins = load_pins(tables);
@@ -1241,12 +1221,12 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
     }
     typedef typename TabSelect<TAB_SMEM>::type Tab;
     const Tab logtab{TAB_SMEM ? logtab_s : reinterpret_cast<const double2 *>(p.logtab)};
-    if (!inject && p.spm > 0 && AHEAD) {
+    if (!inject && p.spm > 0 && DEEP) {
         gen_draws<L, STRICT, Tab>(rng, step_first, tables, cur, pins, p, logtab, lt);
-        if (DEEP) gen_bits<L>(rng, step_first + 1u, raw_a);
+        gen_bits<L>(rng, step_first + 1u, raw_a);
     }
 
-    /* one step: consumes the draws in `use`, generates the draws of the following step into `make` */
+    /* one step: consumes the draws in `use`; small shapes generate the draws of the following step into `make` */
     unsigned step32 = step_first;
     auto one_step = [&](const Gains &g, Draws<L> &use, Draws<L> &make, Raw<L> &raw_in, Raw<L> &raw_out) {
         double prop[D];
@@ -1271,8 +1251,6 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
             } else if (DEEP) {
                 gen_bits<L>(rng, step32 + 2u, raw_out);
                 shape_draws<L, STRICT, Tab>(raw_in, tables, make, pins, p, logtab, 0u, lt);
-            } else if (AHEAD) {
-                gen_draws<L, STRICT, Tab>(rng, step32 + 1u, tables, make, pins, p, logtab, lt);
             } else {
                 gen_draws<L, STRICT, Tab>(rng, step32, tables, use, pins, p, logtab, lt);
             }
@@ -1315,22 +1293,22 @@ __device__ __forceinline__ void run_body(const MeParams &p) {
             /* steps in pairs so that the two draw buffers swap roles by name instead of by register moves */
             Draws<L> nxt;
             unsigned k = 0;
-            if (ME_PAIR_BIG || DEEP) {
+            if (DEEP) {
                 for (; k + 1 < spm; k += 2) {
                     one_step(g, cur, nxt, raw_a, raw_b);
                     one_step(g, nxt, cur, raw_b, raw_a);
                 }
                 if (k < spm) {
                     one_step(g, cur, nxt, raw_a, raw_b);
-                    if (!inject) { cur = nxt; if (DEEP) raw_a = raw_b; }
+                    if (!inject) { cur = nxt; raw_a = raw_b; }
                 }
             } else {
-                /* larger shapes: one step per iteration (the pair-unrolled loop of a 3r+4c shape is 27 KB of code) */
+                /* larger shapes: one step per iteration, without look-ahead.  Measured on the 3r+4c shape, 262,144 chains:
+                   pairs + look-ahead 1.51e10, single steps + look-ahead 1.55e10, single steps without look-ahead 1.70e10
+                   chain-steps/s (ceil(D/2) independent generator calls per step already give the warp its ILP; the look-ahead
+                   costs D+2 doubles of registers and the 27 KB pair-unrolled loop stalls on instruction fetch) */
 #pragma unroll 1
-                for (; k < spm; k++) {
-                    one_step(g, cur, nxt, raw_a, raw_b);
-                    if (!inject && AHEAD) cur = nxt;
-                }
+                for (; k < spm; k++) one_step(g, cur, nxt, raw_a, raw_b);
             }
             if (p.do_measure) {
                 n += 1;

@@ -25,12 +25,6 @@
 #include "me_k4_device.cuh"
 #include "me_rt.h"
 
-extern "C" int me_k4v1_steps(double *state, long long ld, long long n_chains, unsigned long long chain_offset,
-                             unsigned long long seed, unsigned long long step0, long long n_steps, int n_sm_avail,
-                             long long n_meas, double temp, double target, double ratio, const double *consts4, int use_wall,
-                             const void *factor, const double *s_a, unsigned char *last_accept, float *dbg_z,
-                             float *dbg_delta, void *stream);
-
 namespace {
 
 using k4::Layout;
@@ -415,8 +409,7 @@ struct me_k4 {
     unsigned long long step = 0;
     int n_sm = 148;
     int reserved_sms = 0;          /* SMs the step kernel leaves free (for a concurrent factor refresh) */
-    bool use_v1 = false;           /* ME_K4_V1=1: the first-version step kernel (n_c = 64, built-in functor) */
-    bool no_tma = false;           /* ME_K4_NO_TMA=1, or the driver has no cuTensorMapEncodeTiled */
+    bool no_tma = false;           /* the driver has no cuTensorMapEncodeTiled */
     /* step / init kernels: ahead-of-time (built-in functor) or runtime-compiled (user functor) */
     const void *steps_rt = nullptr, *steps_xp_rt = nullptr, *init_rt = nullptr;
     CUfunction steps_drv = nullptr, init_drv = nullptr;
@@ -501,10 +494,6 @@ int me_k4_create(const me_k4_config *cfg, me_k4 **out) {
     int n_sm = 0;
     if (cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, cfg->device) == cudaSuccess && n_sm > 0) e->n_sm = n_sm;
     else cudaGetLastError();
-    const char *v1 = getenv("ME_K4_V1");
-    e->use_v1 = v1 && atoi(v1) != 0 && e->nc == 64;
-    const char *nt = getenv("ME_K4_NO_TMA");
-    e->no_tma = nt && atoi(nt) != 0;
     k4_bind_builtin(e);
     *out = e;
     return ME_OK;
@@ -556,7 +545,6 @@ int me_k4_set_energy_source(me_k4 *e, const char *src, const double *consts, int
     memset(e->consts, 0, sizeof(e->consts));
     for (int i = 0; i < n_consts; i++) e->consts[i] = consts[i];
     e->use_reject = use_reject ? 1 : 0;
-    e->use_v1 = false;
     return ME_OK;
 }
 
@@ -683,17 +671,7 @@ int me_k4_step(me_k4 *e, int64_t n_steps, const double *s_a, float *dbg_z, float
     if (n_steps <= 0) return ME_OK;
     if (e->step + (unsigned long long)n_steps >= 0xffffffffull) return k4_fail(e, ME_ERR_INVALID, "step counter overflow");
     int prev = -1; cudaGetDevice(&prev); cudaSetDevice(e->cfg.device);
-    int rc = ME_OK;
-    if (e->use_v1) {
-        const int avail = e->n_sm - e->reserved_sms > 0 ? e->n_sm - e->reserved_sms : 1;
-        const int ce = me_k4v1_steps(e->state, e->cfg.n_chains, e->cfg.n_chains, (unsigned long long)e->cfg.chain_offset,
-                                     e->cfg.seed, e->step, n_steps, avail, e->n_measure, e->cfg.temp,
-                                     e->cfg.target_acceptance, e->cfg.ratio, e->consts, e->use_reject, e->factor, s_a,
-                                     e->last_accept, dbg_z, dbg_delta, stream);
-        if (ce != 0) rc = k4_fail(e, ME_ERR_CUDA, std::string("k4_steps: ") + cudaGetErrorString((cudaError_t)ce));
-    } else {
-        rc = k4_launch_steps(e, n_steps, s_a, dbg_z, dbg_delta, dbg_scal, nullptr, nullptr, stream);
-    }
+    const int rc = k4_launch_steps(e, n_steps, s_a, dbg_z, dbg_delta, dbg_scal, nullptr, nullptr, stream);
     cudaSetDevice(prev);
     if (rc != ME_OK) return rc;
     e->step += (unsigned long long)n_steps;
@@ -732,7 +710,6 @@ int me_k4_step_measure(me_k4 *e, int64_t n_steps, const double *s_a, double *ts,
                        void *stream) {
     if (!e || !e->state || !s_a || !shift || !scratch || !inc) return ME_ERR_INVALID;
     if (n_steps <= 0) return k4_fail(e, ME_ERR_INVALID, "me_k4_step_measure needs at least one step");
-    if (e->use_v1) return k4_fail(e, ME_ERR_UNSUPPORTED, "the first-version step kernel has no fused measure");
     if (e->step + (unsigned long long)n_steps >= 0xffffffffull) return k4_fail(e, ME_ERR_INVALID, "step counter overflow");
     const int max_parts = e->n_sm < 1 ? 1 : e->n_sm;
     if (scratch_doubles < (int64_t)(max_parts + 1) * partw(e->nc)) return k4_fail(e, ME_ERR_INVALID, "moments scratch too small");

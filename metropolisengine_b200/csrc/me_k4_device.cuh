@@ -6,7 +6,7 @@
  *        Delta[128 chains x N] = Z[128 x K normals] . B^T[K x N],     N = K = 2 n_c,
  * B the real embedding of conj(G)/sqrt2 in interleaved (Re, Im) coordinates, C_c = G G^H.
  *
- * Roles inside a CTA of 16 warps (no CTA-wide barrier in the step loop; K4_WIDE=1 doubles both roles):
+ * Roles inside a CTA of 16 warps (no CTA-wide barrier in the step loop):
  *   warps 8..15  GENERATORS  Philox4x32-7 -> BF16 normals by table (inverse CDF), written straight into the UMMA canonical K-major
  *                            operand layout.  The K dimension is produced in two halves, each its own pipeline stage
  *                            (mbarriers z_full / z_empty), so the generators of step s+1 start as soon as the MMAs of step
@@ -50,15 +50,12 @@ typedef unsigned int u32;
 typedef unsigned long long u64;
 
 constexpr int TILE = 128;               /* chains per tile = MMA M = TMEM lanes */
-/* CTA shape.  Default: 16 warps = 8 epilogue warps (2 column groups x 4 lane quarters) + 8 generator warps, 128 registers
- * each.  K4_WIDE=1 builds 32 warps (16 + 16, launched at 64 registers, epilogue warpgroups grown to 80 and generator
- * warpgroups shrunk to 48 with setmaxnreg).  Measured on B200 (profiles/r02_k4_probe_*.txt, 32,768 chains, 10 / 100 steps per
- * launch): 16 warps 90.5 / 766 us, 32 warps 96.2 / 832 us — with twice the warps the issue slots fill up (52 -> 58 %) but
- * the four threads of a chain repeat the decision and the scalar draws, the mbarrier polls double, and the shared-memory
+/* CTA shape: 16 warps = 8 epilogue warps (2 column groups x 4 lane quarters) + 8 generator warps, 128 registers each.
+ * It beat a 32-warp layout (16 + 16, launched at 64 registers, epilogue warpgroups grown to 80 and generator warpgroups
+ * shrunk to 48 with setmaxnreg) on B200 (profiles/r02_k4_probe_*.txt, 32,768 chains, 10 / 100 steps per launch):
+ * 16 warps 90.5 / 766 us, 32 warps 96.2 / 832 us — with twice the warps the issue slots fill up (52 -> 58 %) but the
+ * four threads of a chain repeat the decision and the scalar draws, the mbarrier polls double, and the shared-memory
  * pipe (state tile, partial sums, the generator's table) becomes the limiter (51 % of its cycles, MIO-throttle stalls). */
-#ifndef K4_WIDE
-#define K4_WIDE 0
-#endif
 /* Two instantiations of the step kernel (template parameter XP):
  *   XP = true   the proposed state x' = x + sigma Delta of a step is parked in TMEM (FP64 = two 32-bit columns per coordinate,
  *               the thread's own lane) between the energy pass and the accept pass, which then is a TMEM load + the stores of
@@ -69,13 +66,15 @@ constexpr int TILE = 128;               /* chains per tile = MMA M = TMEM lanes 
  *   XP = false  the accept pass recomputes x' from the increments and the state tile; the tail's accumulators have their own
  *               TMEM columns, accumulate over all tiles of the CTA and are written once (+14 us per measure otherwise at
  *               two tiles per CTA). */
-constexpr int EPI_GROUPS = K4_WIDE ? 4 : 2;                 /* threads per chain in the epilogue (column groups) */
-constexpr int EPI_WARPS = 4 * EPI_GROUPS, GEN_WARPS = K4_WIDE ? 16 : 8;
+constexpr int EPI_GROUPS = 2;                               /* threads per chain in the epilogue (column groups) */
+constexpr int EPI_WARPS = 4 * EPI_GROUPS, GEN_WARPS = 8;
 constexpr int GEN_PAR = GEN_WARPS * 32 / TILE;              /* generator threads per operand row */
+/* the measure tail pairs generator thread (chain m, c_par) with epilogue thread (chain m, column group c_par): it takes the
+   per-chain measurement of the second half of that thread's modes */
+static_assert(EPI_GROUPS == GEN_PAR, "one generator thread per epilogue column group");
 constexpr int GEN_WARP0 = EPI_WARPS, MMA_WARP = GEN_WARP0;  /* lane 0 of the first generator warp also issues the MMAs: registers
                                                                are granted in groups of four warps, a 33rd warp would cost four */
 constexpr int THREADS = 32 * (EPI_WARPS + GEN_WARPS);
-constexpr int EPI_REGS = 80, GEN_REGS = 48;                 /* setmaxnreg targets (K4_WIDE) */
 constexpr u32 SCALAR_SLOT = 0x10000u;   /* Philox slot of the per-chain scalar draws (beyond any operand chunk) */
 constexpr int PHILOX_ROUNDS = 7;
 
@@ -464,9 +463,6 @@ __device__ __forceinline__ void steps_body(const StepParams &p, const TensorMap 
 
     if (warp >= GEN_WARP0) {
         /* ================================================================== generators (+ the MMA issuer) */
-#if K4_WIDE
-        asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(GEN_REGS));
-#endif
         const bool issuer = warp == MMA_WARP && lane == 0;
         if (issuer && p.use_tma) {
             constexpr int ROWS = CHUNKS * N;                 /* rows of 16 bytes */
@@ -561,7 +557,7 @@ __device__ __forceinline__ void steps_body(const StepParams &p, const TensorMap 
                     *reinterpret_cast<unsigned short *>(yh_row + (2 * j + 1) * 16) = (unsigned short)(hi_pair >> 16);
                     ylp[jj] = bf16x2_rn(yr - bf16_lo_to_float(hi_pair), yi - bf16_hi_to_float(hi_pair));
                 }
-                if (EPI_GROUPS == GEN_PAR && act) {
+                if (act) {
                     /* the second half of the modes of (chain m, column group c_par): their per-chain measurement */
                     constexpr int EM = NC / EPI_GROUPS, SHARE = EM / 2;
                     const double dn = (double)p.n_meas_after, inv_n = 1.0 / dn, shrink = (dn - 1.0) * inv_n;
@@ -605,13 +601,10 @@ __device__ __forceinline__ void steps_body(const StepParams &p, const TensorMap 
         }
     } else {
         /* ================================================================== epilogue */
-#if K4_WIDE
-        asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(EPI_REGS));
-#endif
         const int q4 = warp & 3, g = warp >> 2;        /* lane quarter (TMEM lanes 32 q4 ..), column group */
         const int m = 32 * q4 + lane;                  /* chain within the tile = TMEM lane */
         constexpr int MODES = NC / EPI_GROUPS;         /* modes per thread */
-        constexpr int GEN_SHARE = (EPI_GROUPS == GEN_PAR) ? MODES / 2 : 0;   /* modes whose measurement the generators take */
+        constexpr int GEN_SHARE = MODES / 2;           /* modes whose measurement the generators take */
         constexpr int COLS = 2 * MODES;                /* accumulator columns per thread */
         constexpr int LDCH = COLS < 32 ? COLS : 32;    /* columns per tcgen05.ld */
         constexpr int LD1 = XP ? (COLS < 16 ? COLS : 16) : LDCH;     /* energy pass: increments per load (x' words are held
@@ -699,14 +692,8 @@ __device__ __forceinline__ void steps_body(const StepParams &p, const TensorMap 
                 named_barrier(1 + q4, 32 * EPI_GROUPS);      /* the column groups of this lane quarter exchange their sums */
                 if (act) {
                     /* ---- decision, evaluated identically by every thread of the chain (ME:247-258) */
-                    double t0, t1;
-                    if (EPI_GROUPS == 4) {
-                        t0 = (S.part[it & 1][0][0][m] + S.part[it & 1][1][0][m]) + (S.part[it & 1][2][0][m] + S.part[it & 1][3][0][m]);
-                        t1 = (S.part[it & 1][0][1][m] + S.part[it & 1][1][1][m]) + (S.part[it & 1][2][1][m] + S.part[it & 1][3][1][m]);
-                    } else {
-                        t0 = S.part[it & 1][0][0][m] + S.part[it & 1][1][0][m];
-                        t1 = S.part[it & 1][0][1][m] + S.part[it & 1][1][1][m];
-                    }
+                    const double t0 = S.part[it & 1][0][0][m] + S.part[it & 1][1][0][m];
+                    const double t1 = S.part[it & 1][0][1][m] + S.part[it & 1][1][1][m];
                     const double a_new = fma(sig * s_a, za, a);
                     const bool wall = p.use_wall && Energy::reject(a_new, p.consts);
                     if (!wall) {

@@ -23,24 +23,15 @@ struct Cfg {
  * work-queue time segmentation of run_body. */
 template <class C, bool SMALL = (C::NR + 2 * C::NC <= 4)>
 struct RunKernel;
-#ifndef ME_SMALL_MAXNREG
-#define ME_SMALL_MAXNREG 160     /* build-time experiment knob (make SMALL_NREG=...): see tests/scripts/nreg_probe.py */
-#endif
+#define ME_SMALL_MAXNREG 160
 template <class C>
 __global__ void __maxnreg__(ME_SMALL_MAXNREG) k_run_small(const __grid_constant__ MeParams p) {
     run_body<C>(p);
 }
-#ifdef ME_BIG_MAXNREG
-template <class C>
-__global__ void __maxnreg__(ME_BIG_MAXNREG) k_run(const __grid_constant__ MeParams p) {
-    run_body<C>(p);
-}
-#else
 template <class C>
 __global__ void __launch_bounds__(ME_MAX_BLOCK, 1) k_run(const __grid_constant__ MeParams p) {
     run_body<C>(p);
 }
-#endif
 #ifndef ME_NVRTC   /* host-side selection; the run-time compiled kernels (me_api.cu) name their entry points directly */
 template <class C>
 struct RunKernel<C, true> { static const void *get() { return (const void *)&k_run_small<C>; } };
@@ -52,33 +43,19 @@ template <class C>
 __global__ void __maxnreg__(ME_SMALL_MAXNREG) k_run_pt_small(const __grid_constant__ MeParams p) {
     run_body<C, false, LADDER_TEMP>(p);
 }
-#ifdef ME_BIG_MAXNREG
-template <class C>
-__global__ void __maxnreg__(ME_BIG_MAXNREG) k_run_pt(const __grid_constant__ MeParams p) {
-    run_body<C, false, LADDER_TEMP>(p);
-}
-#else
 template <class C>
 __global__ void __launch_bounds__(ME_MAX_BLOCK, 1) k_run_pt(const __grid_constant__ MeParams p) {
     run_body<C, false, LADDER_TEMP>(p);
 }
-#endif
 /* Hamiltonian ladders (me_set_hamiltonian_ladder): the same register policy */
 template <class C>
 __global__ void __maxnreg__(ME_SMALL_MAXNREG) k_run_hx_small(const __grid_constant__ MeParams p) {
     run_body<C, false, LADDER_HAM>(p);
 }
-#ifdef ME_BIG_MAXNREG
-template <class C>
-__global__ void __maxnreg__(ME_BIG_MAXNREG) k_run_hx(const __grid_constant__ MeParams p) {
-    run_body<C, false, LADDER_HAM>(p);
-}
-#else
 template <class C>
 __global__ void __launch_bounds__(ME_MAX_BLOCK, 1) k_run_hx(const __grid_constant__ MeParams p) {
     run_body<C, false, LADDER_HAM>(p);
 }
-#endif
 #ifndef ME_NVRTC
 /* caller-evaluated energies never run fused, so they get no ladder kernel */
 template <class C> struct IsExternal { static constexpr bool value = false; };

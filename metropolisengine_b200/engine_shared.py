@@ -17,7 +17,6 @@ measure b use the factor of measure b-1.  The lag is deterministic and only shap
 ``async_refresh=False`` gives the strictly sequential schedule.
 """
 import ctypes
-import os
 import math
 
 import numpy as np
@@ -160,8 +159,6 @@ class SharedCovarianceEngine:
                                           self._stream()))
         self.record = bool(record)
         self._ts_chunks, self._ts_chunk_rows = [], int(ts_chunk_rows)
-        self._fused_measure = not (os.environ.get("ME_K4_SPLIT_MEASURE", "0") not in ("", "0")
-                                   or os.environ.get("ME_K4_V1", "0") not in ("", "0"))
 
     @classmethod
     def from_reference_arguments(cls, energy_functions, reject_condition=None, initial_real_params=None,
@@ -379,12 +376,9 @@ class SharedCovarianceEngine:
         if refresh:
             self._in_flight = (ev, idx)
 
-    def run(self, n_measures, steps_per_measure, fused_measure=None):
+    def run(self, n_measures, steps_per_measure, fused_measure=True):
         """``n_measures`` x [``steps_per_measure`` x step_all(), measure()].  By default every block is one step_measure()
-        launch; ``fused_measure=False`` (or ME_K4_SPLIT_MEASURE=1) keeps step() and measure() as separate kernels with
-        all-FP64 pooled moments."""
-        if fused_measure is None:
-            fused_measure = self._fused_measure
+        launch; ``fused_measure=False`` keeps step() and measure() as separate kernels with all-FP64 pooled moments."""
         for _ in range(int(n_measures)):
             if fused_measure and steps_per_measure >= 1:
                 self.step_measure(int(steps_per_measure))
